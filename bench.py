@@ -12,7 +12,7 @@ data-path collective).  One tile =
 The FC head between extractor and NMS is dense GEMM in Jittor (out of scope): its outputs (class
 scores, decoded boxes) are synthetic, random-init-like softmax scores.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
 
 `value` : tiles/s, inputs resident in HBM, device-timed (CUDA events), max over ranks.  The 8 tiles of a step are a batch
@@ -180,7 +180,6 @@ def run_reference(args, rank, world):
         if R.available(name):
             R._lib(name)
     inputs = tile_inputs(0)
-    args.steps = min(args.steps, 20)  # ~0.5 s per 1-tile step on 16 cores: keeps the arm within a minute
     for _ in range(args.warmup_ref):
         reference_tile(nproc, inputs)
     t0 = time.perf_counter()
@@ -333,6 +332,30 @@ def verify_tile0(tile_np, tile_dev, out_bufs, device_step, cfg, core, last_np=No
             "checksum_out_tile0": float(got_feat.double().sum())}
 
 
+DUMP_ROI_ROWS = 1024   # RoI feature rows dumped (256 x 7 x 7 float32 = 50 kB each; all 32 000 would be 1.6 GB)
+
+
+def dump_outputs(path, out8, step_results):
+    """What the last timed step computed, as a caller of it receives it, written to path/<name>.npy (float32, or
+    float64 for indices and counts; 53 MB in all): a fixed seeded sample of the RoI feature rows of the batched
+    extractor output, every tile's obb2poly polygons, and every tile's kept detections and labels, concatenated in
+    tile order with the per-tile counts."""
+    import torch
+    os.makedirs(path, exist_ok=True)
+    rows = np.sort(np.random.default_rng(0).choice(out8.shape[0], DUMP_ROI_ROWS, replace=False))
+    counts = [int(r[3].item()) for r in step_results]
+    arrays = {
+        "roi_feature_rows": rows.astype(np.float64),
+        "roi_features": out8[torch.from_numpy(rows).to(out8.device)].cpu().numpy(),
+        "polygons": np.stack([r[0].cpu().numpy() for r in step_results]),
+        "detections": np.concatenate([r[1][:k].cpu().numpy() for r, k in zip(step_results, counts)]),
+        "labels": np.concatenate([r[2][:k].cpu().numpy() for r, k in zip(step_results, counts)]).astype(np.float32),
+        "detections_per_tile": np.array(counts, np.float64),
+    }
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 def run_ours(args, rank, world, local_rank):
     numa = bind_to_gpu_numa_node(local_rank) if world > 1 else None
     import torch
@@ -378,16 +401,18 @@ def run_ours(args, rank, world, local_rank):
     out_bufs = [out8[i * K_ROIS:(i + 1) * K_ROIS] for i in range(TILES_PER_GPU)]   # tile i's rows of the batched output
 
     def device_step():
+        """Issue one step; returns per tile (polygons, dets, labels, count); the RoI features land in out8."""
         main = torch.cuda.current_stream()
         for st in side + side2:
             st.wait_stream(main)
         # a tile's NMS chain (sorts -> decision matrix -> per-class scan: long, mostly latency-bound) does not depend
         # on its RoI features, so it goes on a stream of its own and is issued first: the scans (10 CTAs per tile)
         # then run beside the RoI kernels instead of forming the tail of the step
+        results = []
         for i, (feats, rois, boxes, scores) in enumerate(tiles):
             with torch.cuda.stream(side[i % NSTREAMS]):
-                core.obb2poly(boxes)
-                core.multiclass_nms_rotated(boxes, scores, SCORE_THR, IOU_THR, MAX_NUM)
+                polys = core.obb2poly(boxes)
+                results.append((polys,) + core.multiclass_nms_rotated(boxes, scores, SCORE_THR, IOU_THR, MAX_NUM))
         # the RoI features of all 8 tiles: ONE extractor call (32 000 RoIs; the persistent gather pays its start-up and
         # tail once per step instead of once per tile)
         for g in range(TILES_PER_GPU // ROI_BATCH):
@@ -399,6 +424,7 @@ def run_ours(args, rank, world, local_rank):
                     core.roi_align_rotated_forward(cfgb, [f8[lo:hi] for f8 in feats8], roisb[g], out=out8[lo * K_ROIS:hi * K_ROIS])
         for st in side + side2:
             main.wait_stream(st)
+        return results
 
     def barrier():
         torch.cuda.synchronize()
@@ -421,7 +447,7 @@ def run_ours(args, rank, world, local_rank):
     launches0 = _lib.launch_count()
     graph = torch.cuda.CUDAGraph()
     with torch.cuda.graph(graph):
-        device_step()
+        step_results = device_step()   # tensors of the graph's pool: every replay rewrites them
     launches_per_step = _lib.launch_count() - launches0
     sampler = ClockSampler(local_rank)
     if rank == 0:
@@ -439,6 +465,8 @@ def run_ours(args, rank, world, local_rank):
     ms_total = max_over_ranks(e0.elapsed_time(e1))
     clocks = sampler.stop() if rank == 0 else None
     value = world * TILES_PER_GPU * args.steps / (ms_total * 1e-3)
+    if args.dump_outputs and rank == 0:   # before anything else writes out8
+        dump_outputs(args.dump_outputs, out8, step_results)
 
     # ---- component timings (same tiles, same process): per-kernel CUDA events
     def timed(fn, reps):
@@ -732,7 +760,12 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-verify", action="store_true", help="skip the oracle check of tile 0 after the timed region")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed to DIR/<name>.npy (inputs are seeded: two builds can "
+                         "be compared output for output)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     args.warmup_ref = min(args.warmup, 1)
     rank = int(os.environ.get("RANK", "0"))

@@ -28,22 +28,24 @@ _pi = C.POINTER(C.c_int)
 _pu8 = C.POINTER(C.c_uint8)
 
 
+_SO_COUNT = os.path.join(HERE, "liborsdet_oracle_count.so")
+
+
 def build(force: bool = False) -> str:
-    """gcc -O2 -ffp-contract=off: IEEE single ops exactly as written (no FMA contraction)."""
-    if force or not os.path.exists(_SO) or os.path.getmtime(_SO) < os.path.getmtime(_SRC):
-        subprocess.check_call(["gcc", "-std=c99", "-O2", "-ffp-contract=off", "-fno-fast-math", "-shared",
-                               "-fPIC", _SRC, "-o", _SO, "-lm"])
+    """gcc -O2 -ffp-contract=off: IEEE single ops exactly as written (no FMA contraction).  Also builds the
+    -DORC_COUNT_FLOPS variant `flop_census` loads, so that bench.py compiles nothing at run time."""
+    for so, extra in ((_SO, []), (_SO_COUNT, ["-DORC_COUNT_FLOPS"])):
+        if force or not os.path.exists(so) or os.path.getmtime(so) < os.path.getmtime(_SRC):
+            subprocess.check_call(["gcc", "-std=c99", "-O2", "-ffp-contract=off", "-fno-fast-math", *extra, "-shared",
+                                   "-fPIC", _SRC, "-o", so, "-lm"])
     return _SO
 
 
 def flop_census(boxes1, boxes2, version: int = 1):
     """FLOPs the reference's rotated-IoU algorithm spends on `boxes1 x boxes2` (every pair, no early exit), counted by
     a -DORC_COUNT_FLOPS build of the same C restatement (SURVEY 8d).  Returns (flops, pairs)."""
-    so = _SO.replace(".so", "_count.so")
-    if not os.path.exists(so) or os.path.getmtime(so) < os.path.getmtime(_SRC):
-        subprocess.check_call(["gcc", "-std=c99", "-O2", "-ffp-contract=off", "-fno-fast-math", "-DORC_COUNT_FLOPS", "-shared",
-                               "-fPIC", _SRC, "-o", so, "-lm"])
-    L = C.CDLL(so)
+    build()
+    L = C.CDLL(_SO_COUNT)
     L.orc_flops_read.restype = C.c_ulonglong
     L.orc_pairs_read.restype = C.c_ulonglong
     L.orc_box_iou_rotated.argtypes = [_pf, C.c_int, _pf, C.c_int, C.c_int, C.c_int, _pf]
