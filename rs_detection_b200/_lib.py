@@ -124,22 +124,39 @@ def ptr(t) -> int:
 
 
 _workspaces: dict = {}
+# A CUDA graph keeps the raw address of every scratch buffer it was captured with, so a buffer handed out while a graph
+# was being captured must never go back to the caching allocator: every replay would write into whatever tensor the
+# allocator placed there next.  `_graph_held` names the keys whose current buffer a capture used; when such a buffer is
+# replaced (growth) or released it moves to `_retired`, which lives as long as the process.  Sizes grow by more than
+# 1.25x per replacement, so growth alone retires at most 4x the live buffer of a key; each release_workspaces() after a
+# capture retires one more buffer per key that capture used.
+_graph_held: set = set()
+_retired: list = []
 
 
 def workspace(nbytes: int, tag: str = "default") -> torch.Tensor:
     """Cached per-(device, stream, tag) scratch buffer, grown geometrically; contents are undefined.
-    Keyed by the current stream so that tiles processed on different streams never share scratch."""
+    Keyed by the current stream so that tiles processed on different streams never share scratch.
+    A buffer handed out during a CUDA-graph capture stays alive for the rest of the process."""
     dev = torch.cuda.current_device()
     key = (dev, torch.cuda.current_stream().cuda_stream, tag)
     buf = _workspaces.get(key)
     if buf is None or buf.numel() < nbytes:
+        if key in _graph_held:
+            _retired.append(buf)
+            _graph_held.discard(key)
         size = max(int(nbytes * 1.25) + 4096, 1 << 20)
         buf = torch.empty(size, dtype=torch.uint8, device=f"cuda:{dev}")
         _workspaces[key] = buf
+    if torch.cuda.is_current_stream_capturing():
+        _graph_held.add(key)
     return buf
 
 
 def release_workspaces():
+    """Drop the cached scratch buffers, except those a captured CUDA graph still uses (they are retired, not freed)."""
+    _retired.extend(_workspaces[k] for k in _graph_held if k in _workspaces)
+    _graph_held.clear()
     _workspaces.clear()
 
 
