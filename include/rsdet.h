@@ -135,7 +135,24 @@ typedef struct {
 } rsdet_roi_align_cfg;
 
 /* feats[l]: (N,C,H_l,W_l) fp32 (NCHW, or NHWC when channels_last); rois (K,6);
- * out (K,C,ph,pw) fp32 -- always the reference's NCHW-style layout.  levels_out: optional int32 (K). */
+ * out (K,C,ph,pw) fp32 -- always the reference's NCHW-style layout.  levels_out: optional int32 (K).
+ *
+ * Alignment.  fp32 / int32 pointers need only their natural 4-byte alignment; 16-byte alignment selects faster
+ * kernels, never different results beyond what is stated here.  The fast path is C % 4 == 0, sampling_ratio > 0 and
+ * pooled_h * pooled_w * sampling_ratio^2 <= 1024; outside it every call runs the scalar generic kernel.
+ *   forward  feats[l]    NCHW: read by the NCHW->NHWC copy, which uses 16-byte loads where the map allows them.
+ *                        NHWC: the fast kernels read 16-byte vectors from each map's base; if any base is not 16-byte
+ *                        aligned the call runs the generic kernel (same results to the forward tolerance, slower).
+ *            rois        read as scalars.
+ *            out         16-byte aligned: the 7x7 / sampling_ratio 2 / C % 256 == 0 geometry runs the persistent kernel
+ *                        and the kernels write with bulk (TMA) stores; otherwise a one-CTA-per-RoI kernel with scalar
+ *                        stores.  Bit-identical results either way.
+ *            levels_out  written as scalars.
+ *   backward grad_out    16-byte aligned: staged with 16-byte loads; otherwise with scalar loads.  Same results.
+ *            grad_feats  NCHW: written by the NHWC->NCHW copy, which uses 16-byte stores where the map allows them.
+ *                        NHWC: the fast kernel accumulates with 16-byte vector reductions from each map's base; if
+ *                        any base is not 16-byte aligned the call runs the generic kernel (scalar atomics).
+ * Backward results are sums of atomics in an unspecified order: equal across these paths to the backward tolerance. */
 size_t rsdet_roi_align_rotated_workspace_bytes(const rsdet_roi_align_cfg* cfg, int num_rois, int backward);
 int rsdet_roi_align_rotated_forward(const rsdet_roi_align_cfg* cfg, const float* const* feats_host, const float* rois,
                                     int num_rois, float* out, int32_t* levels_out, void* workspace,

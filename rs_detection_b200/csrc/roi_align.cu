@@ -1122,7 +1122,7 @@ roi_align_bwd_kernel(LevelSet L, const float* __restrict__ rois, const int* __re
     // stage this chunk's gradient block [c_local][bin] (= memory order)
     const float* __restrict__ src = grad_out + ((size_t)roi * C + chunk0) * nbins;
     const int total = Qc * 4 * nbins;
-    if ((((size_t)roi * C + chunk0) * nbins & 3) == 0 && (total & 3) == 0) {
+    if ((((size_t)roi * C + chunk0) * nbins & 3) == 0 && (total & 3) == 0 && (((size_t)grad_out) & 15) == 0) {
         float4* s4 = reinterpret_cast<float4*>(s_stage);
         for (int e = tid; e < total / 4; e += kRoiThreads) s4[e] = ldg_cs_v4(src + (size_t)e * 4);
     } else {
@@ -1235,6 +1235,16 @@ static bool fast_path_ok(const rsdet_roi_align_cfg* c) {
            c->pooled_h * c->pooled_w * c->sampling_ratio * c->sampling_ratio <= kMaxSamples;
 }
 
+// The fast kernels read (forward) or accumulate into (backward) a channels-last caller's maps with 16-byte vector
+// accesses from each level's base pointer; a base that is not 16-byte aligned goes to the scalar generic kernel, which
+// addresses NHWC maps directly.  NCHW maps are only read by the transposes, which check alignment themselves.
+static bool nhwc_bases_aligned(const rsdet_roi_align_cfg* c, const float* const* maps) {
+    if (!c->channels_last) return true;
+    for (int l = 0; l < c->num_levels; l++)
+        if (((size_t)maps[l]) & 15) return false;
+    return true;
+}
+
 static int check_cfg(const rsdet_roi_align_cfg* c) {
     if (!c) return RSDET_EINVAL;
     if (c->num_levels < 1 || c->num_levels > RSDET_MAX_LEVELS || c->batch < 1 || c->channels < 1) return RSDET_EINVAL;
@@ -1307,7 +1317,7 @@ extern "C" int rsdet_roi_align_rotated_forward(const rsdet_roi_align_cfg* cfg, c
         if (!feats_host[l]) return RSDET_EINVAL;
     cudaStream_t st = (cudaStream_t)stream;
     LevelSet L = make_levels(cfg);
-    if (!fast_path_ok(cfg)) {
+    if (!fast_path_ok(cfg) || !nhwc_bases_aligned(cfg, feats_host)) {
         GenericMaps M;
         M.channels_last = cfg->channels_last;
         for (int l = 0; l < RSDET_MAX_LEVELS; l++) { M.feat[l] = l < cfg->num_levels ? feats_host[l] : nullptr; M.grad[l] = nullptr; }
@@ -1504,7 +1514,7 @@ extern "C" int rsdet_roi_align_rotated_backward(const rsdet_roi_align_cfg* cfg, 
         if (!grad_feats_host[l]) return RSDET_EINVAL;
     cudaStream_t st = (cudaStream_t)stream;
     LevelSet L = make_levels(cfg);
-    const bool fast = fast_path_ok(cfg);
+    const bool fast = fast_path_ok(cfg) && nhwc_bases_aligned(cfg, grad_feats_host);
     const bool direct = cfg->channels_last || !fast;  // accumulate straight into the caller's buffers
     float* acc[RSDET_MAX_LEVELS];
     if (workspace_bytes < rsdet_roi_align_rotated_workspace_bytes(cfg, num_rois, 1)) return RSDET_EWORKSPACE;
