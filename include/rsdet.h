@@ -162,6 +162,37 @@ int rsdet_roi_align_rotated_backward(const rsdet_roi_align_cfg* cfg, const float
                                      int num_rois, float* const* grad_feats_host, void* workspace,
                                      size_t workspace_bytes, void* stream);
 
+/* Half-precision feature pyramids.  The three calls above are these with RSDET_DTYPE_F32 everywhere.
+ *   feat_dtype      element type of every feats[l] (forward) and grad_feats[l] (backward): F32, F16 or BF16.
+ *   out_dtype       forward output: F32 or feat_dtype.
+ *   grad_out_dtype  backward grad_out: F32 or feat_dtype.
+ * rois stay fp32 and levels_out int32.  Any other dtype, or an out_dtype / grad_out_dtype that is neither F32 nor
+ * feat_dtype, returns RSDET_EINVAL before anything is launched (the workspace query returns 0).
+ * Arithmetic.  Every fp16 / bf16 value converts exactly to fp32; after that the computation is the fp32 one unchanged
+ * (same sample positions, tap lists, tap order and FMA order, fp32 accumulation).  Hence a forward with fp32 output is
+ * bit-identical to the fp32 call on the maps converted to fp32, in the same layout and with buffers of the same
+ * alignment class, and a forward with half output is that result rounded once to nearest-even.  The backward
+ * accumulates in fp32 workspace maps and writes the gradient maps once, rounded to nearest-even; its atomic order is
+ * unspecified as above.  The workspace query counts those accumulators (forward: a half NHWC copy of NCHW maps, half
+ * the bytes of the fp32 copy).
+ * Alignment with 2-byte maps.  The fast kernels read four channels (8 bytes) at a time: channels-last feature maps
+ * (forward) need 8-byte aligned bases, otherwise the call runs the generic kernel.  Half gradient maps are written by a
+ * transpose (NCHW) or a conversion pass (NHWC) from the fp32 accumulators, so no alignment selects a different kernel
+ * for them.  out and grad_out follow the rules above: a 16-byte aligned out takes the persistent kernel and bulk stores;
+ * a grad_out whose base is aligned to four elements (8 bytes when half) is staged with vector loads.  Results do not
+ * depend on alignment beyond what is stated above for fp32. */
+#define RSDET_DTYPE_F32 0
+#define RSDET_DTYPE_F16 1
+#define RSDET_DTYPE_BF16 2
+size_t rsdet_roi_align_rotated_workspace_bytes_typed(const rsdet_roi_align_cfg* cfg, int num_rois, int backward,
+                                                     int feat_dtype);
+int rsdet_roi_align_rotated_forward_typed(const rsdet_roi_align_cfg* cfg, int feat_dtype, const void* const* feats_host,
+                                          const float* rois, int num_rois, int out_dtype, void* out, int32_t* levels_out,
+                                          void* workspace, size_t workspace_bytes, void* stream);
+int rsdet_roi_align_rotated_backward_typed(const rsdet_roi_align_cfg* cfg, int grad_out_dtype, const void* grad_out,
+                                           const float* rois, int num_rois, int feat_dtype, void* const* grad_feats_host,
+                                           void* workspace, size_t workspace_bytes, void* stream);
+
 /* Measurement aid (bench.py's roofline): arm two cudaEvent_t (created with timing enabled by the caller).  The NEXT
  * rsdet_roi_align_rotated_forward call issued by this host thread records `start_event` right before and `stop_event`
  * right after its gather kernel on the call's stream (the geometry / order / transpose kernels of the call stay outside),

@@ -17,6 +17,7 @@ LIB_PATH = os.path.join(HERE, "librsdet.so")
 
 NMS_ROTATED, NMS_ROTATED_GE, NMS_POLY, NMS_MERGE, NMS_HBB, NMS_HBB_P1, NMS_HBB_P1_F64 = 0, 1, 2, 3, 4, 5, 6
 MAX_LEVELS = 8
+DTYPE_F32, DTYPE_F16, DTYPE_BF16 = 0, 1, 2
 
 _vp = C.c_void_p
 
@@ -63,6 +64,11 @@ SIGNATURES = {
                                                   C.c_size_t, _vp]),
     "rsdet_roi_align_rotated_backward": (C.c_int, [C.POINTER(RoiAlignCfg), _vp, _vp, C.c_int, C.POINTER(_vp), _vp,
                                                    C.c_size_t, _vp]),
+    "rsdet_roi_align_rotated_workspace_bytes_typed": (C.c_size_t, [C.POINTER(RoiAlignCfg), C.c_int, C.c_int, C.c_int]),
+    "rsdet_roi_align_rotated_forward_typed": (C.c_int, [C.POINTER(RoiAlignCfg), C.c_int, C.POINTER(_vp), _vp, C.c_int, C.c_int,
+                                                        _vp, _vp, _vp, C.c_size_t, _vp]),
+    "rsdet_roi_align_rotated_backward_typed": (C.c_int, [C.POINTER(RoiAlignCfg), C.c_int, _vp, _vp, C.c_int, C.c_int,
+                                                         C.POINTER(_vp), _vp, C.c_size_t, _vp]),
     "rsdet_oriented_head_results_workspace_bytes": (C.c_size_t, [C.c_int]),
     "rsdet_oriented_head_results": (C.c_int, [_vp, _vp, _vp, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_float), C.POINTER(C.c_float),
                                               C.c_float, C.POINTER(C.c_float), C.c_float, C.c_int, _vp, _vp, _vp, _vp, C.c_size_t,

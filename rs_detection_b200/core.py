@@ -13,8 +13,8 @@ import numpy as np
 import torch
 
 from . import _lib
-from ._lib import (MAX_LEVELS, NMS_HBB, NMS_MERGE, NMS_POLY, NMS_ROTATED, NMS_ROTATED_GE, RoiAlignCfg, check, load, ptr,
-                   stream_ptr, workspace)
+from ._lib import (DTYPE_BF16, DTYPE_F16, DTYPE_F32, MAX_LEVELS, NMS_HBB, NMS_MERGE, NMS_POLY, NMS_ROTATED, NMS_ROTATED_GE,
+                   RoiAlignCfg, check, load, ptr, stream_ptr, workspace)
 
 _F64_KINDS = (NMS_MERGE, NMS_HBB, 6)  # 6 = NMS_HBB_P1_F64 (py_cpu_nms)
 _ROW = {NMS_ROTATED: 5, NMS_ROTATED_GE: 5, NMS_POLY: 8, NMS_MERGE: 8, NMS_HBB: 4, 5: 4, 6: 4}  # 5 = NMS_HBB_P1 (jt.nms)
@@ -271,23 +271,53 @@ def _ptr_array(tensors):
     return arr
 
 
+# element types the RoIAlignRotated entry points read and write natively (include/rsdet.h)
+_ROI_DTYPES = {torch.float32: DTYPE_F32, torch.float16: DTYPE_F16, torch.bfloat16: DTYPE_BF16}
+
+
+def roi_feature_dtype(feats: Sequence[torch.Tensor]) -> torch.dtype:
+    """The element type the kernels read: fp16 and bf16 levels pass through uncast (all levels must then share that
+    dtype, else ValueError); any other dtype is cast to fp32."""
+    dtypes = {f.dtype for f in feats}
+    half = dtypes & {torch.float16, torch.bfloat16}
+    if not half:
+        return torch.float32
+    if len(dtypes) > 1:
+        raise ValueError(f"RoIAlignRotated: feature levels mix dtypes {sorted(str(d) for d in dtypes)}")
+    return half.pop()
+
+
 def roi_align_rotated_forward(cfg: RoiAlignCfg, feats: Sequence[torch.Tensor], rois: torch.Tensor, want_levels: bool = False,
-                              out: Optional[torch.Tensor] = None):
-    feats = [_f32(f) for f in feats]
+                              out: Optional[torch.Tensor] = None, out_dtype: Optional[torch.dtype] = None):
+    """Half-precision levels (fp16 / bf16) are read natively; `out_dtype` is fp32 (None) or the levels' dtype.  An fp32
+    output equals, bit for bit, the call on the levels converted to fp32; a half output is that result rounded once."""
+    fdt = roi_feature_dtype(feats)
+    odt = torch.float32 if out_dtype is None else out_dtype
+    if odt not in (torch.float32, fdt):
+        raise ValueError(f"RoIAlignRotated: out_dtype must be float32 or the features' {fdt}, got {odt}")
+    if out is not None and out.dtype != odt:
+        raise ValueError(f"RoIAlignRotated: out has dtype {out.dtype}, expected {odt}")
+    if fdt == torch.float32:
+        feats = [_f32(f) for f in feats]
+    elif all(f.is_cuda for f in feats):
+        feats = [f.contiguous() for f in feats]
+    else:
+        raise RuntimeError("expected a CUDA tensor (no CPU fallback)")
     r = _f32(rois)
     if r.dim() != 2 or r.shape[1] != 6:
         raise AssertionError("rois must be (K,6)")  # roi_align_rotated_v1.py:306
     K = r.shape[0]
     dev = r.device
     if out is None:
-        out = torch.empty((K, cfg.channels, cfg.pooled_h, cfg.pooled_w), dtype=torch.float32, device=dev)
+        out = torch.empty((K, cfg.channels, cfg.pooled_h, cfg.pooled_w), dtype=odt, device=dev)
     lv = torch.empty((K,), dtype=torch.int32, device=dev) if want_levels else None
     if K:
         L = load()
-        wsb = L.rsdet_roi_align_rotated_workspace_bytes(C.byref(cfg), K, 0)
+        wsb = L.rsdet_roi_align_rotated_workspace_bytes_typed(C.byref(cfg), K, 0, _ROI_DTYPES[fdt])
         ws = workspace(wsb, "roi")
-        check(L.rsdet_roi_align_rotated_forward(C.byref(cfg), _ptr_array(feats), ptr(r), K, ptr(out), ptr(lv), ptr(ws),
-                                                ws.numel(), stream_ptr()), "roi_align_rotated_forward")
+        check(L.rsdet_roi_align_rotated_forward_typed(C.byref(cfg), _ROI_DTYPES[fdt], _ptr_array(feats), ptr(r), K,
+                                                      _ROI_DTYPES[odt], ptr(out), ptr(lv), ptr(ws), ws.numel(), stream_ptr()),
+              "roi_align_rotated_forward")
     return (out, lv) if want_levels else out
 
 
@@ -297,25 +327,36 @@ def roi_gather_kernel_ms(cfg: RoiAlignCfg, feats: Sequence[torch.Tensor], rois: 
     a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     a.record(); b.record()                       # materialise the cudaEvent_t handles
     check(load().rsdet_roi_align_profile_events(C.c_void_p(a.cuda_event), C.c_void_p(b.cuda_event)), "roi_align_profile_events")
-    roi_align_rotated_forward(cfg, feats, rois, out=out)
+    roi_align_rotated_forward(cfg, feats, rois, out=out, out_dtype=out.dtype)
     torch.cuda.synchronize()
     return a.elapsed_time(b)
 
 
-def roi_align_rotated_backward(cfg: RoiAlignCfg, grad_out: torch.Tensor, rois: torch.Tensor, feat_shapes):
-    g = _f32(grad_out)
+def roi_align_rotated_backward(cfg: RoiAlignCfg, grad_out: torch.Tensor, rois: torch.Tensor, feat_shapes,
+                               feat_dtype: torch.dtype = torch.float32):
+    """-> gradient maps in `feat_dtype` (fp32, fp16 or bf16; accumulated in fp32, rounded once).  A grad_out in fp32 or
+    in `feat_dtype` is read natively, any other dtype is cast to fp32."""
+    if feat_dtype not in _ROI_DTYPES:
+        raise ValueError(f"RoIAlignRotated: gradient maps can be float32, float16 or bfloat16, not {feat_dtype}")
+    if grad_out.dtype in (torch.float32, feat_dtype):
+        if not grad_out.is_cuda:
+            raise RuntimeError("expected a CUDA tensor (no CPU fallback)")
+        g = grad_out.contiguous()
+    else:
+        g = _f32(grad_out)
     r = _f32(rois)
     K = r.shape[0]
     dev = r.device
     grads = []
     for l, shp in enumerate(feat_shapes):
         n, c, h, w = [int(v) for v in shp]
-        grads.append(torch.empty((n, h, w, c) if cfg.channels_last else (n, c, h, w), dtype=torch.float32, device=dev))
+        grads.append(torch.empty((n, h, w, c) if cfg.channels_last else (n, c, h, w), dtype=feat_dtype, device=dev))
     L = load()
-    wsb = L.rsdet_roi_align_rotated_workspace_bytes(C.byref(cfg), K, 1)
+    fdt = _ROI_DTYPES[feat_dtype]
+    wsb = L.rsdet_roi_align_rotated_workspace_bytes_typed(C.byref(cfg), K, 1, fdt)
     ws = workspace(wsb, "roi")
-    check(L.rsdet_roi_align_rotated_backward(C.byref(cfg), ptr(g), ptr(r), K, _ptr_array(grads), ptr(ws), ws.numel(),
-                                             stream_ptr()), "roi_align_rotated_backward")
+    check(L.rsdet_roi_align_rotated_backward_typed(C.byref(cfg), _ROI_DTYPES[g.dtype], ptr(g), ptr(r), K, fdt, _ptr_array(grads),
+                                                   ptr(ws), ws.numel(), stream_ptr()), "roi_align_rotated_backward")
     return grads
 
 

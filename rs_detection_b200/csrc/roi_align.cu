@@ -25,10 +25,18 @@
 //
 // Sample coordinates are computed with explicitly un-contracted IEEE operations in the reference's
 // order: the validity test `y < -1 || y > H` is discontinuous, so coordinates must not drift.
+//
+// Element types (include/rsdet.h): feature maps, grad_out and gradient maps may be fp16 or bf16 as well as fp32.  Every
+// kernel below is templated on them; a half value is converted exactly to fp32 where it is read, the arithmetic is the
+// fp32 arithmetic unchanged, and a half result is rounded once, to nearest-even, where it is stored.  Four consecutive
+// channels are the unit of every vector access: a float4 (16 bytes) or four 2-byte values (8 bytes).
 #include <cuda.h>
+#include <cuda_bf16.h>
+#include <cuda_fp16.h>
 
 #include <cstdlib>
 #include <mutex>
+#include <type_traits>
 
 #include "common.cuh"
 
@@ -37,8 +45,53 @@ namespace rsdet {
 constexpr int kRoiThreads = 256;
 constexpr int kMaxSamples = 1024;  // fast path: pooled_h*pooled_w*grid_h*grid_w
 
+// ---------------------------------------------------------------------------------- element types
+template <typename T> struct Quad { using V = float4; };            // four channels as one vector
+template <> struct Quad<__half> { using V = uint2; };
+template <> struct Quad<__nv_bfloat16> { using V = uint2; };
+template <typename T> constexpr bool kIsF32 = std::is_same<T, float>::value;
+
+__device__ __forceinline__ float to_f32(float v) { return v; }
+__device__ __forceinline__ float to_f32(__half v) { return __half2float(v); }
+__device__ __forceinline__ float to_f32(__nv_bfloat16 v) { return __bfloat162float(v); }
+template <typename T> __device__ __forceinline__ T from_f32(float v) {
+    if constexpr (std::is_same<T, __half>::value) return __float2half_rn(v);
+    else if constexpr (std::is_same<T, __nv_bfloat16>::value) return __float2bfloat16_rn(v);
+    else return v;
+}
+template <typename T> __device__ __forceinline__ float4 unpack4(uint2 u) {   // four 2-byte values -> fp32, exact
+    if constexpr (std::is_same<T, __half>::value) {
+        const float2 a = __half22float2(*reinterpret_cast<const __half2*>(&u.x));
+        const float2 b = __half22float2(*reinterpret_cast<const __half2*>(&u.y));
+        return make_float4(a.x, a.y, b.x, b.y);
+    } else {
+        return make_float4(__uint_as_float(u.x << 16), __uint_as_float(u.x & 0xffff0000u),
+                           __uint_as_float(u.y << 16), __uint_as_float(u.y & 0xffff0000u));
+    }
+}
+template <typename T> __device__ __forceinline__ uint2 pack4(float4 v) {     // fp32 -> four 2-byte values, nearest-even
+    uint2 u;
+    if constexpr (std::is_same<T, __half>::value) {
+        const __half2 a = __floats2half2_rn(v.x, v.y), b = __floats2half2_rn(v.z, v.w);
+        u.x = *reinterpret_cast<const unsigned*>(&a); u.y = *reinterpret_cast<const unsigned*>(&b);
+    } else {
+        const __nv_bfloat162 a = __floats2bfloat162_rn(v.x, v.y), b = __floats2bfloat162_rn(v.z, v.w);
+        u.x = *reinterpret_cast<const unsigned*>(&a); u.y = *reinterpret_cast<const unsigned*>(&b);
+    }
+    return u;
+}
+// read-only 4-channel load / 4-channel store (p aligned to 4 * sizeof(T))
+template <typename T> __device__ __forceinline__ float4 ldg4_ro(const T* p) {
+    if constexpr (kIsF32<T>) return __ldg(reinterpret_cast<const float4*>(p));
+    else return unpack4<T>(__ldg(reinterpret_cast<const uint2*>(p)));
+}
+template <typename T> __device__ __forceinline__ void st4(T* p, float4 v) {
+    if constexpr (kIsF32<T>) *reinterpret_cast<float4*>(p) = v;
+    else *reinterpret_cast<uint2*>(p) = pack4<T>(v);
+}
+
 struct LevelSet {
-    const float* feat[RSDET_MAX_LEVELS];  // channels-last maps
+    const float* feat[RSDET_MAX_LEVELS];  // channels-last maps; their element type is the kernel's T (feat_base)
     float* grad[RSDET_MAX_LEVELS];
     int H[RSDET_MAX_LEVELS], W[RSDET_MAX_LEVELS];
     float scale[RSDET_MAX_LEVELS];
@@ -49,21 +102,25 @@ struct LevelSet {
     unsigned dbg_mask;  // profiling aid (RSDET_ROI_DBG_MASK, RSDET_TUNING builds only): tap offsets are ANDed with it (shrinks the gather's footprint)
     int dbg_skip_main;  // profiling aid (RSDET_ROI_DBG_SKIP_MAIN=1, RSDET_TUNING builds only): tap lists are built, then treated as empty
 };
+template <typename T> __device__ __forceinline__ const T* feat_base(const LevelSet& L, int level) {
+    return reinterpret_cast<const T*>(L.feat[level]);
+}
 
 // ---------------------------------------------------------------------------------- transposes
-// (N, C, HW) <-> (N, HW, C), 64x64 tiles through padded shared memory.
+// (N, C, HW) <-> (N, HW, C), 64x64 tiles through padded shared memory; source elements S, destination elements D
+// (fp32 tile: a half source converts exactly, a half destination rounds to nearest-even).
 struct TransposeJob {
-    const float* src[RSDET_MAX_LEVELS];
-    float* dst[RSDET_MAX_LEVELS];
+    const void* src[RSDET_MAX_LEVELS];
+    void* dst[RSDET_MAX_LEVELS];
     int HW[RSDET_MAX_LEVELS];
     int tile_begin[RSDET_MAX_LEVELS + 1];  // prefix of tiles over levels
     int num_levels, N, C;
 };
 
-// 64(channels) x 64(pixels) tiles, 16-byte global accesses on both sides: a thread reads a float4 along the
-// source's contiguous dimension, scatters it into a padded shared tile, and writes a float4 along the
-// destination's contiguous dimension.  Falls back to scalar accesses at ragged edges / unaligned bases.
-template <bool TO_NHWC>
+// 64(channels) x 64(pixels) tiles, 4-channel vector accesses on both sides (16 bytes for fp32, 8 for half): a thread
+// reads four elements along the source's contiguous dimension, scatters them into a padded shared tile, and writes four
+// along the destination's contiguous dimension.  Falls back to scalar accesses at ragged edges / unaligned bases.
+template <typename S, typename D, bool TO_NHWC>
 __device__ __forceinline__ void transpose_tile(const TransposeJob& job, int t, float (*tile)[65]) {
     int l = 0;
     while (l + 1 < job.num_levels && t >= job.tile_begin[l + 1]) l++;
@@ -73,26 +130,26 @@ __device__ __forceinline__ void transpose_tile(const TransposeJob& job, int t, f
     const int n = t / (tiles_hw * tiles_c);
     const int r = t % (tiles_hw * tiles_c);
     const int hw0 = (r % tiles_hw) * 64, c0 = (r / tiles_hw) * 64;
-    const float* src = job.src[l] + (size_t)n * C * HW;
-    float* dst = job.dst[l] + (size_t)n * C * HW;
+    const S* src = static_cast<const S*>(job.src[l]) + (size_t)n * C * HW;
+    D* dst = static_cast<D*>(job.dst[l]) + (size_t)n * C * HW;
     const int tid = threadIdx.x;
     // source: rows of `SR` index, contiguous along `SC`; destination the other way round
     const int srcRows = TO_NHWC ? C : HW, srcCols = TO_NHWC ? HW : C;      // src[row * srcCols + col]
     const int r0 = TO_NHWC ? c0 : hw0, q0 = TO_NHWC ? hw0 : c0;            // tile origin (row, col) in the source
-    const bool vec_in = (srcCols & 3) == 0 && ((size_t)src & 15) == 0;
-    const bool vec_out = (srcRows & 3) == 0 && ((size_t)dst & 15) == 0;
+    const bool vec_in = (srcCols & 3) == 0 && ((size_t)src & (4 * sizeof(S) - 1)) == 0;
+    const bool vec_out = (srcRows & 3) == 0 && ((size_t)dst & (4 * sizeof(D) - 1)) == 0;
 #pragma unroll
     for (int k = 0; k < 4; k++) {
-        const int idx = tid + 256 * k;            // 1024 float4 slots: 64 rows x 16 float4
+        const int idx = tid + 256 * k;            // 1024 4-element slots: 64 rows x 16 slots
         const int rr = idx >> 4, cc = (idx & 15) * 4;
         const int gr = r0 + rr, gc = q0 + cc;
         if (gr < srcRows) {
             if (vec_in && gc + 3 < srcCols) {
-                const float4 v = __ldg(reinterpret_cast<const float4*>(src + (size_t)gr * srcCols + gc));
+                const float4 v = ldg4_ro(src + (size_t)gr * srcCols + gc);
                 tile[rr][cc] = v.x; tile[rr][cc + 1] = v.y; tile[rr][cc + 2] = v.z; tile[rr][cc + 3] = v.w;
             } else {
                 for (int e = 0; e < 4; e++)
-                    if (gc + e < srcCols) tile[rr][cc + e] = __ldg(src + (size_t)gr * srcCols + gc + e);
+                    if (gc + e < srcCols) tile[rr][cc + e] = to_f32(__ldg(src + (size_t)gr * srcCols + gc + e));
             }
         }
     }
@@ -106,19 +163,44 @@ __device__ __forceinline__ void transpose_tile(const TransposeJob& job, int t, f
         if (gc < srcCols) {
             if (vec_out && gr + 3 < srcRows) {
                 const float4 v = make_float4(tile[rr][cc], tile[rr + 1][cc], tile[rr + 2][cc], tile[rr + 3][cc]);
-                *reinterpret_cast<float4*>(dst + (size_t)gc * srcRows + gr) = v;
+                st4(dst + (size_t)gc * srcRows + gr, v);
             } else {
                 for (int e = 0; e < 4; e++)
-                    if (gr + e < srcRows) dst[(size_t)gc * srcRows + gr + e] = tile[rr + e][cc];
+                    if (gr + e < srcRows) dst[(size_t)gc * srcRows + gr + e] = from_f32<D>(tile[rr + e][cc]);
             }
         }
     }
 }
 
-template <bool TO_NHWC>
+template <typename S, typename D, bool TO_NHWC>
 __global__ void __launch_bounds__(256) transpose_kernel(TransposeJob job) {
     __shared__ float tile[64][65];
-    transpose_tile<TO_NHWC>(job, blockIdx.x, tile);
+    transpose_tile<S, D, TO_NHWC>(job, blockIdx.x, tile);
+}
+
+// fp32 accumulators -> a caller's half gradient maps in the same layout, rounded to nearest-even (blockIdx.y = level).
+// Four elements per step: a 16-byte load (the accumulators are workspace slices, 256-byte aligned) and an 8-byte store
+// when the destination allows it, scalar stores otherwise.
+struct ConvertJob {
+    const float* src[RSDET_MAX_LEVELS];
+    void* dst[RSDET_MAX_LEVELS];
+    size_t n[RSDET_MAX_LEVELS];
+};
+template <typename D>
+__global__ void __launch_bounds__(256) convert_maps_kernel(ConvertJob job) {
+    const float* __restrict__ src = job.src[blockIdx.y];
+    D* __restrict__ dst = static_cast<D*>(job.dst[blockIdx.y]);
+    const size_t n = job.n[blockIdx.y];
+    const bool vec = ((size_t)dst & (4 * sizeof(D) - 1)) == 0;
+    for (size_t i = 4 * ((size_t)blockIdx.x * blockDim.x + threadIdx.x); i < n; i += 4 * (size_t)gridDim.x * blockDim.x) {
+        if (i + 3 < n) {
+            const float4 v = __ldcs(reinterpret_cast<const float4*>(src + i));
+            if (vec) st4(dst + i, v);
+            else { dst[i] = from_f32<D>(v.x); dst[i + 1] = from_f32<D>(v.y); dst[i + 2] = from_f32<D>(v.z); dst[i + 3] = from_f32<D>(v.w); }
+        } else {
+            for (size_t e = i; e < n; e++) dst[e] = from_f32<D>(src[e]);
+        }
+    }
 }
 
 struct LevelSet;
@@ -133,7 +215,8 @@ struct PrepArgs {                 // order block riding along with the NCHW->NHW
     int32_t* levels_out = nullptr;
     unsigned* counter = nullptr;
 };
-static int launch_transpose(bool to_nhwc, const float* const* src, float* const* dst, const int* H, const int* W, int L, int N,
+template <typename S, typename D>
+static int launch_transpose(bool to_nhwc, const S* const* src, D* const* dst, const int* H, const int* W, int L, int N,
                             int C, cudaStream_t st, const PrepArgs* prep = nullptr);
 
 // ---------------------------------------------------------------------------------- geometry
@@ -241,6 +324,55 @@ __device__ __forceinline__ float4 ldg_flavour_v4(const float* p) {
     else asm volatile("ld.global.nc.v4.f32 {%0,%1,%2,%3}, [%4];" : "=f"(r.x), "=f"(r.y), "=f"(r.z), "=f"(r.w) : "l"(p));
     return r;
 }
+// base + off * sizeof(Quad<T>::V) as ONE mad.wide.u32: tap offsets count 4-channel units of a channels-last map
+template <typename T>
+__device__ __forceinline__ const T* quad_ptr(const typename Quad<T>::V* base, unsigned off) {
+    unsigned long long a;
+    asm("mad.wide.u32 %0, %1, %2, %3;" : "=l"(a) : "r"(off), "n"((int)sizeof(typename Quad<T>::V)), "l"((unsigned long long)base));
+    return reinterpret_cast<const T*>(a);
+}
+// four channels at p as fp32 through the non-coherent path: one 16-byte load (fp32, FLAVOUR as above) or one 8-byte load
+template <typename T, int FLAVOUR = 0>
+__device__ __forceinline__ float4 ldg4(const T* p) {
+    if constexpr (kIsF32<T>) {
+        return ldg_flavour_v4<FLAVOUR>(p);
+    } else {
+        uint2 u;
+        asm volatile("ld.global.nc.v2.b32 {%0,%1}, [%2];" : "=r"(u.x), "=r"(u.y) : "l"(p));
+        return unpack4<T>(u);
+    }
+}
+// the same load without the conversion (raw vector), and the conversion: lets a loop keep 2-byte values in flight
+template <typename T, int FLAVOUR = 0>
+__device__ __forceinline__ typename Quad<T>::V ldg4_raw(const T* p) {
+    if constexpr (kIsF32<T>) {
+        return ldg_flavour_v4<FLAVOUR>(p);
+    } else {
+        uint2 u;
+        asm volatile("ld.global.nc.v2.b32 {%0,%1}, [%2];" : "=r"(u.x), "=r"(u.y) : "l"(p));
+        return u;
+    }
+}
+template <typename T> __device__ __forceinline__ decltype(auto) quad_f32(const typename Quad<T>::V& v) {
+    if constexpr (kIsF32<T>) return (v);    // a reference: the fp32 kernels compile exactly as without this step
+    else return unpack4<T>(v);
+}
+__device__ __forceinline__ float4 ldg_cs_v4(const float* p);
+template <typename T>
+__device__ __forceinline__ float4 ldcs4(const T* p) {     // streaming 4-channel load
+    if constexpr (kIsF32<T>) {
+        return ldg_cs_v4(p);
+    } else {
+        uint2 u;
+        asm volatile("ld.global.cs.v2.b32 {%0,%1}, [%2];" : "=r"(u.x), "=r"(u.y) : "l"(p));
+        return unpack4<T>(u);
+    }
+}
+template <typename T>
+__device__ __forceinline__ void stcs1(T* p, T v) {           // streaming scalar store
+    if constexpr (kIsF32<T>) __stcs(p, v);
+    else asm volatile("st.global.cs.b16 [%0], %1;" ::"l"(p), "h"(*reinterpret_cast<const unsigned short*>(&v)) : "memory");
+}
 __device__ __forceinline__ void stg_cs_v4(float* p, float4 v) {
     asm volatile("st.global.cs.v4.f32 [%0], {%1,%2,%3,%4};" ::"l"(p), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w) : "memory");
 }
@@ -252,7 +384,7 @@ __device__ __forceinline__ float4 ldg_cs_v4(const float* p) {
 // shared -> global bulk copy (cp.async.bulk, SASS UBLKCP) with an evict-first L2 policy: the output stream must
 // not push the feature pyramid out of L2.  Returns once the source has been read (shared memory may be reused
 // or the CTA may exit); global visibility follows at kernel end.
-__device__ __forceinline__ void bulk_store_evict_first(float* dst, const float* src_smem, unsigned bytes) {
+__device__ __forceinline__ void bulk_store_evict_first(void* dst, const void* src_smem, unsigned bytes) {
     unsigned long long pol;
     asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(pol));
     asm volatile("cp.async.bulk.global.shared::cta.bulk_group.L2::cache_hint [%0], [%1], %2, %3;"
@@ -446,6 +578,7 @@ __global__ void __launch_bounds__(1024) roi_prep_kernel(LevelSet L, const float*
 }
 
 // NCHW callers: the pyramid transpose with the order block riding along as block 0
+template <typename T>
 __global__ void __launch_bounds__(256) transpose_prep_kernel(TransposeJob job, LevelSet L, const float* __restrict__ rois, int K,
                                                              int* __restrict__ order, RoiGeom* __restrict__ geoms,
                                                              int32_t* __restrict__ levels_out, unsigned* __restrict__ counter,
@@ -465,10 +598,12 @@ __global__ void __launch_bounds__(256) transpose_prep_kernel(TransposeJob job, L
         roi_geometry_by_index(L, rois, K, ((int)blockIdx.x - 1) * 256 + threadIdx.x, geoms, levels_out);
         return;
     }
-    transpose_tile<true>(job, blockIdx.x - 1 - geom_blocks, tile);
+    transpose_tile<T, T, true>(job, blockIdx.x - 1 - geom_blocks, tile);
 }
 
-static int launch_transpose(bool to_nhwc, const float* const* src, float* const* dst, const int* H, const int* W, int L, int N,
+// S == D: either direction (NCHW -> NHWC may carry the prep blocks); S != D: NHWC fp32 accumulators -> NCHW half maps
+template <typename S, typename D>
+static int launch_transpose(bool to_nhwc, const S* const* src, D* const* dst, const int* H, const int* W, int L, int N,
                             int C, cudaStream_t st, const PrepArgs* prep) {
     TransposeJob job;
     job.num_levels = L; job.N = N; job.C = C;
@@ -479,16 +614,22 @@ static int launch_transpose(bool to_nhwc, const float* const* src, float* const*
         total += N * ceil_div(job.HW[l], 64) * ceil_div(C, 64);
     }
     job.tile_begin[L] = total;
-    if (prep && to_nhwc) {
-        const int geom_blocks = prep->geoms ? ceil_div(prep->K, 256) : 0;
-        transpose_prep_kernel<<<total + 1 + geom_blocks, 256, 0, st>>>(job, *prep->L, prep->rois, prep->K, prep->order, prep->geoms,
-                                                                        prep->levels_out, prep->counter, geom_blocks);
-        count_launch();
-        return cuda_status();
+    if constexpr (std::is_same<S, D>::value) {
+        if (prep && to_nhwc) {
+            const int geom_blocks = prep->geoms ? ceil_div(prep->K, 256) : 0;
+            transpose_prep_kernel<S><<<total + 1 + geom_blocks, 256, 0, st>>>(job, *prep->L, prep->rois, prep->K, prep->order,
+                                                                               prep->geoms, prep->levels_out, prep->counter,
+                                                                               geom_blocks);
+            count_launch();
+            return cuda_status();
+        }
+        if (total == 0) return RSDET_OK;
+        if (to_nhwc) transpose_kernel<S, D, true><<<total, 256, 0, st>>>(job);
+        else transpose_kernel<S, D, false><<<total, 256, 0, st>>>(job);
+    } else {
+        if (to_nhwc || total == 0) return to_nhwc ? RSDET_EINVAL : RSDET_OK;
+        transpose_kernel<S, D, false><<<total, 256, 0, st>>>(job);
     }
-    if (total == 0) return RSDET_OK;
-    if (to_nhwc) transpose_kernel<true><<<total, 256, 0, st>>>(job);
-    else transpose_kernel<false><<<total, 256, 0, st>>>(job);
     count_launch();
     return cuda_status();
 }
@@ -667,10 +808,10 @@ __device__ __forceinline__ float4 unrot4(float4 v, int o) { return rot4(v, (4 - 
 // One CTA per (RoI, chunk of up to 64 channel quads), thread = (channel quad(s), bin group).  QPT = 2:
 // the second channel quad is an immediate +512 B off the same address.  Launch bounds for THREE CTAs per SM: the driver then
 // picks the 196 KB carve-out (60 KB of L1 instead of 28) -- 143.2 -> 131.9 us per bench tile (profiles/README.md, third pass).
-template <int QPT>
+template <int QPT, typename T = float, typename O = float>   // T: feature elements, O: output elements
 __global__ void __launch_bounds__(kRoiThreads, 3)
 roi_align_fwd_kernel(LevelSet L, const float* __restrict__ rois, const int* __restrict__ order, const RoiGeom* __restrict__ geoms,
-                     int K, float* __restrict__ out, int32_t* __restrict__ levels_out) {
+                     int K, O* __restrict__ out, int32_t* __restrict__ levels_out) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int roi = order ? order[blockIdx.x] : blockIdx.x;
     const int tid = threadIdx.x;
@@ -684,7 +825,7 @@ roi_align_fwd_kernel(LevelSet L, const float* __restrict__ rois, const int* __re
     // smem: [merged lists: nbins*cap int2][counts: nbins int, padded][staging [c][bin] | phase-A scratch]
     int2* s_list = reinterpret_cast<int2*>(smem_raw);
     int* s_cnt = reinterpret_cast<int*>(smem_raw + list_bytes(nbins, cap));
-    float* s_stage = reinterpret_cast<float*>(smem_raw + list_bytes(nbins, cap) + ((nbins * 4 + 15) & ~15));
+    O* s_stage = reinterpret_cast<O*>(smem_raw + list_bytes(nbins, cap) + ((nbins * 4 + 15) & ~15));
     __shared__ RoiGeom s_g;
 
     if (!geoms) {
@@ -697,18 +838,18 @@ roi_align_fwd_kernel(LevelSet L, const float* __restrict__ rois, const int* __re
     const RoiGeom g = geoms ? geoms[roi] : s_g;
     const int H = L.H[g.level], W = L.W[g.level];
 #ifdef RSDET_TUNING   // A/B builds: phase-cost measurements (lists only / nothing); the shipped kernel has no such switch
-    if (L.dbg_skip_main < 2) build_tap_lists(g, L, H, W, s_list, s_cnt, s_stage, C >> 2, 0);
+    if (L.dbg_skip_main < 2) build_tap_lists(g, L, H, W, s_list, s_cnt, reinterpret_cast<float*>(s_stage), C >> 2, 0);
     if (L.dbg_skip_main) { for (int b = tid; b < nbins; b += kRoiThreads) s_cnt[b] = 0; __syncthreads(); }
 #else
-    build_tap_lists(g, L, H, W, s_list, s_cnt, s_stage, C >> 2, 0);   // the scratch is dead after its final barrier
+    build_tap_lists(g, L, H, W, s_list, s_cnt, reinterpret_cast<float*>(s_stage), C >> 2, 0);   // the scratch is dead after its final barrier
 #endif
 
     const int lanes = QPT == 2 ? 32 : Qc;                  // threads per bin group
     const int groups = kRoiThreads / lanes;
     const int cq = tid % lanes, grp = tid / lanes;
     const int oct = (cq >> 3) & 3;
-    const float4* __restrict__ feat =
-        reinterpret_cast<const float4*>(L.feat[g.level] + (size_t)g.batch * H * W * C + chunk0) + cq;
+    const typename Quad<T>::V* __restrict__ feat =
+        reinterpret_cast<const typename Quad<T>::V*>(feat_base<T>(L, g.level) + (size_t)g.batch * H * W * C + chunk0) + cq;
     const bool pow2 = (spb & (spb - 1)) == 0;
     const float count = (float)max(spb, 1), inv_count = 1.f / count;
     if (grp < groups) {
@@ -731,7 +872,7 @@ roi_align_fwd_kernel(LevelSet L, const float* __restrict__ rois, const int* __re
                 for (int k = 0; k < 4; k++)
                     if (e + k < cnt) {
 #pragma unroll
-                        for (int u = 0; u < QPT; u++) v[u][k] = ldg_nc_v4(tap_ptr(feat, (unsigned)en[k].x) + u * 128);
+                        for (int u = 0; u < QPT; u++) v[u][k] = ldg4(quad_ptr<T>(feat, (unsigned)en[k].x) + u * 128);
                     }
 #pragma unroll
                 for (int k = 0; k < 4; k++)
@@ -753,10 +894,10 @@ roi_align_fwd_kernel(LevelSet L, const float* __restrict__ rois, const int* __re
                 else { acc[u].x /= count; acc[u].y /= count; acc[u].z /= count; acc[u].w /= count; }
                 const int c0 = (cq + u * 32) * 4;
                 const float4 r = rot4(acc[u], oct);
-                s_stage[(c0 + ((0 + oct) & 3)) * nbins + b] = r.x;
-                s_stage[(c0 + ((1 + oct) & 3)) * nbins + b] = r.y;
-                s_stage[(c0 + ((2 + oct) & 3)) * nbins + b] = r.z;
-                s_stage[(c0 + ((3 + oct) & 3)) * nbins + b] = r.w;
+                s_stage[(c0 + ((0 + oct) & 3)) * nbins + b] = from_f32<O>(r.x);
+                s_stage[(c0 + ((1 + oct) & 3)) * nbins + b] = from_f32<O>(r.y);
+                s_stage[(c0 + ((2 + oct) & 3)) * nbins + b] = from_f32<O>(r.z);
+                s_stage[(c0 + ((3 + oct) & 3)) * nbins + b] = from_f32<O>(r.w);
             }
         }
     }
@@ -764,12 +905,13 @@ roi_align_fwd_kernel(LevelSet L, const float* __restrict__ rois, const int* __re
     __syncthreads();
     // the staged block IS the output block of this (roi, chunk): one bulk copy shared -> global (TMA) when it is
     // 16-byte aligned, else a coalesced copy with streaming stores
-    float* __restrict__ dst = out + ((size_t)roi * C + chunk0) * nbins;
+    O* __restrict__ dst = out + ((size_t)roi * C + chunk0) * nbins;
     const int total = Qc * 4 * nbins;
-    if ((((size_t)roi * C + chunk0) * nbins & 3) == 0 && (total & 3) == 0 && (((size_t)out) & 15) == 0) {
-        if (tid == 0) bulk_store_evict_first(dst, s_stage, (unsigned)total * 4u);
+    constexpr int kVec = 16 / sizeof(O);                   // elements per 16 bytes
+    if ((((size_t)roi * C + chunk0) * nbins % kVec) == 0 && (total % kVec) == 0 && (((size_t)out) & 15) == 0) {
+        if (tid == 0) bulk_store_evict_first(dst, s_stage, (unsigned)(total * sizeof(O)));
     } else {
-        for (int e = tid; e < total; e += kRoiThreads) __stcs(dst + e, s_stage[e]);
+        for (int e = tid; e < total; e += kRoiThreads) stcs1(dst + e, s_stage[e]);
     }
 }
 
@@ -787,45 +929,47 @@ roi_align_fwd_kernel(LevelSet L, const float* __restrict__ rois, const int* __re
 //   * a CTA starts from the geometry record in processing order (one global round trip instead of order -> geoms).
 // Arithmetic and tap order are those of roi_align_fwd_kernel<2>; results are bit-identical.
 constexpr size_t kStage77Offset = (8 * 49 * 17 + 15 + ((49 * 4 + 15) & ~15) + 127) & ~(size_t)127;   // lists + counts, rounded up
-template <int WARPS, int FLAVOUR = 0, int MINB = 4>
+template <int WARPS, int FLAVOUR = 0, int MINB = 4, typename T = float, typename O = float>
 __global__ void __launch_bounds__(32 * WARPS, MINB)
-roi_align_fwd77_kernel(LevelSet L, const RoiGeom* __restrict__ gsorted, int K, float* __restrict__ out) {
+roi_align_fwd77_kernel(LevelSet L, const RoiGeom* __restrict__ gsorted, int K, O* __restrict__ out) {
     constexpr int NB = 49, CAP = 16, PITCH = CAP + 1, THREADS = 32 * WARPS;
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     int2* s_list = reinterpret_cast<int2*>(smem_raw);
     int* s_cnt = reinterpret_cast<int*>(smem_raw + list_bytes(NB, CAP));
     // staging block on a 128-byte boundary: the bulk store reads it in 128-byte lines
-    float* s_stage = reinterpret_cast<float*>(smem_raw + kStage77Offset);
+    O* s_stage = reinterpret_cast<O*>(smem_raw + kStage77Offset);
     RoiGeom g = gsorted[blockIdx.x];
     const int roi = g.gh;                                   // processing-order record: gh carries the RoI index
     g.gh = 2; g.gw = 2;
     const int C = L.C, chunk0 = blockIdx.y * 256;
     const int H = L.H[g.level], W = L.W[g.level];
-    build_tap_lists<THREADS, true>(g, L, H, W, s_list, s_cnt, s_stage, C >> 2, 0);   // the scratch (staging block) is dead after its final barrier
+    build_tap_lists<THREADS, true>(g, L, H, W, s_list, s_cnt, reinterpret_cast<float*>(s_stage), C >> 2, 0);   // the scratch (staging block) is dead after its final barrier
 
-    const float4* __restrict__ feat =
-        reinterpret_cast<const float4*>(L.feat[g.level] + (size_t)g.batch * H * W * C + chunk0) + lane;
+    const typename Quad<T>::V* __restrict__ feat =
+        reinterpret_cast<const typename Quad<T>::V*>(feat_base<T>(L, g.level) + (size_t)g.batch * H * W * C + chunk0) + lane;
     const int oct = (lane >> 3) & 3;
     // staging slot of component j of a quad: channel 4*lane + ((j + oct) & 3) (conflict-free, see rot4); computed per bin
     // instead of held in four registers
-    float* const sbase = s_stage + lane * 4 * NB;
+    O* const sbase = s_stage + lane * 4 * NB;
     auto stage = [&](float4 a0, float4 a1, int b) {
         a0.x *= 0.25f; a0.y *= 0.25f; a0.z *= 0.25f; a0.w *= 0.25f;   // output_val /= count (:143), count = 4: exact
         a1.x *= 0.25f; a1.y *= 0.25f; a1.z *= 0.25f; a1.w *= 0.25f;
         const float4 r0 = rot4(a0, oct), r1 = rot4(a1, oct);
-        float* const sb = sbase + b;
-        float* const q0 = sb + ((0 + oct) & 3) * NB;
-        float* const q1 = sb + ((1 + oct) & 3) * NB;
-        float* const q2 = sb + ((2 + oct) & 3) * NB;
-        float* const q3 = sb + ((3 + oct) & 3) * NB;
-        q0[0] = r0.x; q1[0] = r0.y; q2[0] = r0.z; q3[0] = r0.w;
-        q0[128 * NB] = r1.x; q1[128 * NB] = r1.y; q2[128 * NB] = r1.z; q3[128 * NB] = r1.w;
+        O* const sb = sbase + b;
+        O* const q0 = sb + ((0 + oct) & 3) * NB;
+        O* const q1 = sb + ((1 + oct) & 3) * NB;
+        O* const q2 = sb + ((2 + oct) & 3) * NB;
+        O* const q3 = sb + ((3 + oct) & 3) * NB;
+        q0[0] = from_f32<O>(r0.x); q1[0] = from_f32<O>(r0.y); q2[0] = from_f32<O>(r0.z); q3[0] = from_f32<O>(r0.w);
+        q0[128 * NB] = from_f32<O>(r1.x); q1[128 * NB] = from_f32<O>(r1.y); q2[128 * NB] = from_f32<O>(r1.z); q3[128 * NB] = from_f32<O>(r1.w);
     };
     // one batch: up to four taps = eight 16-byte loads in flight per thread; the list entries of the following batch
     // (same bin, or the first four of this warp's next bin) are read while the loads fly
-#define RSDET_ACC(P, WT, VA, VB)                                                                                        \
+#define RSDET_ACC(P, WT, RA, RB)                                                                                        \
         if (P) {                                                                                                        \
+            const auto& VA = quad_f32<T>(RA);                                                                           \
+            const auto& VB = quad_f32<T>(RB);                                                                           \
             acc0.x = fmaf(WT, VA.x, acc0.x); acc0.y = fmaf(WT, VA.y, acc0.y); acc0.z = fmaf(WT, VA.z, acc0.z); acc0.w = fmaf(WT, VA.w, acc0.w); \
             acc1.x = fmaf(WT, VB.x, acc1.x); acc1.y = fmaf(WT, VB.y, acc1.y); acc1.z = fmaf(WT, VB.z, acc1.z); acc1.w = fmaf(WT, VB.w, acc1.w); \
         }
@@ -841,11 +985,11 @@ roi_align_fwd77_kernel(LevelSet L, const RoiGeom* __restrict__ gsorted, int K, f
 #pragma unroll 1
         do {
             const bool p0 = e < cnt, p1 = e + 1 < cnt, p2 = e + 2 < cnt, p3 = e + 3 < cnt;
-            float4 v00, v01, v10, v11, v20, v21, v30, v31;
-            if (p0) { const float* q = tap_ptr(feat, (unsigned)en0.x); v00 = ldg_flavour_v4<FLAVOUR>(q); v01 = ldg_flavour_v4<FLAVOUR>(q + 128); }
-            if (p1) { const float* q = tap_ptr(feat, (unsigned)en1.x); v10 = ldg_flavour_v4<FLAVOUR>(q); v11 = ldg_flavour_v4<FLAVOUR>(q + 128); }
-            if (p2) { const float* q = tap_ptr(feat, (unsigned)en2.x); v20 = ldg_flavour_v4<FLAVOUR>(q); v21 = ldg_flavour_v4<FLAVOUR>(q + 128); }
-            if (p3) { const float* q = tap_ptr(feat, (unsigned)en3.x); v30 = ldg_flavour_v4<FLAVOUR>(q); v31 = ldg_flavour_v4<FLAVOUR>(q + 128); }
+            typename Quad<T>::V v00, v01, v10, v11, v20, v21, v30, v31;   // raw: 2-byte values convert right before their FMAs
+            if (p0) { const T* q = quad_ptr<T>(feat, (unsigned)en0.x); v00 = ldg4_raw<T, FLAVOUR>(q); v01 = ldg4_raw<T, FLAVOUR>(q + 128); }
+            if (p1) { const T* q = quad_ptr<T>(feat, (unsigned)en1.x); v10 = ldg4_raw<T, FLAVOUR>(q); v11 = ldg4_raw<T, FLAVOUR>(q + 128); }
+            if (p2) { const T* q = quad_ptr<T>(feat, (unsigned)en2.x); v20 = ldg4_raw<T, FLAVOUR>(q); v21 = ldg4_raw<T, FLAVOUR>(q + 128); }
+            if (p3) { const T* q = quad_ptr<T>(feat, (unsigned)en3.x); v30 = ldg4_raw<T, FLAVOUR>(q); v31 = ldg4_raw<T, FLAVOUR>(q + 128); }
             const float w0 = __int_as_float(en0.y), w1 = __int_as_float(en1.y), w2 = __int_as_float(en2.y), w3 = __int_as_float(en3.y);
             e += 4;
             const bool more = e < cnt;
@@ -861,11 +1005,11 @@ roi_align_fwd77_kernel(LevelSet L, const RoiGeom* __restrict__ gsorted, int K, f
 #undef RSDET_ACC
     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
     __syncthreads();
-    float* __restrict__ dst = out + ((size_t)roi * C + chunk0) * NB;
+    O* __restrict__ dst = out + ((size_t)roi * C + chunk0) * NB;
     if ((((size_t)out) & 15) == 0 && ((C * NB) & 3) == 0) {
-        if (tid == 0) bulk_store_evict_first(dst, s_stage, 256u * NB * 4u);
+        if (tid == 0) bulk_store_evict_first(dst, s_stage, 256u * NB * (unsigned)sizeof(O));
     } else {
-        for (int i = tid; i < 256 * NB; i += THREADS) __stcs(dst + i, s_stage[i]);
+        for (int i = tid; i < 256 * NB; i += THREADS) stcs1(dst + i, s_stage[i]);
     }
 }
 
@@ -884,10 +1028,13 @@ roi_align_fwd77_kernel(LevelSet L, const RoiGeom* __restrict__ gsorted, int K, f
 // Lists have a pitch of 18 entries (16-byte aligned: a batch's four entries are two LDS.128; the count sits in entry 16).
 // Arithmetic and tap order are those of roi_align_fwd77_kernel: bit-identical results.
 constexpr size_t kStage77pOffset = (8 * 49 * 18 + 16 + 48 + 127) & ~(size_t)127;   // lists | next item | next record | staging
-template <int WARPS, int MINB, int TAPS = 4>   // TAPS: list entries per batch (4, 6 or 8 = 8 / 12 / 16 16-byte loads in flight per thread)
+// TAPS: list entries per batch (4, 6 or 8 = 8 / 12 / 16 vector loads in flight per thread); T: feature elements (a half
+// map halves the bytes of every tap load: two 8-byte loads per lane and tap); O: output elements (a half output halves
+// the staging block and its bulk store)
+template <int WARPS, int MINB, int TAPS = 4, typename T = float, typename O = float>
 __global__ void __launch_bounds__(32 * WARPS, MINB)
 roi_align_fwd77p_kernel(LevelSet L, const int* __restrict__ order, const RoiGeom* __restrict__ geoms, int K, int chunks,
-                        float* __restrict__ out, unsigned* __restrict__ counter) {
+                        O* __restrict__ out, unsigned* __restrict__ counter) {
     constexpr int NB = 49, PITCH = 18, THREADS = 32 * WARPS;
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -895,10 +1042,10 @@ roi_align_fwd77p_kernel(LevelSet L, const int* __restrict__ order, const RoiGeom
     volatile int* s_next = reinterpret_cast<volatile int*>(smem_raw + 8 * NB * PITCH);
     volatile int* s_roi = reinterpret_cast<volatile int*>(smem_raw + 8 * NB * PITCH + 4);      // RoI index of the record in s_geom
     const RoiGeom* s_geom = reinterpret_cast<const RoiGeom*>(smem_raw + 8 * NB * PITCH + 16);
-    float* s_stage = reinterpret_cast<float*>(smem_raw + kStage77pOffset);
+    O* s_stage = reinterpret_cast<O*>(smem_raw + kStage77pOffset);
     const int C = L.C, items = K * chunks;
     const int oct = (lane >> 3) & 3;
-    float* const sbase = s_stage + lane * 4 * NB;
+    O* const sbase = s_stage + lane * 4 * NB;
     int idx = blockIdx.x;
     if (tid < 3 && idx < items) {
         const int r = order ? order[idx / chunks] : idx / chunks;      // position in processing order -> RoI
@@ -968,19 +1115,19 @@ roi_align_fwd77p_kernel(LevelSet L, const int* __restrict__ order, const RoiGeom
             asm volatile("cp.async.commit_group;" ::: "memory");
         }
 
-        const float4* __restrict__ feat =
-            reinterpret_cast<const float4*>(L.feat[g.level] + (size_t)g.batch * H * W * C + chunk0) + lane;
+        const typename Quad<T>::V* __restrict__ feat =
+            reinterpret_cast<const typename Quad<T>::V*>(feat_base<T>(L, g.level) + (size_t)g.batch * H * W * C + chunk0) + lane;
         auto stage = [&](float4 a0, float4 a1, int b) {
             a0.x *= 0.25f; a0.y *= 0.25f; a0.z *= 0.25f; a0.w *= 0.25f;   // output_val /= count (:143), count = 4: exact
             a1.x *= 0.25f; a1.y *= 0.25f; a1.z *= 0.25f; a1.w *= 0.25f;
             const float4 r0 = rot4(a0, oct), r1 = rot4(a1, oct);
-            float* const sb = sbase + b;
-            float* const q0 = sb + ((0 + oct) & 3) * NB;
-            float* const q1 = sb + ((1 + oct) & 3) * NB;
-            float* const q2 = sb + ((2 + oct) & 3) * NB;
-            float* const q3 = sb + ((3 + oct) & 3) * NB;
-            q0[0] = r0.x; q1[0] = r0.y; q2[0] = r0.z; q3[0] = r0.w;
-            q0[128 * NB] = r1.x; q1[128 * NB] = r1.y; q2[128 * NB] = r1.z; q3[128 * NB] = r1.w;
+            O* const sb = sbase + b;
+            O* const q0 = sb + ((0 + oct) & 3) * NB;
+            O* const q1 = sb + ((1 + oct) & 3) * NB;
+            O* const q2 = sb + ((2 + oct) & 3) * NB;
+            O* const q3 = sb + ((3 + oct) & 3) * NB;
+            q0[0] = from_f32<O>(r0.x); q1[0] = from_f32<O>(r0.y); q2[0] = from_f32<O>(r0.z); q3[0] = from_f32<O>(r0.w);
+            q0[128 * NB] = from_f32<O>(r1.x); q1[128 * NB] = from_f32<O>(r1.y); q2[128 * NB] = from_f32<O>(r1.z); q3[128 * NB] = from_f32<O>(r1.w);
         };
         const int2* lp = s_list + warp * PITCH;
         int4 en[TAPS / 2];
@@ -995,13 +1142,13 @@ roi_align_fwd77p_kernel(LevelSet L, const int* __restrict__ order, const RoiGeom
             int e = 0;
 #pragma unroll 1
             do {
-                float4 va[TAPS], vb[TAPS];
+                typename Quad<T>::V va[TAPS], vb[TAPS];   // raw: 2-byte values convert right before their FMAs
                 float wt[TAPS];
 #pragma unroll
                 for (int t = 0; t < TAPS; t++) {
                     const int off = (t & 1) ? en[t >> 1].z : en[t >> 1].x;
                     wt[t] = __int_as_float((t & 1) ? en[t >> 1].w : en[t >> 1].y);
-                    if (e + t < cnt) { const float* q = tap_ptr(feat, (unsigned)off); va[t] = ldg_nc_v4(q); vb[t] = ldg_nc_v4(q + 128); }
+                    if (e + t < cnt) { const T* q = quad_ptr<T>(feat, (unsigned)off); va[t] = ldg4_raw(q); vb[t] = ldg4_raw(q + 128); }
                 }
                 const int e0 = e;
                 e += TAPS;
@@ -1013,8 +1160,10 @@ roi_align_fwd77p_kernel(LevelSet L, const int* __restrict__ order, const RoiGeom
 #pragma unroll
                 for (int t = 0; t < TAPS; t++)
                     if (e0 + t < cnt) {
-                        acc0.x = fmaf(wt[t], va[t].x, acc0.x); acc0.y = fmaf(wt[t], va[t].y, acc0.y); acc0.z = fmaf(wt[t], va[t].z, acc0.z); acc0.w = fmaf(wt[t], va[t].w, acc0.w);
-                        acc1.x = fmaf(wt[t], vb[t].x, acc1.x); acc1.y = fmaf(wt[t], vb[t].y, acc1.y); acc1.z = fmaf(wt[t], vb[t].z, acc1.z); acc1.w = fmaf(wt[t], vb[t].w, acc1.w);
+                        const auto& a = quad_f32<T>(va[t]);
+                        const auto& c = quad_f32<T>(vb[t]);
+                        acc0.x = fmaf(wt[t], a.x, acc0.x); acc0.y = fmaf(wt[t], a.y, acc0.y); acc0.z = fmaf(wt[t], a.z, acc0.z); acc0.w = fmaf(wt[t], a.w, acc0.w);
+                        acc1.x = fmaf(wt[t], c.x, acc1.x); acc1.y = fmaf(wt[t], c.y, acc1.y); acc1.z = fmaf(wt[t], c.z, acc1.z); acc1.w = fmaf(wt[t], c.w, acc1.w);
                     }
             } while (e < cnt);
             stage(acc0, acc1, b);
@@ -1028,7 +1177,7 @@ roi_align_fwd77p_kernel(LevelSet L, const int* __restrict__ order, const RoiGeom
             unsigned long long pol;
             asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(pol));
             asm volatile("cp.async.bulk.global.shared::cta.bulk_group.L2::cache_hint [%0], [%1], %2, %3;"
-                         ::"l"(out + ((size_t)roi * C + chunk0) * NB), "r"((unsigned)__cvta_generic_to_shared(s_stage)), "r"(256u * NB * 4u), "l"(pol) : "memory");
+                         ::"l"(out + ((size_t)roi * C + chunk0) * NB), "r"((unsigned)__cvta_generic_to_shared(s_stage)), "r"(256u * NB * (unsigned)sizeof(O)), "l"(pol) : "memory");
             asm volatile("cp.async.bulk.commit_group;" ::: "memory");
         }
         idx = *s_next;
@@ -1092,10 +1241,10 @@ static bool fwd77_ok(const rsdet_roi_align_cfg* c) {
 // Same CTA shape and tap lists.  The RoI's (C,7,7) gradient block is copied into shared memory as it
 // lies in memory (coalesced 16-byte loads); every merged tap becomes ONE 16-byte vector reduction per
 // channel quad (red.global.add.v4.f32) into the channels-last accumulator.
-template <int QPT>
+template <int QPT, typename G = float>   // G: grad_out elements (staged as fp32); the accumulators are always fp32
 __global__ void __launch_bounds__(kRoiThreads, 4)
 roi_align_bwd_kernel(LevelSet L, const float* __restrict__ rois, const int* __restrict__ order, const RoiGeom* __restrict__ geoms,
-                     int K, const float* __restrict__ grad_out) {
+                     int K, const G* __restrict__ grad_out) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int roi = order ? order[blockIdx.x] : blockIdx.x;
     const int tid = threadIdx.x;
@@ -1120,13 +1269,13 @@ roi_align_bwd_kernel(LevelSet L, const float* __restrict__ rois, const int* __re
     build_tap_lists(g, L, H, W, s_list, s_cnt, s_stage, C >> 2, 0);
 
     // stage this chunk's gradient block [c_local][bin] (= memory order)
-    const float* __restrict__ src = grad_out + ((size_t)roi * C + chunk0) * nbins;
+    const G* __restrict__ src = grad_out + ((size_t)roi * C + chunk0) * nbins;
     const int total = Qc * 4 * nbins;
-    if ((((size_t)roi * C + chunk0) * nbins & 3) == 0 && (total & 3) == 0 && (((size_t)grad_out) & 15) == 0) {
+    if ((((size_t)roi * C + chunk0) * nbins & 3) == 0 && (total & 3) == 0 && (((size_t)grad_out) & (4 * sizeof(G) - 1)) == 0) {
         float4* s4 = reinterpret_cast<float4*>(s_stage);
-        for (int e = tid; e < total / 4; e += kRoiThreads) s4[e] = ldg_cs_v4(src + (size_t)e * 4);
+        for (int e = tid; e < total / 4; e += kRoiThreads) s4[e] = ldcs4(src + (size_t)e * 4);
     } else {
-        for (int e = tid; e < total; e += kRoiThreads) s_stage[e] = __ldg(src + e);
+        for (int e = tid; e < total; e += kRoiThreads) s_stage[e] = to_f32(__ldg(src + e));
     }
     __syncthreads();
 
@@ -1174,7 +1323,7 @@ roi_align_bwd_kernel(LevelSet L, const float* __restrict__ rois, const int* __re
 // output element like the reference, but with the level mapping fused.  Used only when the fast path's
 // preconditions (C % 4 == 0, fixed sampling grid, <= kMaxSamples samples) do not hold.
 struct GenericMaps {
-    const float* feat[RSDET_MAX_LEVELS];
+    const float* feat[RSDET_MAX_LEVELS];   // element type: the kernel's T
     float* grad[RSDET_MAX_LEVELS];
     int channels_last;
 };
@@ -1183,9 +1332,11 @@ __device__ __forceinline__ size_t feat_index(int cl, int n, int c, int pix, int 
     return cl ? ((size_t)n * HW + pix) * C + c : ((size_t)n * C + c) * HW + pix;
 }
 
-template <bool BACKWARD>
+// T: feature elements (forward); O: output elements (forward) or grad_out elements (backward); gradients accumulate in
+// fp32 maps (M.grad) in the caller's layout
+template <bool BACKWARD, typename T = float, typename O = float>
 __global__ void roi_align_generic_kernel(LevelSet L, GenericMaps M, const float* __restrict__ rois, int K,
-                                         float* __restrict__ out_or_gradout, int32_t* __restrict__ levels_out) {
+                                         O* __restrict__ out_or_gradout, int32_t* __restrict__ levels_out) {
     const int nbins = L.PH * L.PW;
     const long long total = (long long)K * L.C * nbins;
     for (long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x; idx < total; idx += (long long)gridDim.x * blockDim.x) {
@@ -1202,17 +1353,17 @@ __global__ void roi_align_generic_kernel(LevelSet L, GenericMaps M, const float*
                     float x, y;
                     sample_xy(g, L.version, ph, pw, iy, ix, x, y);
                     Taps t = make_taps(H, W, y, x);
-                    const float* f = M.feat[g.level];
-                    float v = t.w[0] * f[feat_index(M.channels_last, g.batch, c, t.o[0], L.C, H * W)] +
-                              t.w[1] * f[feat_index(M.channels_last, g.batch, c, t.o[1], L.C, H * W)] +
-                              t.w[2] * f[feat_index(M.channels_last, g.batch, c, t.o[2], L.C, H * W)] +
-                              t.w[3] * f[feat_index(M.channels_last, g.batch, c, t.o[3], L.C, H * W)];
+                    const T* f = reinterpret_cast<const T*>(M.feat[g.level]);
+                    float v = t.w[0] * to_f32(f[feat_index(M.channels_last, g.batch, c, t.o[0], L.C, H * W)]) +
+                              t.w[1] * to_f32(f[feat_index(M.channels_last, g.batch, c, t.o[1], L.C, H * W)]) +
+                              t.w[2] * to_f32(f[feat_index(M.channels_last, g.batch, c, t.o[2], L.C, H * W)]) +
+                              t.w[3] * to_f32(f[feat_index(M.channels_last, g.batch, c, t.o[3], L.C, H * W)]);
                     acc += v;
                 }
-            out_or_gradout[idx] = acc / count;
+            out_or_gradout[idx] = from_f32<O>(acc / count);
         } else {
             const float count = (float)(g.gh * g.gw);
-            const float top = out_or_gradout[idx];
+            const float top = to_f32(out_or_gradout[idx]);
             for (int iy = 0; iy < g.gh; iy++)
                 for (int ix = 0; ix < g.gw; ix++) {
                     float x, y;
@@ -1235,13 +1386,15 @@ static bool fast_path_ok(const rsdet_roi_align_cfg* c) {
            c->pooled_h * c->pooled_w * c->sampling_ratio * c->sampling_ratio <= kMaxSamples;
 }
 
-// The fast kernels read (forward) or accumulate into (backward) a channels-last caller's maps with 16-byte vector
-// accesses from each level's base pointer; a base that is not 16-byte aligned goes to the scalar generic kernel, which
-// addresses NHWC maps directly.  NCHW maps are only read by the transposes, which check alignment themselves.
-static bool nhwc_bases_aligned(const rsdet_roi_align_cfg* c, const float* const* maps) {
+// The fast kernels read (forward) or accumulate into (backward) a channels-last caller's maps with 4-channel vector
+// accesses from each level's base pointer (16 bytes for fp32, 8 for half maps); a base that is not aligned to that goes
+// to the scalar generic kernel, which addresses NHWC maps directly.  NCHW maps are only read by the transposes, which
+// check alignment themselves.
+template <typename P>
+static bool nhwc_bases_aligned(const rsdet_roi_align_cfg* c, P const* maps, size_t align) {
     if (!c->channels_last) return true;
     for (int l = 0; l < c->num_levels; l++)
-        if (((size_t)maps[l]) & 15) return false;
+        if (((size_t)maps[l]) & (align - 1)) return false;
     return true;
 }
 
@@ -1287,9 +1440,10 @@ static size_t fwd_smem_bytes(const rsdet_roi_align_cfg* c) {
 
 using namespace rsdet;
 
-extern "C" size_t rsdet_roi_align_rotated_workspace_bytes(const rsdet_roi_align_cfg* cfg, int num_rois, int backward) {
-    (void)backward;
-    if (check_cfg(cfg) != RSDET_OK) return 0;
+static bool dtype_ok(int dt) { return dt == RSDET_DTYPE_F32 || dt == RSDET_DTYPE_F16 || dt == RSDET_DTYPE_BF16; }
+
+// elem: bytes of one feature-map element
+static size_t roi_workspace_bytes(const rsdet_roi_align_cfg* cfg, int num_rois, int backward, size_t elem) {
     // order, geometry, geometry in processing order (+ one record: the work counter of the persistent forward kernel)
     size_t b = ws_bytes<int>(num_rois > 0 ? num_rois : 1) + ws_bytes<RoiGeom>(num_rois > 0 ? num_rois : 1) +
                ws_bytes<RoiGeom>((num_rois > 0 ? num_rois : 1) + 1);
@@ -1299,47 +1453,59 @@ extern "C" size_t rsdet_roi_align_rotated_workspace_bytes(const rsdet_roi_align_
                                      (rec_stride((size_t)cfg->pooled_h * cfg->pooled_w, 4 * (size_t)cfg->sampling_ratio * cfg->sampling_ratio) +
                                       stream_rec_stride((size_t)cfg->pooled_h * cfg->pooled_w, 4 * (size_t)cfg->sampling_ratio * cfg->sampling_ratio)));
 #endif
+    if (backward && elem != sizeof(float)) {    // half gradient maps: fp32 accumulators on every path
+        for (int l = 0; l < cfg->num_levels; l++)
+            b += ws_bytes<float>((size_t)cfg->batch * cfg->channels * cfg->height[l] * cfg->width[l]);
+        return b + 256;
+    }
     if (cfg->channels_last || !fast_path_ok(cfg)) return b + 256;
-    for (int l = 0; l < cfg->num_levels; l++)
-        b += ws_bytes<float>((size_t)cfg->batch * cfg->channels * cfg->height[l] * cfg->width[l]);
+    for (int l = 0; l < cfg->num_levels; l++)      // NHWC copy of the pyramid (forward) / fp32 NHWC accumulators (backward)
+        b += align256(elem * cfg->batch * cfg->channels * cfg->height[l] * cfg->width[l]);
     return b + 256;
 }
 
-extern "C" int rsdet_roi_align_rotated_forward(const rsdet_roi_align_cfg* cfg, const float* const* feats_host, const float* rois,
-                                               int num_rois, float* out, int32_t* levels_out, void* workspace,
-                                               size_t workspace_bytes, void* stream) {
-    int rc = check_cfg(cfg);
-    if (rc != RSDET_OK) return rc;
-    if (num_rois < 0) return RSDET_EINVAL;
-    if (num_rois == 0) return RSDET_OK;
-    if (!feats_host || !rois || !out) return RSDET_EINVAL;
-    for (int l = 0; l < cfg->num_levels; l++)
-        if (!feats_host[l]) return RSDET_EINVAL;
-    cudaStream_t st = (cudaStream_t)stream;
+extern "C" size_t rsdet_roi_align_rotated_workspace_bytes_typed(const rsdet_roi_align_cfg* cfg, int num_rois, int backward,
+                                                                 int feat_dtype) {
+    if (!dtype_ok(feat_dtype) || check_cfg(cfg) != RSDET_OK) return 0;
+    return roi_workspace_bytes(cfg, num_rois, backward, feat_dtype == RSDET_DTYPE_F32 ? sizeof(float) : 2);
+}
+
+extern "C" size_t rsdet_roi_align_rotated_workspace_bytes(const rsdet_roi_align_cfg* cfg, int num_rois, int backward) {
+    return rsdet_roi_align_rotated_workspace_bytes_typed(cfg, num_rois, backward, RSDET_DTYPE_F32);
+}
+
+// T: feature elements, O: output elements (float or T).  Arguments are checked by the caller.
+template <typename T, typename O>
+static int forward_impl(const rsdet_roi_align_cfg* cfg, const T* const* feats_host, const float* rois, int num_rois, O* out,
+                        int32_t* levels_out, void* workspace, size_t workspace_bytes, cudaStream_t st) {
+#ifdef RSDET_TUNING
+    constexpr bool kF32Call = kIsF32<T> && kIsF32<O>;   // the A/B kernels of RSDET_TUNING builds exist for fp32 only
+#endif
+    int rc = RSDET_OK;
     LevelSet L = make_levels(cfg);
-    if (!fast_path_ok(cfg) || !nhwc_bases_aligned(cfg, feats_host)) {
+    if (!fast_path_ok(cfg) || !nhwc_bases_aligned(cfg, feats_host, 4 * sizeof(T))) {
         GenericMaps M;
         M.channels_last = cfg->channels_last;
-        for (int l = 0; l < RSDET_MAX_LEVELS; l++) { M.feat[l] = l < cfg->num_levels ? feats_host[l] : nullptr; M.grad[l] = nullptr; }
+        for (int l = 0; l < RSDET_MAX_LEVELS; l++) {
+            M.feat[l] = l < cfg->num_levels ? reinterpret_cast<const float*>(feats_host[l]) : nullptr;
+            M.grad[l] = nullptr;
+        }
         long long total = (long long)num_rois * cfg->channels * cfg->pooled_h * cfg->pooled_w;
         int grid = (int)(ceil_div_ll(total, 256) < (long long)kNumSMs * 16 ? ceil_div_ll(total, 256) : (long long)kNumSMs * 16);
-        roi_align_generic_kernel<false><<<grid, 256, 0, st>>>(L, M, rois, num_rois, out, levels_out);
+        roi_align_generic_kernel<false, T, O><<<grid, 256, 0, st>>>(L, M, rois, num_rois, out, levels_out);
         count_launch();
         return cuda_status();
     }
-    if (workspace_bytes < rsdet_roi_align_rotated_workspace_bytes(cfg, num_rois, 0)) return RSDET_EWORKSPACE;
+    if (workspace_bytes < roi_workspace_bytes(cfg, num_rois, 0, sizeof(T))) return RSDET_EWORKSPACE;
     Workspace ws(workspace, workspace_bytes);
     int* order_ws = ws.take<int>(num_rois);
     RoiGeom* geoms = ws.take<RoiGeom>(num_rois);
     RoiGeom* gsorted = ws.take<RoiGeom>(num_rois + 1);
     if (cfg->channels_last) {
-        for (int l = 0; l < cfg->num_levels; l++) L.feat[l] = feats_host[l];
+        for (int l = 0; l < cfg->num_levels; l++) L.feat[l] = reinterpret_cast<const float*>(feats_host[l]);
     } else {
-        float* dst[RSDET_MAX_LEVELS];
-        for (int l = 0; l < cfg->num_levels; l++) {
-            dst[l] = ws.take<float>((size_t)cfg->batch * cfg->channels * cfg->height[l] * cfg->width[l]);
-            L.feat[l] = dst[l];
-        }
+        for (int l = 0; l < cfg->num_levels; l++)
+            L.feat[l] = reinterpret_cast<const float*>(ws.take<T>((size_t)cfg->batch * cfg->channels * cfg->height[l] * cfg->width[l]));
         if (!ws.ok()) return RSDET_EWORKSPACE;
     }
     // locality order (needs the int[K] slot at the start of the workspace; skipped for tiny calls)
@@ -1366,8 +1532,8 @@ extern "C" int rsdet_roi_align_rotated_forward(const rsdet_roi_align_cfg* cfg, c
         // NCHW -> NHWC copy of the pyramid; the locality-order block rides along as block 0 of the same launch
         PrepArgs prep = {&L, rois, num_rois, order};
         if (lean) { prep.geoms = geoms; prep.levels_out = levels_out; prep.counter = counter; }
-        float* dst[RSDET_MAX_LEVELS];
-        for (int l = 0; l < cfg->num_levels; l++) dst[l] = const_cast<float*>(L.feat[l]);
+        T* dst[RSDET_MAX_LEVELS];
+        for (int l = 0; l < cfg->num_levels; l++) dst[l] = reinterpret_cast<T*>(const_cast<float*>(L.feat[l]));
         rc = launch_transpose(true, feats_host, dst, cfg->height, cfg->width, cfg->num_levels, cfg->batch, cfg->channels, st,
                               ride ? &prep : nullptr);
         if (rc != RSDET_OK) return rc;
@@ -1377,10 +1543,10 @@ extern "C" int rsdet_roi_align_rotated_forward(const rsdet_roi_align_cfg* cfg, c
 #ifdef RSDET_TUNING
     if (const char* e = getenv("RSDET_ROI_PAD_SMEM")) smem += (size_t)atoi(e) * 1024;   // fewer resident CTAs per SM
 #endif
-    set_dyn_smem((const void*)roi_align_fwd_kernel<1>, smem);
-    set_dyn_smem((const void*)roi_align_fwd_kernel<2>, smem);
+    set_dyn_smem((const void*)roi_align_fwd_kernel<1, T, O>, smem);
+    set_dyn_smem((const void*)roi_align_fwd_kernel<2, T, O>, smem);
 #ifdef RSDET_TUNING
-    {
+    if constexpr (kF32Call) {
         int trc = RSDET_OK;
         if (tuning_forward(cfg, L, ws, rois, order, geoms, num_rois, out, levels_out, st, &trc)) return trc;
     }
@@ -1393,13 +1559,12 @@ extern "C" int rsdet_roi_align_rotated_forward(const rsdet_roi_align_cfg* cfg, c
         if (const char* e = getenv("RSDET_ROI_WARPS")) warps = atoi(e);
 #endif
 #ifdef RSDET_TUNING
+        if constexpr (kF32Call) {
         const int flavour = getenv("RSDET_ROI_LD") ? atoi(getenv("RSDET_ROI_LD")) : 0;
         dim3 g77(num_rois, cfg->channels / 256);
         if (flavour == 1) { set_dyn_smem((const void*)roi_align_fwd77_kernel<8, 1>, smem); roi_align_fwd77_kernel<8, 1><<<g77, 256, smem, st>>>(L, gsorted, num_rois, out); count_launch(); return cuda_status(); }
         if (flavour == 2) { set_dyn_smem((const void*)roi_align_fwd77_kernel<8, 2>, smem); roi_align_fwd77_kernel<8, 2><<<g77, 256, smem, st>>>(L, gsorted, num_rois, out); count_launch(); return cuda_status(); }
         if (flavour == 3) { set_dyn_smem((const void*)roi_align_fwd77_kernel<8, 3>, smem); roi_align_fwd77_kernel<8, 3><<<g77, 256, smem, st>>>(L, gsorted, num_rois, out); count_launch(); return cuda_status(); }
-#endif
-#ifdef RSDET_TUNING
         if (const char* e = getenv("RSDET_ROI_MINB3")) {     // A/B: three CTAs per SM by launch bounds (more registers, smaller carve-out)
             const int w = atoi(e);
             const int carve = getenv("RSDET_ROI_CARVE") ? atoi(getenv("RSDET_ROI_CARVE")) : -1;
@@ -1430,8 +1595,6 @@ extern "C" int rsdet_roi_align_rotated_forward(const rsdet_roi_align_cfg* cfg, c
             }
             if (atoi(e) == 2) { set_dyn_smem((const void*)roi_align_fwd77v8_kernel<7, true>, sm8); roi_align_fwd77v8_kernel<7, true><<<g77, 224, sm8, st>>>(L, gsorted, num_rois, out); count_launch(); return cuda_status(); }
         }
-#endif
-#ifdef RSDET_TUNING
         if (getenv("RSDET_ROI_Q")) {      // A/B (old prologue: records in processing order): pipelined list build (1: dynamic bins, 2: static columns)
             const int chunks = cfg->channels / 256;
             const long long items = (long long)num_rois * chunks;
@@ -1449,6 +1612,7 @@ extern "C" int rsdet_roi_align_rotated_forward(const rsdet_roi_align_cfg* cfg, c
             count_launch();
             return cuda_status();
         }
+        }
 #endif
         if (lean) {                                     // persistent kernel (needs a 16-byte aligned output block for its bulk store)
             const int chunks = cfg->channels / 256;
@@ -1458,7 +1622,7 @@ extern "C" int rsdet_roi_align_rotated_forward(const rsdet_roi_align_cfg* cfg, c
             if (const char* e = getenv("RSDET_ROI_PCTAS")) ctas = atoi(e);
 #endif
 #ifdef RSDET_TUNING
-            if (const char* e = getenv("RSDET_ROI_PVAR")) {     // A/B: warps x CTAs/SM x taps per batch of the persistent kernel
+            if constexpr (kF32Call) if (const char* e = getenv("RSDET_ROI_PVAR")) {     // A/B: warps x CTAs/SM x taps per batch of the persistent kernel
                 const size_t smv = kStage77pOffset + sizeof(float) * 49 * 256;
                 unsigned* ctr = reinterpret_cast<unsigned*>(gsorted + num_rois);
                 const int v = atoi(e);
@@ -1478,18 +1642,18 @@ extern "C" int rsdet_roi_align_rotated_forward(const rsdet_roi_align_cfg* cfg, c
             }
 #endif
             const size_t smp = kStage77pOffset + sizeof(float) * 49 * 256;
-            set_dyn_smem((const void*)roi_align_fwd77p_kernel<8, 3>, smp);
-            roi_align_fwd77p_kernel<8, 3><<<(int)(items < ctas ? items : ctas), 256, smp, st>>>(
+            set_dyn_smem((const void*)roi_align_fwd77p_kernel<8, 3, 4, T, O>, smp);
+            roi_align_fwd77p_kernel<8, 3, 4, T, O><<<(int)(items < ctas ? items : ctas), 256, smp, st>>>(
                 L, order, geoms, num_rois, chunks, out, counter);
             count_launch();
             return cuda_status();
         }
         if (warps == 7) {
-            set_dyn_smem((const void*)roi_align_fwd77_kernel<7>, smem);
-            roi_align_fwd77_kernel<7><<<dim3(num_rois, cfg->channels / 256), 224, smem, st>>>(L, gsorted, num_rois, out);
+            set_dyn_smem((const void*)roi_align_fwd77_kernel<7, 0, 4, T, O>, smem);
+            roi_align_fwd77_kernel<7, 0, 4, T, O><<<dim3(num_rois, cfg->channels / 256), 224, smem, st>>>(L, gsorted, num_rois, out);
         } else {
-            set_dyn_smem((const void*)roi_align_fwd77_kernel<8>, smem);
-            roi_align_fwd77_kernel<8><<<dim3(num_rois, cfg->channels / 256), 256, smem, st>>>(L, gsorted, num_rois, out);
+            set_dyn_smem((const void*)roi_align_fwd77_kernel<8, 0, 4, T, O>, smem);
+            roi_align_fwd77_kernel<8, 0, 4, T, O><<<dim3(num_rois, cfg->channels / 256), 256, smem, st>>>(L, gsorted, num_rois, out);
         }
         count_launch();
         return cuda_status();
@@ -1497,32 +1661,77 @@ extern "C" int rsdet_roi_align_rotated_forward(const rsdet_roi_align_cfg* cfg, c
     const int Q = quads_per_chunk(cfg->channels);
     dim3 grid(num_rois, ceil_div(cfg->channels / 4, Q));
     if (cfg->channels % 256 == 0)
-        roi_align_fwd_kernel<2><<<grid, kRoiThreads, smem, st>>>(L, rois, order, geoms, num_rois, out, nullptr);
+        roi_align_fwd_kernel<2, T, O><<<grid, kRoiThreads, smem, st>>>(L, rois, order, geoms, num_rois, out, nullptr);
     else
-        roi_align_fwd_kernel<1><<<grid, kRoiThreads, smem, st>>>(L, rois, order, geoms, num_rois, out, nullptr);
+        roi_align_fwd_kernel<1, T, O><<<grid, kRoiThreads, smem, st>>>(L, rois, order, geoms, num_rois, out, nullptr);
     count_launch();
     return cuda_status();
 }
 
-extern "C" int rsdet_roi_align_rotated_backward(const rsdet_roi_align_cfg* cfg, const float* grad_out, const float* rois,
-                                                int num_rois, float* const* grad_feats_host, void* workspace,
-                                                size_t workspace_bytes, void* stream) {
+extern "C" int rsdet_roi_align_rotated_forward_typed(const rsdet_roi_align_cfg* cfg, int feat_dtype, const void* const* feats_host,
+                                                     const float* rois, int num_rois, int out_dtype, void* out,
+                                                     int32_t* levels_out, void* workspace, size_t workspace_bytes, void* stream) {
+    if (!dtype_ok(feat_dtype) || (out_dtype != RSDET_DTYPE_F32 && out_dtype != feat_dtype)) return RSDET_EINVAL;
     int rc = check_cfg(cfg);
     if (rc != RSDET_OK) return rc;
-    if (num_rois < 0 || !grad_feats_host) return RSDET_EINVAL;
+    if (num_rois < 0) return RSDET_EINVAL;
+    if (num_rois == 0) return RSDET_OK;
+    if (!feats_host || !rois || !out) return RSDET_EINVAL;
     for (int l = 0; l < cfg->num_levels; l++)
-        if (!grad_feats_host[l]) return RSDET_EINVAL;
+        if (!feats_host[l]) return RSDET_EINVAL;
     cudaStream_t st = (cudaStream_t)stream;
+    const bool half_out = out_dtype != RSDET_DTYPE_F32;
+#define RSDET_FWD(T_, O_) forward_impl<T_, O_>(cfg, reinterpret_cast<const T_* const*>(feats_host), rois, num_rois, static_cast<O_*>(out), \
+                                               levels_out, workspace, workspace_bytes, st)
+    if (feat_dtype == RSDET_DTYPE_F16) return half_out ? RSDET_FWD(__half, __half) : RSDET_FWD(__half, float);
+    if (feat_dtype == RSDET_DTYPE_BF16) return half_out ? RSDET_FWD(__nv_bfloat16, __nv_bfloat16) : RSDET_FWD(__nv_bfloat16, float);
+    return RSDET_FWD(float, float);
+#undef RSDET_FWD
+}
+
+extern "C" int rsdet_roi_align_rotated_forward(const rsdet_roi_align_cfg* cfg, const float* const* feats_host, const float* rois,
+                                               int num_rois, float* out, int32_t* levels_out, void* workspace,
+                                               size_t workspace_bytes, void* stream) {
+    return rsdet_roi_align_rotated_forward_typed(cfg, RSDET_DTYPE_F32, reinterpret_cast<const void* const*>(feats_host), rois,
+                                                 num_rois, RSDET_DTYPE_F32, out, levels_out, workspace, workspace_bytes, stream);
+}
+
+// the fp32 accumulators of half gradient maps -> the caller's maps, same layout (see backward_impl)
+template <typename D>
+static int launch_convert(const rsdet_roi_align_cfg* cfg, float* const* acc, D* const* dst, cudaStream_t st) {
+    ConvertJob job;
+    size_t most = 0;
+    for (int l = 0; l < cfg->num_levels; l++) {
+        job.src[l] = acc[l]; job.dst[l] = dst[l];
+        job.n[l] = (size_t)cfg->batch * cfg->channels * cfg->height[l] * cfg->width[l];
+        most = job.n[l] > most ? job.n[l] : most;
+    }
+    const long long blocks = ceil_div_ll(ceil_div_ll((long long)most, 4), 256);
+    convert_maps_kernel<D><<<dim3((unsigned)(blocks < kNumSMs * 16 ? blocks : kNumSMs * 16), cfg->num_levels), 256, 0, st>>>(job);
+    count_launch();
+    return cuda_status();
+}
+
+// G: grad_out elements (float or T), T: gradient-map elements.  fp32 maps: channels-last maps and generic-kernel calls
+// accumulate straight into the caller's maps, NCHW maps through fp32 NHWC accumulators and the NHWC->NCHW transpose.
+// Half maps always accumulate into fp32 workspace maps -- channels-last for the fast kernels, the caller's layout for the
+// generic kernel -- and ONE pass writes the caller's maps from them, rounding to nearest-even: the NHWC->NCHW transpose,
+// or a conversion that keeps the layout.  The fast kernels then never touch the caller's maps, so their alignment does
+// not matter.
+template <typename G, typename T>
+static int backward_impl(const rsdet_roi_align_cfg* cfg, const G* grad_out, const float* rois, int num_rois, T* const* grad_feats_host,
+                         void* workspace, size_t workspace_bytes, cudaStream_t st) {
+    int rc = RSDET_OK;
     LevelSet L = make_levels(cfg);
-    const bool fast = fast_path_ok(cfg) && nhwc_bases_aligned(cfg, grad_feats_host);
-    const bool direct = cfg->channels_last || !fast;  // accumulate straight into the caller's buffers
+    const bool fast = fast_path_ok(cfg) && (!kIsF32<T> || nhwc_bases_aligned(cfg, grad_feats_host, 16));
+    const bool direct = kIsF32<T> && (cfg->channels_last || !fast);  // accumulate straight into the caller's buffers
     float* acc[RSDET_MAX_LEVELS];
-    if (workspace_bytes < rsdet_roi_align_rotated_workspace_bytes(cfg, num_rois, 1)) return RSDET_EWORKSPACE;
+    if (workspace_bytes < roi_workspace_bytes(cfg, num_rois, 1, sizeof(T))) return RSDET_EWORKSPACE;
     Workspace ws(workspace, workspace_bytes);
     int* order_ws = ws.take<int>(num_rois > 0 ? num_rois : 1);
     RoiGeom* geoms = ws.take<RoiGeom>(num_rois > 0 ? num_rois : 1);
     if (direct) {
-        for (int l = 0; l < cfg->num_levels; l++) acc[l] = grad_feats_host[l];
+        for (int l = 0; l < cfg->num_levels; l++) acc[l] = reinterpret_cast<float*>(grad_feats_host[l]);
     } else {
         for (int l = 0; l < cfg->num_levels; l++)
             acc[l] = ws.take<float>((size_t)cfg->batch * cfg->channels * cfg->height[l] * cfg->width[l]);
@@ -1541,25 +1750,54 @@ extern "C" int rsdet_roi_align_rotated_backward(const rsdet_roi_align_cfg* cfg, 
             for (int l = 0; l < RSDET_MAX_LEVELS; l++) { M.feat[l] = nullptr; M.grad[l] = l < cfg->num_levels ? acc[l] : nullptr; }
             long long total = (long long)num_rois * cfg->channels * cfg->pooled_h * cfg->pooled_w;
             int grid = (int)(ceil_div_ll(total, 256) < (long long)kNumSMs * 16 ? ceil_div_ll(total, 256) : (long long)kNumSMs * 16);
-            roi_align_generic_kernel<true><<<grid, 256, 0, st>>>(L, M, rois, num_rois, const_cast<float*>(grad_out), nullptr);
+            roi_align_generic_kernel<true, float, G><<<grid, 256, 0, st>>>(L, M, rois, num_rois, const_cast<G*>(grad_out), nullptr);
         } else {
             size_t smem = fwd_smem_bytes(cfg);
-            set_dyn_smem((const void*)roi_align_bwd_kernel<1>, smem);
-            set_dyn_smem((const void*)roi_align_bwd_kernel<2>, smem);
+            set_dyn_smem((const void*)roi_align_bwd_kernel<1, G>, smem);
+            set_dyn_smem((const void*)roi_align_bwd_kernel<2, G>, smem);
             int* order = num_rois >= 256 ? order_ws : nullptr;
             launch_prep(L, rois, num_rois, geoms, order, nullptr, st);
             int Q = quads_per_chunk(cfg->channels);
             dim3 grid(num_rois, ceil_div(cfg->channels / 4, Q));
-            if (cfg->channels % 256 == 0) roi_align_bwd_kernel<2><<<grid, kRoiThreads, smem, st>>>(L, rois, order, geoms, num_rois, grad_out);
-            else roi_align_bwd_kernel<1><<<grid, kRoiThreads, smem, st>>>(L, rois, order, geoms, num_rois, grad_out);
+            if (cfg->channels % 256 == 0) roi_align_bwd_kernel<2, G><<<grid, kRoiThreads, smem, st>>>(L, rois, order, geoms, num_rois, grad_out);
+            else roi_align_bwd_kernel<1, G><<<grid, kRoiThreads, smem, st>>>(L, rois, order, geoms, num_rois, grad_out);
         }
         count_launch();
     }
     if (!direct) {
+        if constexpr (!kIsF32<T>) {
+            if (!fast || cfg->channels_last) return launch_convert(cfg, acc, grad_feats_host, st);
+        }
         rc = launch_transpose(false, acc, grad_feats_host, cfg->height, cfg->width, cfg->num_levels, cfg->batch, cfg->channels, st);
         if (rc != RSDET_OK) return rc;
     }
     return cuda_status();
+}
+
+extern "C" int rsdet_roi_align_rotated_backward_typed(const rsdet_roi_align_cfg* cfg, int grad_out_dtype, const void* grad_out,
+                                                      const float* rois, int num_rois, int feat_dtype, void* const* grad_feats_host,
+                                                      void* workspace, size_t workspace_bytes, void* stream) {
+    if (!dtype_ok(feat_dtype) || (grad_out_dtype != RSDET_DTYPE_F32 && grad_out_dtype != feat_dtype)) return RSDET_EINVAL;
+    int rc = check_cfg(cfg);
+    if (rc != RSDET_OK) return rc;
+    if (num_rois < 0 || !grad_feats_host) return RSDET_EINVAL;
+    for (int l = 0; l < cfg->num_levels; l++)
+        if (!grad_feats_host[l]) return RSDET_EINVAL;
+    cudaStream_t st = (cudaStream_t)stream;
+    const bool half_g = grad_out_dtype != RSDET_DTYPE_F32;
+#define RSDET_BWD(G_, T_) backward_impl<G_, T_>(cfg, static_cast<const G_*>(grad_out), rois, num_rois, \
+                                                reinterpret_cast<T_* const*>(grad_feats_host), workspace, workspace_bytes, st)
+    if (feat_dtype == RSDET_DTYPE_F16) return half_g ? RSDET_BWD(__half, __half) : RSDET_BWD(float, __half);
+    if (feat_dtype == RSDET_DTYPE_BF16) return half_g ? RSDET_BWD(__nv_bfloat16, __nv_bfloat16) : RSDET_BWD(float, __nv_bfloat16);
+    return RSDET_BWD(float, float);
+#undef RSDET_BWD
+}
+
+extern "C" int rsdet_roi_align_rotated_backward(const rsdet_roi_align_cfg* cfg, const float* grad_out, const float* rois,
+                                                int num_rois, float* const* grad_feats_host, void* workspace,
+                                                size_t workspace_bytes, void* stream) {
+    return rsdet_roi_align_rotated_backward_typed(cfg, RSDET_DTYPE_F32, grad_out, rois, num_rois, RSDET_DTYPE_F32,
+                                                  reinterpret_cast<void* const*>(grad_feats_host), workspace, workspace_bytes, stream);
 }
 
 #ifdef RSDET_PROF

@@ -10,6 +10,7 @@ from torch import nn
 
 from .... import core
 from ...ops import roi_align_rotated_v1
+from ...ops.roi_align_rotated_v1 import _grad_dtype
 
 
 def _pair(x):
@@ -21,13 +22,14 @@ class _FusedExtractFn(torch.autograd.Function):
     def forward(ctx, rois, cfg, *feats):
         ctx.cfg = cfg
         ctx.shapes = [tuple(f.shape) for f in feats]
+        ctx.dtype = _grad_dtype(feats[0].dtype)      # core rejects levels that mix fp16 / bf16 with another dtype
         ctx.save_for_backward(rois)
         return core.roi_align_rotated_forward(cfg, feats, rois)
 
     @staticmethod
     def backward(ctx, grad_output):
         (rois,) = ctx.saved_tensors
-        grads = core.roi_align_rotated_backward(ctx.cfg, grad_output.contiguous(), rois, ctx.shapes)
+        grads = core.roi_align_rotated_backward(ctx.cfg, grad_output.contiguous(), rois, ctx.shapes, feat_dtype=ctx.dtype)
         return (None, None, *grads)
 
 

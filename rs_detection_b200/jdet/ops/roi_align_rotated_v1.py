@@ -16,21 +16,27 @@ def _pair(x):
     return tuple(x) if isinstance(x, (tuple, list)) else (x, x)
 
 
+def _grad_dtype(dtype):
+    """fp16 / bf16 inputs are read natively and get their gradient in their own dtype; the rest is handled in fp32."""
+    return dtype if dtype in (torch.float16, torch.bfloat16) else torch.float32
+
+
 class _RotatedROIAlignFn(torch.autograd.Function):
-    """Forward + backward of one feature map (the reference's jt.Function, :300-351); rois get no grad."""
+    """Forward + backward of one feature map (the reference's jt.Function, :300-351); rois get no grad.  The output is
+    fp32 whatever the input's dtype, like the reference's float kernels."""
 
     @staticmethod
     def forward(ctx, input, rois, output_size, spatial_scale, sampling_ratio, version):
         assert rois.shape[1] == 6
         cfg = core.make_roi_cfg([tuple(input.shape)], [spatial_scale], output_size, int(sampling_ratio), version)
-        ctx.cfg, ctx.shape = cfg, tuple(input.shape)
+        ctx.cfg, ctx.shape, ctx.dtype = cfg, tuple(input.shape), _grad_dtype(input.dtype)
         ctx.save_for_backward(rois)
         return core.roi_align_rotated_forward(cfg, [input], rois)
 
     @staticmethod
     def backward(ctx, grad_output):
         (rois,) = ctx.saved_tensors
-        grads = core.roi_align_rotated_backward(ctx.cfg, grad_output.contiguous(), rois, [ctx.shape])
+        grads = core.roi_align_rotated_backward(ctx.cfg, grad_output.contiguous(), rois, [ctx.shape], feat_dtype=ctx.dtype)
         return grads[0], None, None, None, None, None
 
 

@@ -252,6 +252,36 @@ def _roi_cfg_src(num_levels, scales, ph, pw, sampling_ratio, version, extend_h, 
     return "\n".join(src) + "\n"
 
 
+def _is_half(var):
+    return str(var.dtype) == "float16"
+
+
+def _roi_half_fwd_src(L, what):
+    """forward body for float16 maps in0..in{L-1} and fp32 rois in{L}: the typed entry point, float16 output"""
+    return r'''
+        RSDET_FN(rsdet_roi_align_rotated_workspace_bytes_typed);
+        RSDET_FN(rsdet_roi_align_rotated_forward_typed);
+        int K = in%d_shape0;
+        Scratch s(fn_rsdet_roi_align_rotated_workspace_bytes_typed(&cfg, K, 0, RSDET_DTYPE_F16));
+        const void* feats[RSDET_MAX_LEVELS] = {%s};
+        rsdet_check(fn_rsdet_roi_align_rotated_forward_typed(&cfg, RSDET_DTYPE_F16, feats, (const float*)in%d_p, K, RSDET_DTYPE_F16,
+                                                             out0_p, nullptr, s.p, s.bytes, 0), "%s");''' % (
+        L, ", ".join("in%d_p" % l for l in range(L)), L, what)
+
+
+def _roi_half_bwd_src(L, grad_half, what):
+    """backward body: float16 gradient maps out0..out{L-1} from grad_out in{L+1} (float16 or fp32) and rois in{L}"""
+    return r'''
+        RSDET_FN(rsdet_roi_align_rotated_workspace_bytes_typed);
+        RSDET_FN(rsdet_roi_align_rotated_backward_typed);
+        int K = in%d_shape0;
+        Scratch s(fn_rsdet_roi_align_rotated_workspace_bytes_typed(&cfg, K, 1, RSDET_DTYPE_F16));
+        void* grads[RSDET_MAX_LEVELS] = {%s};
+        rsdet_check(fn_rsdet_roi_align_rotated_backward_typed(&cfg, %s, in%d_p, (const float*)in%d_p, K, RSDET_DTYPE_F16, grads,
+                                                              s.p, s.bytes, 0), "%s");''' % (
+        L, ", ".join("out%d_p" % l for l in range(L)), "RSDET_DTYPE_F16" if grad_half else "RSDET_DTYPE_F32", L + 1, L, what)
+
+
 def make_roi_align(version):
     """Returns the jt.Function class replacing _RotatedROIAlign(_v1) (roi_align_rotated_v1.py:300-353):
     `.apply(input, rois, output_size, spatial_scale, sampling_ratio)`; grad -> (input_grad, None)."""
@@ -266,6 +296,10 @@ def make_roi_align(version):
             shape = (rois.shape[0], input.shape[1], output_size[0], output_size[1])
             if rois.shape[0] == 0:
                 return jt.zeros(shape, dtype=input.dtype)
+            if _is_half(input):      # float16 maps are read natively (include/rsdet.h); rois stay fp32
+                if str(rois.dtype) != "float32":
+                    self.rois = rois = rois.float32()
+                return _code(shape, input.dtype, [input, rois], self.cfg + _roi_half_fwd_src(1, "roi_align_rotated_forward"))
             return _code(shape, input.dtype, [input, rois], self.cfg + r'''
         RSDET_FN(rsdet_roi_align_rotated_forward);
         int K = in1_shape0;
@@ -276,6 +310,10 @@ def make_roi_align(version):
 
         def grad(self, output_grad):
             input, rois = self.input, self.rois
+            if _is_half(input):
+                g = _code(input.shape, input.dtype, [input, rois, output_grad],
+                          self.cfg + _roi_half_bwd_src(1, _is_half(output_grad), "roi_align_rotated_backward"))
+                return g, None
             g = _code(input.shape, input.dtype, [input, rois, output_grad], self.cfg + r'''
         RSDET_FN(rsdet_roi_align_rotated_backward);
         int K = in1_shape0;
@@ -309,6 +347,13 @@ def make_fused_extractor(version=1):
             shape = (rois.shape[0], feats[0].shape[1], ph, pw)
             if rois.shape[0] == 0:
                 return jt.zeros(shape, dtype=feats[0].dtype)
+            if any(_is_half(f) for f in feats):
+                if not all(_is_half(f) for f in feats):
+                    raise ValueError("rsdet RoIAlignRotated: feature levels mix float16 with another dtype")
+                if str(rois.dtype) != "float32":
+                    self.rois = rois = rois.float32()
+                return _code(shape, feats[0].dtype, feats + [rois],
+                             self.cfg + _roi_half_fwd_src(L, "roi_align_rotated_forward (fused levels)"))
             ptrs = ", ".join("in%d_p" % l for l in range(L))
             return _code(shape, feats[0].dtype, feats + [rois], self.cfg + r'''
         RSDET_FN(rsdet_roi_align_rotated_forward);
@@ -321,6 +366,11 @@ def make_fused_extractor(version=1):
         def grad(self, output_grad):
             feats, rois = self.feats, self.rois
             L = len(feats)
+            if _is_half(feats[0]):
+                gs = _code([f.shape for f in feats], [f.dtype for f in feats], feats + [rois, output_grad],
+                           self.cfg + _roi_half_bwd_src(L, _is_half(output_grad), "roi_align_rotated_backward (fused levels)"))
+                gs = list(gs) if isinstance(gs, (list, tuple)) else [gs]
+                return tuple(gs) + (None,) * (1 + self.nconst)
             outs = ", ".join("out%d_p" % l for l in range(L))
             gs = _code([f.shape for f in feats], [f.dtype for f in feats], feats + [rois, output_grad], self.cfg + r'''
         RSDET_FN(rsdet_roi_align_rotated_backward);
