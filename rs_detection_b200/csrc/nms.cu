@@ -175,13 +175,15 @@ struct SegTable {
     double* seg_thr;       // nseg
 };
 
+// Ascending key = descending score.  -0.0 and +0.0 compare equal, so both get the key of +0.0: a tie, which the stable
+// sorts resolve by index like every other tie (the oracle's stable sort of -scores does the same).
 __device__ __forceinline__ uint32_t desc_key(float s) {
-    uint32_t u = __float_as_uint(s);
+    uint32_t u = __float_as_uint(s == 0.f ? 0.f : s);
     u = (u & 0x80000000u) ? ~u : (u | 0x80000000u);
     return ~u;
 }
 __device__ __forceinline__ unsigned long long desc_key(double s) {
-    unsigned long long u = (unsigned long long)__double_as_longlong(s);
+    unsigned long long u = (unsigned long long)__double_as_longlong(s == 0.0 ? 0.0 : s);
     u = (u >> 63) ? ~u : (u | 0x8000000000000000ull);
     return ~u;
 }
