@@ -152,7 +152,8 @@ typedef struct {
  *            grad_feats  NCHW: written by the NHWC->NCHW copy, which uses 16-byte stores where the map allows them.
  *                        NHWC: the fast kernel accumulates with 16-byte vector reductions from each map's base; if
  *                        any base is not 16-byte aligned the call runs the generic kernel (scalar atomics).
- * Backward results are sums of atomics in an unspecified order: equal across these paths to the backward tolerance. */
+ * Backward results are sums of atomics in an unspecified order: equal across these paths to the backward tolerance.
+ * rsdet_roi_align_rotated_backward_deterministic (below) sums in the reference's order instead: the same bits every run. */
 size_t rsdet_roi_align_rotated_workspace_bytes(const rsdet_roi_align_cfg* cfg, int num_rois, int backward);
 int rsdet_roi_align_rotated_forward(const rsdet_roi_align_cfg* cfg, const float* const* feats_host, const float* rois,
                                     int num_rois, float* out, int32_t* levels_out, void* workspace,
@@ -192,6 +193,30 @@ int rsdet_roi_align_rotated_forward_typed(const rsdet_roi_align_cfg* cfg, int fe
 int rsdet_roi_align_rotated_backward_typed(const rsdet_roi_align_cfg* cfg, int grad_out_dtype, const void* grad_out,
                                            const float* rois, int num_rois, int feat_dtype, void* const* grad_feats_host,
                                            void* workspace, size_t workspace_bytes, void* stream);
+
+/* Deterministic backward: same arguments, dtypes and output as rsdet_roi_align_rotated_backward_typed; the caller picks it.
+ *   Summation order.  Every gradient-map element (level, image, channel, pixel) is the fp32 sum, starting from +0, of
+ *     (top * w) / count, one term per (RoI, bin, sample, tap) whose sample is in range, taken in the reference's order
+ *     (roi_align_rotated_v1.py:193-298): RoI index, bin row, bin column, sample row, sample column, tap lt, rt, lb, rb.
+ *     Every multiply, divide and add is rounded separately, and taps that land on the same pixel are not merged.  Terms
+ *     of weight 0 are dropped (adding +-0 to such a sum changes no bit), as are RoIs whose batch index is outside
+ *     [0, batch).  Half maps get that fp32 value rounded once to nearest-even; a half grad_out converts exactly first.
+ *   Consequences.  The same bits on every run, stream, CUDA-graph replay, layout (NCHW / channels-last), buffer alignment
+ *     and batch split (a batched call equals per-image calls with each image's RoIs in the same relative order); and,
+ *     for finite grad_out, bit-identity with the reference's arithmetic wherever the device's cosf / sinf agree with the
+ *     host's (always at theta = 0).
+ *   Geometries.  Every geometry of the atomic backward with sampling_ratio > 0: any pooled size and C, 1..8 levels with
+ *     extension and level mapping, v0 / v1.  sampling_ratio <= 0 (adaptive grid: the term count depends on the RoI sizes)
+ *     returns RSDET_EINVAL and its workspace query returns 0.
+ *   Limit.  K * pooled_h * pooled_w * sampling_ratio^2 * 4 <= 2^28 terms and batch * sum_l(H_l * W_l) < 2^32 - 1 pixels;
+ *     above either RSDET_ELIMIT (the workspace query returns 0).
+ *   Resources.  No atomics, no host synchronisation, no allocation: every scratch buffer, the radix sort's temporary
+ *     storage included, comes from the workspace, whose query is host-only.  Safe under CUDA-graph capture. */
+size_t rsdet_roi_align_rotated_backward_deterministic_workspace_bytes(const rsdet_roi_align_cfg* cfg, int num_rois,
+                                                                      int feat_dtype);
+int rsdet_roi_align_rotated_backward_deterministic(const rsdet_roi_align_cfg* cfg, int grad_out_dtype, const void* grad_out,
+                                                   const float* rois, int num_rois, int feat_dtype, void* const* grad_feats_host,
+                                                   void* workspace, size_t workspace_bytes, void* stream);
 
 /* Measurement aid (bench.py's roofline): arm two cudaEvent_t (created with timing enabled by the caller).  The NEXT
  * rsdet_roi_align_rotated_forward call issued by this host thread records `start_event` right before and `stop_event`

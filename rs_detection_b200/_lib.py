@@ -69,6 +69,9 @@ SIGNATURES = {
                                                         _vp, _vp, _vp, C.c_size_t, _vp]),
     "rsdet_roi_align_rotated_backward_typed": (C.c_int, [C.POINTER(RoiAlignCfg), C.c_int, _vp, _vp, C.c_int, C.c_int,
                                                          C.POINTER(_vp), _vp, C.c_size_t, _vp]),
+    "rsdet_roi_align_rotated_backward_deterministic_workspace_bytes": (C.c_size_t, [C.POINTER(RoiAlignCfg), C.c_int, C.c_int]),
+    "rsdet_roi_align_rotated_backward_deterministic": (C.c_int, [C.POINTER(RoiAlignCfg), C.c_int, _vp, _vp, C.c_int, C.c_int,
+                                                                 C.POINTER(_vp), _vp, C.c_size_t, _vp]),
     "rsdet_oriented_head_results_workspace_bytes": (C.c_size_t, [C.c_int]),
     "rsdet_oriented_head_results": (C.c_int, [_vp, _vp, _vp, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_float), C.POINTER(C.c_float),
                                               C.c_float, C.POINTER(C.c_float), C.c_float, C.c_int, _vp, _vp, _vp, _vp, C.c_size_t,

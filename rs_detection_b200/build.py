@@ -29,6 +29,7 @@ UNITS = {
     "head.cu": ["-fmad=false"],
     "rpn.cu": ["-fmad=false"],
     "roi_align.cu": ["-DRSDET_BULK_ROWS=" + os.environ.get("RSDET_BULK_ROWS", "0")],
+    "radix_sort.cu": [],
 }
 # A/B measurement builds only (RSDET_TUNING=1 python -m rs_detection_b200.build --force): lets the environment pick
 # among the kernels of a path.  The shipped library is built without it and reads no environment variable.

@@ -333,9 +333,14 @@ def roi_gather_kernel_ms(cfg: RoiAlignCfg, feats: Sequence[torch.Tensor], rois: 
 
 
 def roi_align_rotated_backward(cfg: RoiAlignCfg, grad_out: torch.Tensor, rois: torch.Tensor, feat_shapes,
-                               feat_dtype: torch.dtype = torch.float32):
+                               feat_dtype: torch.dtype = torch.float32, deterministic: bool = False):
     """-> gradient maps in `feat_dtype` (fp32, fp16 or bf16; accumulated in fp32, rounded once).  A grad_out in fp32 or
-    in `feat_dtype` is read natively, any other dtype is cast to fp32."""
+    in `feat_dtype` is read natively, any other dtype is cast to fp32.
+
+    deterministic=False: the atomic backward (sums in an unspecified order).  deterministic=True: every gradient element
+    is the reference's sequential fp32 sum in the reference's order, the same bits on every run
+    (`rsdet_roi_align_rotated_backward_deterministic`); it needs a fixed sampling grid (sampling_ratio > 0, ValueError
+    otherwise) and at most 2^28 terms K * PH * PW * sampling_ratio^2 * 4 (RuntimeError above)."""
     if feat_dtype not in _ROI_DTYPES:
         raise ValueError(f"RoIAlignRotated: gradient maps can be float32, float16 or bfloat16, not {feat_dtype}")
     if grad_out.dtype in (torch.float32, feat_dtype):
@@ -353,6 +358,13 @@ def roi_align_rotated_backward(cfg: RoiAlignCfg, grad_out: torch.Tensor, rois: t
         grads.append(torch.empty((n, h, w, c) if cfg.channels_last else (n, c, h, w), dtype=feat_dtype, device=dev))
     L = load()
     fdt = _ROI_DTYPES[feat_dtype]
+    if deterministic:
+        wsb = L.rsdet_roi_align_rotated_backward_deterministic_workspace_bytes(C.byref(cfg), K, fdt)
+        ws = workspace(wsb, "roi")
+        check(L.rsdet_roi_align_rotated_backward_deterministic(C.byref(cfg), _ROI_DTYPES[g.dtype], ptr(g), ptr(r), K, fdt,
+                                                               _ptr_array(grads), ptr(ws), ws.numel(), stream_ptr()),
+              "roi_align_rotated_backward (deterministic)")
+        return grads
     wsb = L.rsdet_roi_align_rotated_workspace_bytes_typed(C.byref(cfg), K, 1, fdt)
     ws = workspace(wsb, "roi")
     check(L.rsdet_roi_align_rotated_backward_typed(C.byref(cfg), _ROI_DTYPES[g.dtype], ptr(g), ptr(r), K, fdt, _ptr_array(grads),

@@ -1800,6 +1800,288 @@ extern "C" int rsdet_roi_align_rotated_backward(const rsdet_roi_align_cfg* cfg, 
                                                   reinterpret_cast<void* const*>(grad_feats_host), workspace, workspace_bytes, stream);
 }
 
+// ---------------------------------------------------------------------------------- backward (deterministic)
+// The reference (roi_align_rotated_v1.py:193-298) accumulates every gradient element as one sequential fp32 sum: for a
+// fixed (level, image, channel, pixel) the terms (top * w) / count arrive in the order RoI, bin row, bin column, sample
+// row, sample column, tap (lt, rt, lb, rb).  Entry e = ((roi * nbins + bin) * spb + sample) * 4 + tap enumerates every
+// term in exactly that order, so
+//   1. roi_bwd_det_entries_kernel: one thread per (RoI, bin, sample) writes the sample's four entries: a 32-bit pixel
+//      key over (level, image, y, x) (all ones when the sample is out of range or the weight is 0: such terms add
+//      nothing to a sum that starts at +0), the entry index and the weight;
+//   2. a stable LSD radix sort of (key, entry index) over the key's bits groups the entries by pixel and keeps the
+//      reference's order inside each pixel;
+//   3. grad_out (K, C, bins) is copied bin-major to (K, bins, C), so that a term reads C contiguous values;
+//   4. roi_bwd_det_gather_kernel: one warp per touched pixel, lanes over channels, adds the pixel's terms in sorted
+//      order with separately rounded multiply, divide and add, and stores the C sums once (plain stores, no atomics).
+// Untouched pixels keep the zero fill that precedes step 4; NCHW and fp32-accumulated half maps reuse the output passes
+// of the atomic backward.  Results do not depend on the stream, the launch configuration, the layout or the alignment.
+namespace rsdet {
+
+constexpr long long kDetMaxEntries = 1ll << 28;   // K * PH * PW * sr^2 * 4 (include/rsdet.h)
+constexpr int kDetChannelsPerLane = 8;            // a warp covers 256 channels per walk of a pixel's entries
+
+// radix_sort.cu: stable sort of (key, value) pairs on the key's low `key_bits` bits (CUB, in a unit of its own)
+int sort_pairs_u32(void* tmp, size_t* tmp_bytes, uint32_t* key_a, uint32_t* key_b, int* val_a, int* val_b, int n, int key_bits,
+                   bool* in_b, cudaStream_t st);
+
+struct DetJob {
+    LevelSet L;                                   // geometry only (feat / grad unused)
+    unsigned pix_base[RSDET_MAX_LEVELS + 1];      // key of (level l, image 0, pixel 0): prefix of batch * H * W
+    void* out[RSDET_MAX_LEVELS];                  // channels-last destinations (fp32 accumulators or the caller's maps)
+    unsigned sentinel;                            // key of a term that is dropped; sorts after every pixel
+};
+
+__global__ void __launch_bounds__(256) roi_bwd_det_entries_kernel(DetJob J, const float* __restrict__ rois, int K,
+                                                                  uint32_t* __restrict__ keys, int* __restrict__ idx,
+                                                                  float* __restrict__ wts) {
+    const LevelSet& L = J.L;
+    const int spb = L.sampling_ratio * L.sampling_ratio, per_roi = L.PH * L.PW * spb;
+    const long long total = (long long)K * per_roi;
+    for (long long s = (long long)blockIdx.x * blockDim.x + threadIdx.x; s < total; s += (long long)gridDim.x * blockDim.x) {
+        const int roi = (int)(s / per_roi), r = (int)(s % per_roi);
+        const int bin = r / spb, smp = r % spb;
+        const RoiGeom g = roi_geometry(rois + (size_t)roi * 6, L);
+        float x, y;
+        sample_xy(g, L.version, bin / L.PW, bin % L.PW, smp / L.sampling_ratio, smp % L.sampling_ratio, x, y);
+        const int H = L.H[g.level], W = L.W[g.level];
+        const Taps t = make_taps(H, W, y, x);
+        const bool image_ok = g.batch >= 0 && g.batch < L.batch;
+        const unsigned base = J.pix_base[g.level] + (unsigned)g.batch * (unsigned)(H * W);
+        uint4 k, e;
+        k.x = image_ok && t.w[0] != 0.f ? base + t.o[0] : J.sentinel;
+        k.y = image_ok && t.w[1] != 0.f ? base + t.o[1] : J.sentinel;
+        k.z = image_ok && t.w[2] != 0.f ? base + t.o[2] : J.sentinel;
+        k.w = image_ok && t.w[3] != 0.f ? base + t.o[3] : J.sentinel;
+        const unsigned e0 = (unsigned)(4 * s);
+        e.x = e0; e.y = e0 + 1; e.z = e0 + 2; e.w = e0 + 3;
+        reinterpret_cast<uint4*>(keys)[s] = k;
+        reinterpret_cast<uint4*>(idx)[s] = e;
+        reinterpret_cast<float4*>(wts)[s] = make_float4(t.w[0], t.w[1], t.w[2], t.w[3]);
+    }
+}
+
+// (p / count) rounded once to fp32, without the subroutine call of the fp32 division (whose calling convention costs the
+// gather kernel spills): the fp64 product with rd = 1/count rounded, one exact-remainder correction (fp64 fma) that
+// makes it p / count rounded to fp64, then the rounding to fp32.  fp64 carries more than 2 * 24 + 2 bits, so rounding
+// a quotient twice equals rounding it once; p is finite here and p / count stays far inside the fp64 range.
+__device__ __forceinline__ float div_by_count(float p, double count, double rcp) {
+    const double q = __dmul_rn((double)p, rcp);
+    const double r = __fma_rn(-q, count, (double)p);
+    return p == 0.f ? p : __double2float_rn(__fma_rn(r, rcp, q));
+}
+
+// top: (K, bins, C) fp32.  Warp w scans the sorted keys in chunks of 32 positions (grid-stride) and takes every run that
+// starts in its chunk; a run is walked in batches of 32 entries whose (entry, weight) pairs the lanes load together.
+template <typename O, bool POW2>
+__global__ void __launch_bounds__(256) roi_bwd_det_gather_kernel(DetJob J, const uint32_t* __restrict__ keys,
+                                                                 const int* __restrict__ idx, const float* __restrict__ wts,
+                                                                 const float* __restrict__ top, int E) {
+    const int lane = threadIdx.x & 31;
+    const int warp = (int)((blockIdx.x * blockDim.x + threadIdx.x) >> 5), nwarps = (int)((gridDim.x * blockDim.x) >> 5);
+    const int C = J.L.C, spb = J.L.sampling_ratio * J.L.sampling_ratio;
+    const float inv_count = 1.f / (float)spb;   // POW2: x * 2^-k is x / 2^k rounded once, the same bits as the division
+    const double count_d = (double)spb, rcp_d = 1.0 / count_d;
+    for (long long c0 = 32ll * warp; c0 < E; c0 += 32ll * nwarps) {
+        const int p = (int)c0 + lane;
+        const unsigned k = p < E ? __ldg(keys + p) : J.sentinel;
+        if (__shfl_sync(~0u, k, 0) == J.sentinel) break;          // sorted: only dropped terms from here on
+        const unsigned prev = p > 0 && p < E ? __ldg(keys + p - 1) : ~k;
+        unsigned starts = __ballot_sync(~0u, k != J.sentinel && prev != k);
+        while (starts) {
+            const int s = (int)c0 + __ffs(starts) - 1;
+            const unsigned key = __shfl_sync(~0u, k, __ffs(starts) - 1);
+            starts &= starts - 1;
+            unsigned base = J.pix_base[0];     // the key's level, with constant indices only (no local copy of J)
+            void* out = J.out[0];
+#pragma unroll
+            for (int l = 1; l < RSDET_MAX_LEVELS; l++)
+                if (l < J.L.num_levels && key >= J.pix_base[l]) { base = J.pix_base[l]; out = J.out[l]; }
+            O* __restrict__ dst = static_cast<O*>(out) + (size_t)(key - base) * C;
+            for (int cb = 0; cb < C; cb += 32 * kDetChannelsPerLane) {
+                float acc[kDetChannelsPerLane];
+#pragma unroll
+                for (int u = 0; u < kDetChannelsPerLane; u++) acc[u] = 0.f;
+                for (int j0 = s;; j0 += 32) {
+                    const int j = j0 + lane;
+                    const bool in = j < E && __ldg(keys + j) == key;
+                    const unsigned m = __ballot_sync(~0u, in);     // the run is a prefix of the batch
+                    int rb = 0;
+                    float w = 0.f;
+                    if (in) {
+                        const int e = __ldg(idx + j);
+                        rb = e / (4 * spb);                         // roi * bins + bin
+                        w = __ldg(wts + e);
+                    }
+                    const int n = __popc(m);
+#pragma unroll 4
+                    for (int t = 0; t < n; t++) {
+                        const int rbt = __shfl_sync(~0u, rb, t);
+                        const float wt = __shfl_sync(~0u, w, t);
+                        const float* __restrict__ src = top + (size_t)rbt * C + cb + lane;
+#pragma unroll
+                        for (int u = 0; u < kDetChannelsPerLane; u++) {
+                            if (cb + lane + 32 * u < C) {
+                                const float pr = __fmul_rn(__ldg(src + 32 * u), wt);
+                                acc[u] = __fadd_rn(acc[u], POW2 ? __fmul_rn(pr, inv_count) : div_by_count(pr, count_d, rcp_d));
+                            }
+                        }
+                    }
+                    if (n < 32) break;
+                }
+#pragma unroll
+                for (int u = 0; u < kDetChannelsPerLane; u++)
+                    if (cb + lane + 32 * u < C) dst[cb + lane + 32 * u] = from_f32<O>(acc[u]);
+            }
+        }
+    }
+}
+
+// Sizes of one call; false when the call is outside the contract (adaptive grid, entry or pixel count too large).
+struct DetPlan {
+    long long entries;      // K * bins * sr^2 * 4
+    long long pixels;       // batch * sum of H * W: the key space
+    int key_bits;
+    size_t cub_bytes;       // bound on the radix sort's temporary storage
+};
+static bool det_plan(const rsdet_roi_align_cfg* c, int num_rois, DetPlan* p) {
+    if (c->sampling_ratio <= 0 || num_rois < 0) return false;
+    const long long bins = (long long)c->pooled_h * c->pooled_w;
+    if (c->sampling_ratio > 1 << 14 || bins > kDetMaxEntries) return false;       // no overflow below
+    const long long per_roi = bins * c->sampling_ratio * c->sampling_ratio * 4;
+    if (per_roi > kDetMaxEntries) return false;
+    p->entries = per_roi * num_rois;
+    if (p->entries > kDetMaxEntries) return false;
+    // tiles of the bin-major copy of grad_out (one launch, int tile indices)
+    if ((long long)num_rois * ((bins + 63) / 64) * ((c->channels + 63) / 64) > 0x7fffffffll) return false;
+    p->pixels = 0;
+    for (int l = 0; l < c->num_levels; l++) p->pixels += (long long)c->batch * c->height[l] * c->width[l];
+    if (p->pixels > 0xfffffffell) return false;     // every key below the all-ones sentinel
+    p->key_bits = 1;
+    while (p->key_bits < 32 && (1ll << p->key_bits) <= p->pixels) p->key_bits++;
+    // onesweep: a few KB of bins and counters plus one 256-digit lookback row per tile of thousands of items
+    p->cub_bytes = ((size_t)1 << 20) + 2 * (size_t)p->entries;
+    return true;
+}
+
+static size_t det_workspace_bytes(const rsdet_roi_align_cfg* c, int num_rois, const DetPlan& p) {
+    const size_t E = (size_t)(p.entries > 0 ? p.entries : 1);
+    size_t b = 4 * ws_bytes<uint32_t>(E) + ws_bytes<float>(E);        // keys x2, entry indices x2, weights
+    b += ws_bytes<float>((size_t)(num_rois > 0 ? num_rois : 1) * c->pooled_h * c->pooled_w * c->channels);   // bin-major grad_out
+    if (!c->channels_last)                                             // fp32 NHWC accumulators
+        for (int l = 0; l < c->num_levels; l++) b += ws_bytes<float>((size_t)c->batch * c->channels * c->height[l] * c->width[l]);
+    return b + align256(p.cub_bytes) + 256;
+}
+
+template <typename G, typename T>
+static int backward_det_impl(const rsdet_roi_align_cfg* cfg, const DetPlan& plan, const G* grad_out, const float* rois,
+                             int num_rois, T* const* grad_feats_host, void* workspace, size_t workspace_bytes, cudaStream_t st) {
+    auto map_bytes = [&](int l) { return sizeof(T) * (size_t)cfg->batch * cfg->channels * cfg->height[l] * cfg->width[l]; };
+    if (num_rois == 0) {     // nothing to sum: zero maps
+        for (int l = 0; l < cfg->num_levels; l++) cudaMemsetAsync(grad_feats_host[l], 0, map_bytes(l), st);
+        count_launch(cfg->num_levels);
+        return cuda_status();
+    }
+    if (workspace_bytes < det_workspace_bytes(cfg, num_rois, plan)) return RSDET_EWORKSPACE;
+    const int E = (int)plan.entries, nbins = cfg->pooled_h * cfg->pooled_w;
+    Workspace ws(workspace, workspace_bytes);
+    uint32_t* keyA = ws.take<uint32_t>(E);
+    uint32_t* keyB = ws.take<uint32_t>(E);
+    int* idxA = ws.take<int>(E);
+    int* idxB = ws.take<int>(E);
+    float* wts = ws.take<float>(E);
+    float* top = ws.take<float>((size_t)num_rois * nbins * cfg->channels);
+    float* acc[RSDET_MAX_LEVELS];
+    if (!cfg->channels_last)
+        for (int l = 0; l < cfg->num_levels; l++) acc[l] = ws.take<float>((size_t)cfg->batch * cfg->channels * cfg->height[l] * cfg->width[l]);
+    void* cub_tmp = ws.take<char>(plan.cub_bytes);
+    if (!ws.ok()) return RSDET_EWORKSPACE;
+    size_t need = 0;
+    int rc = sort_pairs_u32(nullptr, &need, keyA, keyB, idxA, idxB, E, plan.key_bits, nullptr, st);
+    if (rc != RSDET_OK) return rc;
+    if (need > plan.cub_bytes) return RSDET_EWORKSPACE;
+
+    DetJob J;
+    J.L = make_levels(cfg);
+    J.sentinel = plan.key_bits == 32 ? 0xffffffffu : (1u << plan.key_bits) - 1;
+    unsigned base = 0;
+    for (int l = 0; l <= RSDET_MAX_LEVELS; l++) {
+        J.pix_base[l] = base;
+        if (l < cfg->num_levels) base += (unsigned)((size_t)cfg->batch * cfg->height[l] * cfg->width[l]);
+        if (l < RSDET_MAX_LEVELS) J.out[l] = l < cfg->num_levels ? (cfg->channels_last ? (void*)grad_feats_host[l] : (void*)acc[l]) : nullptr;
+    }
+    // zero fill of whatever the gather writes into; an NCHW caller's maps are written whole by the transpose
+    for (int l = 0; l < cfg->num_levels; l++) {
+        if (cfg->channels_last) cudaMemsetAsync(grad_feats_host[l], 0, map_bytes(l), st);
+        else cudaMemsetAsync(acc[l], 0, sizeof(float) * (size_t)cfg->batch * cfg->channels * cfg->height[l] * cfg->width[l], st);
+    }
+    count_launch(cfg->num_levels);
+    const long long samples = plan.entries / 4;
+    roi_bwd_det_entries_kernel<<<(unsigned)(ceil_div_ll(samples, 256) < kNumSMs * 16 ? ceil_div_ll(samples, 256) : kNumSMs * 16),
+                                 256, 0, st>>>(J, rois, num_rois, keyA, idxA, wts);
+    count_launch();
+    // bin-major copy of grad_out: the NCHW -> NHWC transpose with K images of PH x PW pixels
+    TransposeJob tj;
+    tj.num_levels = 1; tj.N = num_rois; tj.C = cfg->channels;
+    tj.src[0] = grad_out; tj.dst[0] = top; tj.HW[0] = nbins;
+    tj.tile_begin[0] = 0;
+    tj.tile_begin[1] = num_rois * ceil_div(nbins, 64) * ceil_div(cfg->channels, 64);
+    transpose_kernel<G, float, true><<<tj.tile_begin[1], 256, 0, st>>>(tj);
+    count_launch();
+    bool in_b = false;
+    rc = sort_pairs_u32(cub_tmp, &need, keyA, keyB, idxA, idxB, E, plan.key_bits, &in_b, st);
+    if (rc != RSDET_OK) return rc;
+    count_launch(2 + ceil_div(plan.key_bits, 8));
+    const uint32_t* keys = in_b ? keyB : keyA;
+    const int* idx = in_b ? idxB : idxA;
+    const long long chunks = ceil_div_ll(E, 32);
+    const unsigned blocks = (unsigned)(ceil_div_ll(chunks, 8) < kNumSMs * 8 ? ceil_div_ll(chunks, 8) : kNumSMs * 8);
+    const int spb = cfg->sampling_ratio * cfg->sampling_ratio;
+    const bool pow2 = (spb & (spb - 1)) == 0;
+    if (cfg->channels_last && pow2) roi_bwd_det_gather_kernel<T, true><<<blocks, 256, 0, st>>>(J, keys, idx, wts, top, E);
+    else if (cfg->channels_last) roi_bwd_det_gather_kernel<T, false><<<blocks, 256, 0, st>>>(J, keys, idx, wts, top, E);
+    else if (pow2) roi_bwd_det_gather_kernel<float, true><<<blocks, 256, 0, st>>>(J, keys, idx, wts, top, E);
+    else roi_bwd_det_gather_kernel<float, false><<<blocks, 256, 0, st>>>(J, keys, idx, wts, top, E);
+    count_launch();
+    if (!cfg->channels_last) {
+        rc = launch_transpose(false, acc, grad_feats_host, cfg->height, cfg->width, cfg->num_levels, cfg->batch,
+                                        cfg->channels, st);
+        if (rc != RSDET_OK) return rc;
+    }
+    return cuda_status();
+}
+
+}  // namespace rsdet
+
+extern "C" size_t rsdet_roi_align_rotated_backward_deterministic_workspace_bytes(const rsdet_roi_align_cfg* cfg, int num_rois,
+                                                                                 int feat_dtype) {
+    DetPlan plan;
+    if (!dtype_ok(feat_dtype) || check_cfg(cfg) != RSDET_OK || !det_plan(cfg, num_rois, &plan)) return 0;
+    return det_workspace_bytes(cfg, num_rois, plan);
+}
+
+extern "C" int rsdet_roi_align_rotated_backward_deterministic(const rsdet_roi_align_cfg* cfg, int grad_out_dtype,
+                                                              const void* grad_out, const float* rois, int num_rois,
+                                                              int feat_dtype, void* const* grad_feats_host, void* workspace,
+                                                              size_t workspace_bytes, void* stream) {
+    if (!dtype_ok(feat_dtype) || (grad_out_dtype != RSDET_DTYPE_F32 && grad_out_dtype != feat_dtype)) return RSDET_EINVAL;
+    int rc = check_cfg(cfg);
+    if (rc != RSDET_OK) return rc;
+    if (cfg->sampling_ratio <= 0 || num_rois < 0 || !grad_feats_host) return RSDET_EINVAL;
+    for (int l = 0; l < cfg->num_levels; l++)
+        if (!grad_feats_host[l]) return RSDET_EINVAL;
+    DetPlan plan;
+    if (!det_plan(cfg, num_rois, &plan)) return RSDET_ELIMIT;
+    if (num_rois > 0 && (!grad_out || !rois)) return RSDET_EINVAL;
+    cudaStream_t st = (cudaStream_t)stream;
+    const bool half_g = grad_out_dtype != RSDET_DTYPE_F32;
+#define RSDET_BWD_DET(G_, T_) backward_det_impl<G_, T_>(cfg, plan, static_cast<const G_*>(grad_out), rois, num_rois, \
+                                                        reinterpret_cast<T_* const*>(grad_feats_host), workspace, workspace_bytes, st)
+    if (feat_dtype == RSDET_DTYPE_F16) return half_g ? RSDET_BWD_DET(__half, __half) : RSDET_BWD_DET(float, __half);
+    if (feat_dtype == RSDET_DTYPE_BF16) return half_g ? RSDET_BWD_DET(__nv_bfloat16, __nv_bfloat16) : RSDET_BWD_DET(float, __nv_bfloat16);
+    return RSDET_BWD_DET(float, float);
+#undef RSDET_BWD_DET
+}
+
 #ifdef RSDET_PROF
 // profiling builds only: device buffer of 8 counters filled by roi_align_fwd_px_kernel (per-phase cycle sums)
 extern "C" int rsdet_tuning_set_prof(unsigned long long* dev_counters) {

@@ -10,7 +10,7 @@ from torch import nn
 
 from .... import core
 from ...ops import roi_align_rotated_v1
-from ...ops.roi_align_rotated_v1 import _grad_dtype
+from ...ops.roi_align_rotated_v1 import _deterministic_backward, _grad_dtype
 
 
 def _pair(x):
@@ -29,7 +29,9 @@ class _FusedExtractFn(torch.autograd.Function):
     @staticmethod
     def backward(ctx, grad_output):
         (rois,) = ctx.saved_tensors
-        grads = core.roi_align_rotated_backward(ctx.cfg, grad_output.contiguous(), rois, ctx.shapes, feat_dtype=ctx.dtype)
+        det = _deterministic_backward(ctx.cfg, "RoI extractor (RoIAlignRotated)")
+        grads = core.roi_align_rotated_backward(ctx.cfg, grad_output.contiguous(), rois, ctx.shapes, feat_dtype=ctx.dtype,
+                                                deterministic=det)
         return (None, None, *grads)
 
 

@@ -4,6 +4,8 @@
 configs (`getattr(roi_align_rotated_v1, layer_type)`, oriented_single_level.py:43-51), so class name,
 constructor arguments, the `output_size` tuple attribute and `__repr__` are kept verbatim.
 """
+import warnings
+
 import torch
 from torch import nn
 
@@ -21,6 +23,24 @@ def _grad_dtype(dtype):
     return dtype if dtype in (torch.float16, torch.bfloat16) else torch.float32
 
 
+def _deterministic_backward(cfg, op):
+    """Whether the backward of `op` runs the ordered (bitwise reproducible) kernel: under
+    `torch.use_deterministic_algorithms(True)`.  The adaptive sampling grid (sampling_ratio <= 0) has no deterministic
+    kernel; like torch's own ops it then raises RuntimeError, or with `warn_only=True` warns and runs the atomic one."""
+    if not torch.are_deterministic_algorithms_enabled():
+        return False
+    if cfg.sampling_ratio > 0:
+        return True
+    msg = (f"{op} backward with sampling_ratio <= 0 (adaptive sampling grid) does not have a deterministic implementation, "
+           "but you set 'torch.use_deterministic_algorithms(True)'. You can turn off determinism just for this operation, "
+           "or you can use the 'warn_only=True' option, if that's acceptable for your application. You can also use a "
+           "fixed sampling_ratio > 0, whose backward is deterministic.")
+    if torch.is_deterministic_algorithms_warn_only_enabled():
+        warnings.warn(msg, UserWarning)
+        return False
+    raise RuntimeError(msg)
+
+
 class _RotatedROIAlignFn(torch.autograd.Function):
     """Forward + backward of one feature map (the reference's jt.Function, :300-351); rois get no grad.  The output is
     fp32 whatever the input's dtype, like the reference's float kernels."""
@@ -36,7 +56,9 @@ class _RotatedROIAlignFn(torch.autograd.Function):
     @staticmethod
     def backward(ctx, grad_output):
         (rois,) = ctx.saved_tensors
-        grads = core.roi_align_rotated_backward(ctx.cfg, grad_output.contiguous(), rois, [ctx.shape], feat_dtype=ctx.dtype)
+        det = _deterministic_backward(ctx.cfg, "ROIAlignRotated_v1" if ctx.cfg.version == 1 else "ROIAlignRotated")
+        grads = core.roi_align_rotated_backward(ctx.cfg, grad_output.contiguous(), rois, [ctx.shape], feat_dtype=ctx.dtype,
+                                                deterministic=det)
         return grads[0], None, None, None, None, None
 
 
