@@ -28,17 +28,9 @@ UNITS = {
     "transforms.cu": ["-fmad=false"],
     "head.cu": ["-fmad=false"],
     "rpn.cu": ["-fmad=false"],
-    "roi_align.cu": ["-DRSDET_BULK_ROWS=" + os.environ.get("RSDET_BULK_ROWS", "0")],
+    "roi_align.cu": [],
     "radix_sort.cu": [],
 }
-# A/B measurement builds only (RSDET_TUNING=1 python -m rs_detection_b200.build --force): lets the environment pick
-# among the kernels of a path.  The shipped library is built without it and reads no environment variable.
-if os.environ.get("RSDET_TUNING") == "1":
-    COMMON = COMMON + ["-DRSDET_TUNING"]
-if os.environ.get("RSDET_SCAN_PROF") == "1":   # clock64 phase stamps of reduce_ov_pipe_kernel, printed from the device
-    COMMON = COMMON + ["-DRSDET_SCAN_PROF"]
-if os.environ.get("RSDET_PROF") == "1":   # clock64 phase counters in the one-CTA-per-RoI RoI kernel (tools/roi_sweep.py --prof)
-    COMMON = COMMON + ["-DRSDET_PROF"]
 
 
 def _deps():

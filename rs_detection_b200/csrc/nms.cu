@@ -1286,14 +1286,8 @@ reduce_ov_pipe_kernel(SegTable tb, const int* __restrict__ idx_ls, int cand_per_
         if (nblk > 2) fetch(2);                     // in flight during iteration 0
         __syncthreads();
         int kept_run = 0;
-#ifdef RSDET_SCAN_PROF
-        long long t_p1 = 0, t_b1 = 0, t_p2a = 0, t_p2b = 0, t_b2 = 0, t0, t1;
-#endif
         for (int b = 0; b < nblk; b++) {
             const int nr = min(64, ns - b * 64);
-#ifdef RSDET_SCAN_PROF
-            t0 = clock64();
-#endif
             if (warp == 0) {
                 // greedy resolve as a fixed point (see reduce_ov_staged_kernel)
                 unsigned long long col[2];
@@ -1329,13 +1323,7 @@ reduce_ov_pipe_kernel(SegTable tb, const int* __restrict__ idx_ls, int cand_per_
                 colmask_warp<NW - 1>(s_rows + (size_t)((b + 1) % 3) * 64 * Ts, Ts, s_cand + (b + 1) * 64,
                                                       min(64, ns - (b + 1) * 64), warp - 1, lane, s_colmask[(b + 1) & 1]);
             }
-#ifdef RSDET_SCAN_PROF
-            t1 = clock64(); t_p1 += t1 - t0; t0 = t1;
-#endif
             __syncthreads();
-#ifdef RSDET_SCAN_PROF
-            t1 = clock64(); t_b1 += t1 - t0; t0 = t1;
-#endif
             const unsigned long long kb = s_keep;
             if (tid < nr) {
                 keep_sorted[st + b * 64 + tid] = (uint8_t)((kb >> tid) & 1ull);
@@ -1367,24 +1355,10 @@ reduce_ov_pipe_kernel(SegTable tb, const int* __restrict__ idx_ls, int cand_per_
                     }
                 }
             }
-#ifdef RSDET_SCAN_PROF
-            t1 = clock64(); t_p2a += t1 - t0; t0 = t1;
-#endif
             if (b + 2 < nblk) stash(b + 2);
             if (b + 3 < nblk) fetch(b + 3);
-#ifdef RSDET_SCAN_PROF
-            t1 = clock64(); t_p2b += t1 - t0; t0 = t1;
-#endif
             __syncthreads();
-#ifdef RSDET_SCAN_PROF
-            t1 = clock64(); t_b2 += t1 - t0;
-#endif
         }
-#ifdef RSDET_SCAN_PROF
-        if (s == 0 && (tid == 0 || tid == 32 || tid == 224) && nblk > 0)
-            printf("scan prof tid %d nblk %d: per block cycles: phase1 %lld, barrier1 %lld, keep+OR %lld, stash+fetch %lld, barrier2 %lld\n", tid, nblk,
-                   t_p1 / nblk, t_b1 / nblk, t_p2a / nblk, t_p2b / nblk, t_b2 / nblk);
-#endif
         if (kept_count && tid == 0) kept_count[s] = kept_run;
     }
 }
@@ -2422,13 +2396,6 @@ static SideLane* side_lane(cudaStream_t user) {
     return &lanes->back().lane;
 }
 
-static bool mc_force_generic() {   // A/B builds only: RSDET_MC_GENERIC=1 keeps the generic engine for this entry point
-#ifdef RSDET_TUNING
-    return getenv("RSDET_MC_GENERIC") != nullptr;
-#else
-    return false;
-#endif
-}
 static bool mc_fast_ok(int bbox_dim, int n, int C) {
     return bbox_dim == 5 && n >= 1 && n <= kMcFastMaxBoxes && C <= kMcFastMaxClasses;
 }
@@ -2526,7 +2493,7 @@ extern "C" int rsdet_multiclass_nms_rotated(const float* multi_bboxes, int bbox_
     if (capll > (1 << 20) || n > kMaxNmsBoxes) return RSDET_ELIMIT;
     int cap = (int)capll;
     if (workspace_bytes < rsdet_multiclass_nms_rotated_workspace_bytes(n, num_classes)) return RSDET_EWORKSPACE;
-    if (mc_fast_ok(bbox_dim, n, num_classes) && !mc_force_generic())
+    if (mc_fast_ok(bbox_dim, n, num_classes))
         return mc_fast_run(multi_bboxes, multi_scores, n, num_classes, score_thr, iou_thr, max_num, score_factors, out_dets, out_labels,
                            out_count, workspace, workspace_bytes, st);
     Workspace ws(workspace, workspace_bytes);

@@ -30,11 +30,9 @@
 // kernel below is templated on them; a half value is converted exactly to fp32 where it is read, the arithmetic is the
 // fp32 arithmetic unchanged, and a half result is rounded once, to nearest-even, where it is stored.  Four consecutive
 // channels are the unit of every vector access: a float4 (16 bytes) or four 2-byte values (8 bytes).
-#include <cuda.h>
 #include <cuda_bf16.h>
 #include <cuda_fp16.h>
 
-#include <cstdlib>
 #include <mutex>
 #include <type_traits>
 
@@ -98,9 +96,6 @@ struct LevelSet {
     int num_levels, batch, C;
     int PH, PW, sampling_ratio, version;
     float extend_w, extend_h, finest_scale;
-    int dbg_drop;       // profiling aid (RSDET_ROI_DBG_DROP, RSDET_TUNING builds only)
-    unsigned dbg_mask;  // profiling aid (RSDET_ROI_DBG_MASK, RSDET_TUNING builds only): tap offsets are ANDed with it (shrinks the gather's footprint)
-    int dbg_skip_main;  // profiling aid (RSDET_ROI_DBG_SKIP_MAIN=1, RSDET_TUNING builds only): tap lists are built, then treated as empty
 };
 template <typename T> __device__ __forceinline__ const T* feat_base(const LevelSet& L, int level) {
     return reinterpret_cast<const T*>(L.feat[level]);
@@ -310,20 +305,6 @@ __device__ __forceinline__ const float* tap_ptr(const float4* base, unsigned off
     asm("mad.wide.u32 %0, %1, 16, %2;" : "=l"(a) : "r"(off16), "l"((unsigned long long)base));
     return reinterpret_cast<const float*>(a);
 }
-__device__ __forceinline__ float4 ldg_nc_v4(const float* p) {
-    float4 r;
-    asm volatile("ld.global.nc.v4.f32 {%0,%1,%2,%3}, [%4];" : "=f"(r.x), "=f"(r.y), "=f"(r.z), "=f"(r.w) : "l"(p));
-    return r;
-}
-template <int FLAVOUR>   // A/B builds: 0 nc, 1 nc + L1::no_allocate, 2 nc + L1::evict_first, 3 plain ld.global.cg
-__device__ __forceinline__ float4 ldg_flavour_v4(const float* p) {
-    float4 r;
-    if (FLAVOUR == 1) asm volatile("ld.global.nc.L1::no_allocate.v4.f32 {%0,%1,%2,%3}, [%4];" : "=f"(r.x), "=f"(r.y), "=f"(r.z), "=f"(r.w) : "l"(p));
-    else if (FLAVOUR == 2) asm volatile("ld.global.nc.L1::evict_first.v4.f32 {%0,%1,%2,%3}, [%4];" : "=f"(r.x), "=f"(r.y), "=f"(r.z), "=f"(r.w) : "l"(p));
-    else if (FLAVOUR == 3) asm volatile("ld.global.cg.v4.f32 {%0,%1,%2,%3}, [%4];" : "=f"(r.x), "=f"(r.y), "=f"(r.z), "=f"(r.w) : "l"(p));
-    else asm volatile("ld.global.nc.v4.f32 {%0,%1,%2,%3}, [%4];" : "=f"(r.x), "=f"(r.y), "=f"(r.z), "=f"(r.w) : "l"(p));
-    return r;
-}
 // base + off * sizeof(Quad<T>::V) as ONE mad.wide.u32: tap offsets count 4-channel units of a channels-last map
 template <typename T>
 __device__ __forceinline__ const T* quad_ptr(const typename Quad<T>::V* base, unsigned off) {
@@ -331,33 +312,31 @@ __device__ __forceinline__ const T* quad_ptr(const typename Quad<T>::V* base, un
     asm("mad.wide.u32 %0, %1, %2, %3;" : "=l"(a) : "r"(off), "n"((int)sizeof(typename Quad<T>::V)), "l"((unsigned long long)base));
     return reinterpret_cast<const T*>(a);
 }
-// four channels at p as fp32 through the non-coherent path: one 16-byte load (fp32, FLAVOUR as above) or one 8-byte load
-template <typename T, int FLAVOUR = 0>
-__device__ __forceinline__ float4 ldg4(const T* p) {
-    if constexpr (kIsF32<T>) {
-        return ldg_flavour_v4<FLAVOUR>(p);
-    } else {
-        uint2 u;
-        asm volatile("ld.global.nc.v2.b32 {%0,%1}, [%2];" : "=r"(u.x), "=r"(u.y) : "l"(p));
-        return unpack4<T>(u);
-    }
-}
-// the same load without the conversion (raw vector), and the conversion: lets a loop keep 2-byte values in flight
-template <typename T, int FLAVOUR = 0>
+// four channels at p through the non-coherent path as the raw vector: one 16-byte load (fp32) or one 8-byte load
+template <typename T>
 __device__ __forceinline__ typename Quad<T>::V ldg4_raw(const T* p) {
     if constexpr (kIsF32<T>) {
-        return ldg_flavour_v4<FLAVOUR>(p);
+        float4 r;
+        asm volatile("ld.global.nc.v4.f32 {%0,%1,%2,%3}, [%4];" : "=f"(r.x), "=f"(r.y), "=f"(r.z), "=f"(r.w) : "l"(p));
+        return r;
     } else {
         uint2 u;
         asm volatile("ld.global.nc.v2.b32 {%0,%1}, [%2];" : "=r"(u.x), "=r"(u.y) : "l"(p));
         return u;
     }
 }
+// the conversion of a raw vector to fp32: a loop that keeps 2-byte values in flight converts right before their FMAs
 template <typename T> __device__ __forceinline__ decltype(auto) quad_f32(const typename Quad<T>::V& v) {
     if constexpr (kIsF32<T>) return (v);    // a reference: the fp32 kernels compile exactly as without this step
     else return unpack4<T>(v);
 }
-__device__ __forceinline__ float4 ldg_cs_v4(const float* p);
+// the same load as fp32
+template <typename T> __device__ __forceinline__ float4 ldg4(const T* p) { return quad_f32<T>(ldg4_raw(p)); }
+__device__ __forceinline__ float4 ldg_cs_v4(const float* p) {
+    float4 r;
+    asm volatile("ld.global.cs.v4.f32 {%0,%1,%2,%3}, [%4];" : "=f"(r.x), "=f"(r.y), "=f"(r.z), "=f"(r.w) : "l"(p));
+    return r;
+}
 template <typename T>
 __device__ __forceinline__ float4 ldcs4(const T* p) {     // streaming 4-channel load
     if constexpr (kIsF32<T>) {
@@ -372,14 +351,6 @@ template <typename T>
 __device__ __forceinline__ void stcs1(T* p, T v) {           // streaming scalar store
     if constexpr (kIsF32<T>) __stcs(p, v);
     else asm volatile("st.global.cs.b16 [%0], %1;" ::"l"(p), "h"(*reinterpret_cast<const unsigned short*>(&v)) : "memory");
-}
-__device__ __forceinline__ void stg_cs_v4(float* p, float4 v) {
-    asm volatile("st.global.cs.v4.f32 [%0], {%1,%2,%3,%4};" ::"l"(p), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w) : "memory");
-}
-__device__ __forceinline__ float4 ldg_cs_v4(const float* p) {
-    float4 r;
-    asm volatile("ld.global.cs.v4.f32 {%0,%1,%2,%3}, [%4];" : "=f"(r.x), "=f"(r.y), "=f"(r.z), "=f"(r.w) : "l"(p));
-    return r;
 }
 // shared -> global bulk copy (cp.async.bulk, SASS UBLKCP) with an evict-first L2 policy: the output stream must
 // not push the feature pyramid out of L2.  Returns once the source has been read (shared memory may be reused
@@ -407,18 +378,13 @@ __host__ __device__ inline int quads_per_chunk(int C) { return (C / 4) < 64 ? (C
 // sin/cos/log2/sqrt and six divisions per RoI: done by K parallel threads here instead of by thread 0 of
 // every RoI's CTA (a ~1.5 us serial chain in front of each CTA's barrier).
 __global__ void roi_geometry_kernel(LevelSet L, const float* __restrict__ rois, int K, const int* __restrict__ order,
-                                    RoiGeom* __restrict__ geoms, RoiGeom* __restrict__ gsorted, int32_t* __restrict__ levels_out) {
+                                    RoiGeom* __restrict__ geoms, int32_t* __restrict__ levels_out) {
     const int p = blockIdx.x * blockDim.x + threadIdx.x;   // position in processing order
     if (p >= K) return;
-    // record K of gsorted holds the work counter of the persistent forward kernel, which runs after this one
-    if (p == 0 && gsorted) *reinterpret_cast<unsigned*>(gsorted + K) = 0u;
     const int i = order ? order[p] : p;
-    RoiGeom g = roi_geometry(rois + (size_t)i * 6, L);
+    const RoiGeom g = roi_geometry(rois + (size_t)i * 6, L);
     geoms[i] = g;
     if (levels_out) levels_out[i] = g.level;
-    // gsorted: the records in processing order with the RoI index in `gh` (the fast kernels know the sampling grid from
-    // the configuration): a gather CTA then starts with ONE global round trip instead of order[blockIdx.x] -> geoms[roi]
-    if (gsorted) { g.gh = i; gsorted[p] = g; }
 }
 
 // ---------------------------------------------------------------------------------- processing order
@@ -634,22 +600,22 @@ static int launch_transpose(bool to_nhwc, const S* const* src, D* const* dst, co
     return cuda_status();
 }
 
-// locality order (calls of >= 256 RoIs) and geometry of a call.  The order comes first: the geometry kernel then writes
-// its records in processing order as well (coalesced).  order_rides_with_transpose: the caller's transpose launch
-// produces the order (block 0) and the caller launches the geometry kernel after it.
-static void launch_geometry(const LevelSet& L, const float* rois, int K, const int* order, RoiGeom* geoms, RoiGeom* gsorted,
-                            int32_t* levels_out, cudaStream_t st) {
-    roi_geometry_kernel<<<ceil_div(K, 128), 128, 0, st>>>(L, rois, K, order, geoms, gsorted, levels_out);
+// locality order (calls of >= 256 RoIs) and geometry of a call.  The order comes first: the geometry kernel takes the
+// RoIs in processing order and writes each record at its RoI index.  order_rides_with_transpose: the caller's transpose
+// launch produces the order (block 0) and the caller launches the geometry kernel after it.
+static void launch_geometry(const LevelSet& L, const float* rois, int K, const int* order, RoiGeom* geoms, int32_t* levels_out,
+                            cudaStream_t st) {
+    roi_geometry_kernel<<<ceil_div(K, 128), 128, 0, st>>>(L, rois, K, order, geoms, levels_out);
     count_launch();
 }
 static void launch_prep(const LevelSet& L, const float* rois, int K, RoiGeom* geoms, int* order, int32_t* levels_out, cudaStream_t st,
-                        bool order_rides_with_transpose = false, RoiGeom* gsorted = nullptr) {
+                        bool order_rides_with_transpose = false) {
     if (order_rides_with_transpose) return;
     if (order) {
         roi_order_kernel<<<1, 1024, 0, st>>>(L, rois, K, order);
         count_launch();
     }
-    launch_geometry(L, rois, K, order, geoms, gsorted, levels_out, st);
+    launch_geometry(L, rois, K, order, geoms, levels_out, st);
 }
 
 // ---------------------------------------------------------------------------------- tap lists
@@ -661,17 +627,14 @@ static void launch_prep(const LevelSet& L, const float* rois, int K, RoiGeom* ge
 // collapse to ~9.  Offsets are in 16-byte units of the channels-last map (one mad.wide per address).
 //   s_list [nbins*(cap+1)] int2 {offset, weight bits} (bin pitch cap + 1: conflict-free per-bin lanes),
 //   s_cnt [nbins], tmp: 3*nbins*(cap+1) words of scratch.
-//   unit/base: stored offset = base + pixel * unit (unit = C/4 for float4 addressing, 1 for TMA row indices)
-// FIXED = true: the 7x7-bin, 2x2-sample geometry as compile-time constants (roi_align_fwd77_kernel)
-// LPITCH = 18 (roi_align_fwd77_kernel): list pitch of 18 entries, i.e. every bin's list starts on a 16-byte boundary (two
-// entries per LDS.128 in the gather loop) and the bin's count lives in the pad entry 16 instead of s_cnt.
-template <int kThreads = kRoiThreads, bool FIXED = false, int LPITCH = 17>
+//   unit: stored offset = pixel * unit (C/4: 4-channel units)
+// Called by all kRoiThreads threads of the CTA.
 __device__ __forceinline__ void build_tap_lists(const RoiGeom& g, const LevelSet& L, int H, int W, int2* s_list, int* s_cnt,
-                                                float* tmp, int unit, int base) {
+                                                float* tmp, int unit) {
     const int tid = threadIdx.x;
-    const int PW_ = FIXED ? 7 : L.PW;
-    const int nbins = FIXED ? 49 : L.PH * L.PW;
-    const int spb = FIXED ? 4 : L.sampling_ratio * L.sampling_ratio;
+    const int PW_ = L.PW;
+    const int nbins = L.PH * L.PW;
+    const int spb = L.sampling_ratio * L.sampling_ratio;
     const int nsamp = nbins * spb, cap = 4 * spb, ntaps = nbins * cap;
     const int C4 = unit;
     int* s_off = reinterpret_cast<int*>(tmp);
@@ -680,7 +643,7 @@ __device__ __forceinline__ void build_tap_lists(const RoiGeom& g, const LevelSet
     // A1: one thread per sample.  Scratch pitch per bin = cap + 1 words when the per-bin merge below reads it
     // with one lane per bin (lane stride 17 words: conflict-free; 16 would be a 16-way bank conflict).
     const int tp = cap == 16 ? 17 : cap;
-    for (int s = tid; s < nsamp; s += kThreads) {
+    for (int s = tid; s < nsamp; s += kRoiThreads) {
         int b = s / spb, q = s % spb;
         int ph = b / PW_, pw = b % PW_, iy = q / g.gw, ix = q % g.gw;
         float x, y;
@@ -688,7 +651,7 @@ __device__ __forceinline__ void build_tap_lists(const RoiGeom& g, const LevelSet
         const Taps t = make_taps(H, W, y, x);
 #pragma unroll
         for (int k = 0; k < 4; k++) {
-            s_off[b * tp + q * 4 + k] = base + t.o[k] * C4;
+            s_off[b * tp + q * 4 + k] = t.o[k] * C4;
             s_w[b * tp + q * 4 + k] = t.w[k];
         }
     }
@@ -700,7 +663,7 @@ __device__ __forceinline__ void build_tap_lists(const RoiGeom& g, const LevelSet
         // of the gather loads, profiles/README.md).  Same arithmetic: a tap is a LEADER if its weight is
         // non-zero and no earlier live tap of the bin hits the same pixel; a leader adds the weights of its
         // later duplicates in tap order; leaders are compacted in tap order.
-        for (int b = tid; b < nbins; b += kThreads) {
+        for (int b = tid; b < nbins; b += kRoiThreads) {
             int o[16];
             float w[16];
 #pragma unroll
@@ -716,17 +679,9 @@ __device__ __forceinline__ void build_tap_lists(const RoiGeom& g, const LevelSet
                     acc += same ? w[i] : 0.f;
                     w[i] = same ? 0.f : w[i];
                 }
-                if (w[j] != 0.f) s_list[b * LPITCH + pos++] = make_int2(o[j], __float_as_int(acc));
+                if (w[j] != 0.f) s_list[b * 17 + pos++] = make_int2(o[j], __float_as_int(acc));
             }
-#ifdef RSDET_TUNING   // what-if: 1 of every `dbg_drop` entries removed (wrong results, timing of a deduplicated list)
-            if (L.dbg_drop > 1) {
-                int q = 0;
-                for (int e = 0; e < pos; e++)
-                    if ((e + b) % L.dbg_drop != 0) s_list[b * LPITCH + q++] = s_list[b * LPITCH + e];
-                pos = q;
-            }
-#endif
-            if (LPITCH == 18) s_list[b * 18 + 16] = make_int2(pos, 0); else s_cnt[b] = pos;
+            s_cnt[b] = pos;
         }
         __syncthreads();
         return;
@@ -737,9 +692,9 @@ __device__ __forceinline__ void build_tap_lists(const RoiGeom& g, const LevelSet
         // sums the weights of all live lanes on its pixel in lane order; a ballot of the leaders gives each
         // one its slot in the bin's compacted list.
         const int lane = tid & 31;
-        const int rounds = (ntaps + kThreads - 1) / kThreads;
+        const int rounds = (ntaps + kRoiThreads - 1) / kRoiThreads;
         for (int rd = 0; rd < rounds; rd++) {
-            const int t = rd * kThreads + tid;
+            const int t = rd * kRoiThreads + tid;
             const bool in = t < ntaps;
             const int b = in ? t / cap : 0, j = in ? t - b * cap : 0;
             const int o = in ? s_off[t] : -1;
@@ -765,7 +720,7 @@ __device__ __forceinline__ void build_tap_lists(const RoiGeom& g, const LevelSet
     }
     // A2a: one thread per tap: a tap is a LEADER if its weight is non-zero and no earlier tap of the bin
     // hits the same pixel; a leader collects the weights of its later duplicates (fixed order).
-    for (int t = tid; t < ntaps; t += kThreads) {
+    for (int t = tid; t < ntaps; t += kRoiThreads) {
         const int b = t / cap, j = t - b * cap;
         const int* ob = s_off + b * cap;
         const float* wb = s_w + b * cap;
@@ -780,7 +735,7 @@ __device__ __forceinline__ void build_tap_lists(const RoiGeom& g, const LevelSet
     }
     __syncthreads();
     // A2b: compaction (position = number of leaders before me in my bin)
-    for (int t = tid; t < ntaps; t += kThreads) {
+    for (int t = tid; t < ntaps; t += kRoiThreads) {
         const int b = t / cap, j = t - b * cap;
         const float* ws = s_wsum + b * cap;
         const float w = ws[j];
@@ -837,12 +792,7 @@ roi_align_fwd_kernel(LevelSet L, const float* __restrict__ rois, const int* __re
     }
     const RoiGeom g = geoms ? geoms[roi] : s_g;
     const int H = L.H[g.level], W = L.W[g.level];
-#ifdef RSDET_TUNING   // A/B builds: phase-cost measurements (lists only / nothing); the shipped kernel has no such switch
-    if (L.dbg_skip_main < 2) build_tap_lists(g, L, H, W, s_list, s_cnt, reinterpret_cast<float*>(s_stage), C >> 2, 0);
-    if (L.dbg_skip_main) { for (int b = tid; b < nbins; b += kRoiThreads) s_cnt[b] = 0; __syncthreads(); }
-#else
-    build_tap_lists(g, L, H, W, s_list, s_cnt, reinterpret_cast<float*>(s_stage), C >> 2, 0);   // the scratch is dead after its final barrier
-#endif
+    build_tap_lists(g, L, H, W, s_list, s_cnt, reinterpret_cast<float*>(s_stage), C >> 2);   // the scratch is dead after its final barrier
 
     const int lanes = QPT == 2 ? 32 : Qc;                  // threads per bin group
     const int groups = kRoiThreads / lanes;
@@ -863,10 +813,6 @@ roi_align_fwd_kernel(LevelSet L, const float* __restrict__ rois, const int* __re
                 int2 en[4];
 #pragma unroll
                 for (int k = 0; k < 4; k++) en[k] = lp[min(e + k, cnt - 1)];  // warp-uniform broadcast reads
-#ifdef RSDET_TUNING
-#pragma unroll
-                for (int k = 0; k < 4; k++) en[k].x &= L.dbg_mask;
-#endif
                 float4 v[QPT][4];
 #pragma unroll
                 for (int k = 0; k < 4; k++)
@@ -915,127 +861,41 @@ roi_align_fwd_kernel(LevelSet L, const float* __restrict__ rois, const int* __re
     }
 }
 
-// ---------------------------------------------------------------------------------- forward (7x7 bins, 2x2 samples, 256-channel chunks)
-// The Oriented R-CNN geometry with everything the generic kernel reads at run time fixed at compile time, and the
-// gather loop restructured around what the per-instruction stall samples of the generic kernel showed
-// (profiles/README.md "round 2, second pass"): of its 18 000 warp instructions per RoI only 3 800 were FFMA and 940
-// LDG -- the rest were index clamps, 64-bit address pairs, run-time pitches and the rotate/stage arithmetic -- and a
-// third of the gather's stall samples sat on the LEA that waits for the tap-list LDS, i.e. every batch paid TWO dependent
-// L1 round trips (list entries, then pixels) behind the other CTAs' queued loads.  Here
-//   * the four list entries of the NEXT batch (or of the warp's next bin) are read while the current batch's pixel
-//     loads are in flight, so a batch is one round trip;
+// ---------------------------------------------------------------------------------- forward (7x7, persistent) -- the default
+// The Oriented R-CNN geometry (7x7 bins, 2x2 samples, 256-channel chunks) with everything roi_align_fwd_kernel reads at
+// run time fixed at compile time, and the gather loop restructured around what the per-instruction stall samples of
+// that kernel showed (profiles/README.md "round 2, second pass"): of its 18 000 warp instructions per RoI only 3 800 were
+// FFMA and 940 LDG -- the rest were index clamps, 64-bit address pairs, run-time pitches and the rotate/stage arithmetic
+// -- and a third of the gather's stall samples sat on the LEA that waits for the tap-list LDS, i.e. every batch paid TWO
+// dependent L1 round trips (list entries, then pixels) behind the other CTAs' queued loads.  Here
+//   * the list entries of the NEXT batch (or of the warp's next bin) are read while the current batch's pixel loads are
+//     in flight, so a batch is one round trip;
 //   * a warp walks its bins as one flat sequence of batches; the [c][bin] staging stores of a finished bin are issued
 //     after the first loads of the next bin, not before them;
-//   * a CTA starts from the geometry record in processing order (one global round trip instead of order -> geoms).
-// Arithmetic and tap order are those of roi_align_fwd_kernel<2>; results are bit-identical.
-constexpr size_t kStage77Offset = (8 * 49 * 17 + 15 + ((49 * 4 + 15) & ~15) + 127) & ~(size_t)127;   // lists + counts, rounded up
-template <int WARPS, int FLAVOUR = 0, int MINB = 4, typename T = float, typename O = float>
-__global__ void __launch_bounds__(32 * WARPS, MINB)
-roi_align_fwd77_kernel(LevelSet L, const RoiGeom* __restrict__ gsorted, int K, O* __restrict__ out) {
-    constexpr int NB = 49, CAP = 16, PITCH = CAP + 1, THREADS = 32 * WARPS;
-    extern __shared__ __align__(16) unsigned char smem_raw[];
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    int2* s_list = reinterpret_cast<int2*>(smem_raw);
-    int* s_cnt = reinterpret_cast<int*>(smem_raw + list_bytes(NB, CAP));
-    // staging block on a 128-byte boundary: the bulk store reads it in 128-byte lines
-    O* s_stage = reinterpret_cast<O*>(smem_raw + kStage77Offset);
-    RoiGeom g = gsorted[blockIdx.x];
-    const int roi = g.gh;                                   // processing-order record: gh carries the RoI index
-    g.gh = 2; g.gw = 2;
-    const int C = L.C, chunk0 = blockIdx.y * 256;
-    const int H = L.H[g.level], W = L.W[g.level];
-    build_tap_lists<THREADS, true>(g, L, H, W, s_list, s_cnt, reinterpret_cast<float*>(s_stage), C >> 2, 0);   // the scratch (staging block) is dead after its final barrier
-
-    const typename Quad<T>::V* __restrict__ feat =
-        reinterpret_cast<const typename Quad<T>::V*>(feat_base<T>(L, g.level) + (size_t)g.batch * H * W * C + chunk0) + lane;
-    const int oct = (lane >> 3) & 3;
-    // staging slot of component j of a quad: channel 4*lane + ((j + oct) & 3) (conflict-free, see rot4); computed per bin
-    // instead of held in four registers
-    O* const sbase = s_stage + lane * 4 * NB;
-    auto stage = [&](float4 a0, float4 a1, int b) {
-        a0.x *= 0.25f; a0.y *= 0.25f; a0.z *= 0.25f; a0.w *= 0.25f;   // output_val /= count (:143), count = 4: exact
-        a1.x *= 0.25f; a1.y *= 0.25f; a1.z *= 0.25f; a1.w *= 0.25f;
-        const float4 r0 = rot4(a0, oct), r1 = rot4(a1, oct);
-        O* const sb = sbase + b;
-        O* const q0 = sb + ((0 + oct) & 3) * NB;
-        O* const q1 = sb + ((1 + oct) & 3) * NB;
-        O* const q2 = sb + ((2 + oct) & 3) * NB;
-        O* const q3 = sb + ((3 + oct) & 3) * NB;
-        q0[0] = from_f32<O>(r0.x); q1[0] = from_f32<O>(r0.y); q2[0] = from_f32<O>(r0.z); q3[0] = from_f32<O>(r0.w);
-        q0[128 * NB] = from_f32<O>(r1.x); q1[128 * NB] = from_f32<O>(r1.y); q2[128 * NB] = from_f32<O>(r1.z); q3[128 * NB] = from_f32<O>(r1.w);
-    };
-    // one batch: up to four taps = eight 16-byte loads in flight per thread; the list entries of the following batch
-    // (same bin, or the first four of this warp's next bin) are read while the loads fly
-#define RSDET_ACC(P, WT, RA, RB)                                                                                        \
-        if (P) {                                                                                                        \
-            const auto& VA = quad_f32<T>(RA);                                                                           \
-            const auto& VB = quad_f32<T>(RB);                                                                           \
-            acc0.x = fmaf(WT, VA.x, acc0.x); acc0.y = fmaf(WT, VA.y, acc0.y); acc0.z = fmaf(WT, VA.z, acc0.z); acc0.w = fmaf(WT, VA.w, acc0.w); \
-            acc1.x = fmaf(WT, VB.x, acc1.x); acc1.y = fmaf(WT, VB.y, acc1.y); acc1.z = fmaf(WT, VB.z, acc1.z); acc1.w = fmaf(WT, VB.w, acc1.w); \
-        }
-    const int2* lp = s_list + warp * PITCH;
-    int2 en0 = lp[0], en1 = lp[1], en2 = lp[2], en3 = lp[3];
-    int cnt = s_cnt[warp];
-#pragma unroll 1
-    for (int b = warp; b < NB; b += WARPS) {
-        float4 acc0 = make_float4(0.f, 0.f, 0.f, 0.f), acc1 = acc0;
-        const int nbin = min(b + WARPS, NB - 1);
-        int ncnt = cnt;
-        int e = 0;
-#pragma unroll 1
-        do {
-            const bool p0 = e < cnt, p1 = e + 1 < cnt, p2 = e + 2 < cnt, p3 = e + 3 < cnt;
-            typename Quad<T>::V v00, v01, v10, v11, v20, v21, v30, v31;   // raw: 2-byte values convert right before their FMAs
-            if (p0) { const T* q = quad_ptr<T>(feat, (unsigned)en0.x); v00 = ldg4_raw<T, FLAVOUR>(q); v01 = ldg4_raw<T, FLAVOUR>(q + 128); }
-            if (p1) { const T* q = quad_ptr<T>(feat, (unsigned)en1.x); v10 = ldg4_raw<T, FLAVOUR>(q); v11 = ldg4_raw<T, FLAVOUR>(q + 128); }
-            if (p2) { const T* q = quad_ptr<T>(feat, (unsigned)en2.x); v20 = ldg4_raw<T, FLAVOUR>(q); v21 = ldg4_raw<T, FLAVOUR>(q + 128); }
-            if (p3) { const T* q = quad_ptr<T>(feat, (unsigned)en3.x); v30 = ldg4_raw<T, FLAVOUR>(q); v31 = ldg4_raw<T, FLAVOUR>(q + 128); }
-            const float w0 = __int_as_float(en0.y), w1 = __int_as_float(en1.y), w2 = __int_as_float(en2.y), w3 = __int_as_float(en3.y);
-            e += 4;
-            const bool more = e < cnt;
-            const int2* np = more ? lp + e : s_list + nbin * PITCH;
-            if (!more) ncnt = s_cnt[nbin];
-            en0 = np[0]; en1 = np[1]; en2 = np[2]; en3 = np[3];
-            RSDET_ACC(p0, w0, v00, v01) RSDET_ACC(p1, w1, v10, v11) RSDET_ACC(p2, w2, v20, v21) RSDET_ACC(p3, w3, v30, v31)
-        } while (e < cnt);
-        stage(acc0, acc1, b);
-        lp = s_list + nbin * PITCH;
-        cnt = ncnt;
-    }
-#undef RSDET_ACC
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-    __syncthreads();
-    O* __restrict__ dst = out + ((size_t)roi * C + chunk0) * NB;
-    if ((((size_t)out) & 15) == 0 && ((C * NB) & 3) == 0) {
-        if (tid == 0) bulk_store_evict_first(dst, s_stage, 256u * NB * (unsigned)sizeof(O));
-    } else {
-        for (int i = tid; i < 256 * NB; i += THREADS) stcs1(dst + i, s_stage[i]);
-    }
-}
-
-// ---------------------------------------------------------------------------------- forward (7x7, persistent) -- the default
-// roi_align_fwd77_kernel as a PERSISTENT CTA, three per SM (profiles/README.md "third pass"):
-//   * 148 x 3 CTAs of 8 warps take (RoI, 256-channel chunk) items from a counter in the workspace (dynamic: RoIs differ
-//     in tap count); the counter is zeroed by roi_geometry_kernel, which always runs in front of this kernel on the
-//     same stream, so concurrent calls on different streams and CUDA-graph replays need nothing else;
+//   * the CTA is PERSISTENT, three per SM (profiles/README.md "third pass"): 148 x 3 CTAs of 8 warps take (RoI,
+//     256-channel chunk) items from a counter in the workspace (dynamic: RoIs differ in tap count); the counter is zeroed
+//     by the prologue (roi_prep_kernel or transpose_prep_kernel), which always runs in front of this kernel on the same
+//     stream, so concurrent calls on different streams and CUDA-graph replays need nothing else;
 //   * three CTAs instead of four leave the compiler 78 registers (no spill at 8 warps) and -- what the experiments that
 //     forced the CTA count by padding shared memory could not show -- let the driver pick the 196 KB carve-out: L1 grows
 //     from 28 to 60 KB, its hit rate from 14 % to 27 %, the bytes pulled through the SM's L2 port fall by 16 %;
 //   * the merged lists are built IN PLACE (A1 writes the sixteen raw taps of a bin into the bin's own list slots, A2
-//     reads them into registers and writes the merged entries back), so the list build no longer borrows the staging
+//     reads them into registers and writes the merged entries back), so the list build does not borrow the staging
 //     block and runs while the previous item's bulk store is still reading it; the next item's geometry record is
 //     fetched with cp.async during the gather.
 // Lists have a pitch of 18 entries (16-byte aligned: a batch's four entries are two LDS.128; the count sits in entry 16).
-// Arithmetic and tap order are those of roi_align_fwd77_kernel: bit-identical results.
+// Arithmetic and tap order are those of roi_align_fwd_kernel<2>: bit-identical results.  The measured variants (warps,
+// CTAs per SM, taps per batch, load flavours, one CTA per RoI) are in profiles/README.md.
+constexpr int kFwd77pWarps = 8, kFwd77pCtasPerSm = 3;
+constexpr int kFwd77pTaps = 4;   // list entries per batch: 8 vector loads in flight per thread
 constexpr size_t kStage77pOffset = (8 * 49 * 18 + 16 + 48 + 127) & ~(size_t)127;   // lists | next item | next record | staging
-// TAPS: list entries per batch (4, 6 or 8 = 8 / 12 / 16 vector loads in flight per thread); T: feature elements (a half
-// map halves the bytes of every tap load: two 8-byte loads per lane and tap); O: output elements (a half output halves
-// the staging block and its bulk store)
-template <int WARPS, int MINB, int TAPS = 4, typename T = float, typename O = float>
-__global__ void __launch_bounds__(32 * WARPS, MINB)
+// T: feature elements (a half map halves the bytes of every tap load: two 8-byte loads per lane and tap); O: output
+// elements (a half output halves the staging block and its bulk store)
+template <typename T, typename O>
+__global__ void __launch_bounds__(32 * kFwd77pWarps, kFwd77pCtasPerSm)
 roi_align_fwd77p_kernel(LevelSet L, const int* __restrict__ order, const RoiGeom* __restrict__ geoms, int K, int chunks,
                         O* __restrict__ out, unsigned* __restrict__ counter) {
-    constexpr int NB = 49, PITCH = 18, THREADS = 32 * WARPS;
+    constexpr int NB = 49, PITCH = 18, WARPS = kFwd77pWarps, TAPS = kFwd77pTaps, THREADS = 32 * WARPS;
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     int2* s_list = reinterpret_cast<int2*>(smem_raw);
@@ -1091,14 +951,6 @@ roi_align_fwd77p_kernel(LevelSet L, const int* __restrict__ order, const RoiGeom
                 }
                 if (w[j] != 0.f) s_list[b * PITCH + pos++] = make_int2(o[j], __float_as_int(acc));
             }
-#ifdef RSDET_TUNING   // what-if: 1 of every `dbg_drop` entries removed (wrong results, timing of a deduplicated list)
-            if (L.dbg_drop > 1) {
-                int q = 0;
-                for (int e = 0; e < pos; e++)
-                    if ((e + b) % L.dbg_drop != 0) s_list[b * PITCH + q++] = s_list[b * PITCH + e];
-                pos = q;
-            }
-#endif
             s_list[b * PITCH + 16] = make_int2(pos, 0);
         }
         if (tid == THREADS - 1) {      // a thread without A1 / A2 work: the previous block must have left the staging area; next item
@@ -1206,18 +1058,6 @@ static void set_dyn_smem(const void* func, size_t bytes) {
     cudaFuncSetAttribute(func, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
 }
 
-// Forward path: 1 = bin-major register kernel + TMA bulk store (the default and the only path of the shipped library:
-// fastest measured, profiles/README.md "round 2"), and -- in RSDET_TUNING builds only, selected through RSDET_ROI_PATH
-// for A/B measurements -- 0 = row windows, persistent warp-specialised, 3 = row windows, one CTA per RoI, 2 = TMA gather4.
-static int roi_path_choice() {
-#ifdef RSDET_TUNING
-    if (const char* e = getenv("RSDET_ROI_PATH")) return atoi(e);
-#endif
-    return 1;
-}
-
-static bool fast_path_ok(const rsdet_roi_align_cfg* c);
-static size_t fwd_smem_bytes(const rsdet_roi_align_cfg* c);
 // measurement aid (rsdet_roi_align_profile_events): events recorded around the gather kernel of the next forward call
 static thread_local cudaEvent_t t_prof_start = nullptr, t_prof_stop = nullptr;
 struct GatherTimer {       // records on construction / destruction when armed; disarms itself
@@ -1233,9 +1073,6 @@ struct GatherTimer {       // records on construction / destruction when armed; 
 static bool fwd77_ok(const rsdet_roi_align_cfg* c) {
     return c->pooled_h == 7 && c->pooled_w == 7 && c->sampling_ratio == 2 && c->channels % 256 == 0;
 }
-#ifdef RSDET_TUNING
-#include "roi_align_tuning.cuh"
-#endif
 
 // ---------------------------------------------------------------------------------- backward (fast)
 // Same CTA shape and tap lists.  The RoI's (C,7,7) gradient block is copied into shared memory as it
@@ -1266,7 +1103,7 @@ roi_align_bwd_kernel(LevelSet L, const float* __restrict__ rois, const int* __re
     }
     const RoiGeom g = geoms ? geoms[roi] : s_g;
     const int H = L.H[g.level], W = L.W[g.level];
-    build_tap_lists(g, L, H, W, s_list, s_cnt, s_stage, C >> 2, 0);
+    build_tap_lists(g, L, H, W, s_list, s_cnt, s_stage, C >> 2);
 
     // stage this chunk's gradient block [c_local][bin] (= memory order)
     const G* __restrict__ src = grad_out + ((size_t)roi * C + chunk0) * nbins;
@@ -1412,14 +1249,6 @@ static LevelSet make_levels(const rsdet_roi_align_cfg* c) {
     L.num_levels = c->num_levels; L.batch = c->batch; L.C = c->channels;
     L.PH = c->pooled_h; L.PW = c->pooled_w; L.sampling_ratio = c->sampling_ratio; L.version = c->version;
     L.extend_w = c->extend_w; L.extend_h = c->extend_h; L.finest_scale = c->finest_scale;
-    L.dbg_skip_main = 0;
-    L.dbg_mask = 0xffffffffu;
-    L.dbg_drop = 0;
-#ifdef RSDET_TUNING
-    if (const char* e = getenv("RSDET_ROI_DBG_SKIP_MAIN")) L.dbg_skip_main = atoi(e);
-    if (const char* e = getenv("RSDET_ROI_DBG_MASK")) L.dbg_mask = (unsigned)strtoul(e, nullptr, 0);
-    if (const char* e = getenv("RSDET_ROI_DBG_DROP")) L.dbg_drop = atoi(e);
-#endif
     for (int l = 0; l < RSDET_MAX_LEVELS; l++) {
         L.feat[l] = nullptr; L.grad[l] = nullptr;
         L.H[l] = l < c->num_levels ? c->height[l] : 1;
@@ -1444,15 +1273,9 @@ static bool dtype_ok(int dt) { return dt == RSDET_DTYPE_F32 || dt == RSDET_DTYPE
 
 // elem: bytes of one feature-map element
 static size_t roi_workspace_bytes(const rsdet_roi_align_cfg* cfg, int num_rois, int backward, size_t elem) {
-    // order, geometry, geometry in processing order (+ one record: the work counter of the persistent forward kernel)
+    // order, geometry (+ forward: the work counter of the persistent kernel)
     size_t b = ws_bytes<int>(num_rois > 0 ? num_rois : 1) + ws_bytes<RoiGeom>(num_rois > 0 ? num_rois : 1) +
-               ws_bytes<RoiGeom>((num_rois > 0 ? num_rois : 1) + 1);
-#ifdef RSDET_TUNING
-    if (fast_path_ok(cfg) && split_path_ok(cfg))   // tap-list records of the A/B kernels
-        b += ws_bytes<unsigned char>((size_t)(num_rois > 0 ? num_rois : 1) *
-                                     (rec_stride((size_t)cfg->pooled_h * cfg->pooled_w, 4 * (size_t)cfg->sampling_ratio * cfg->sampling_ratio) +
-                                      stream_rec_stride((size_t)cfg->pooled_h * cfg->pooled_w, 4 * (size_t)cfg->sampling_ratio * cfg->sampling_ratio)));
-#endif
+               (backward ? 0 : ws_bytes<unsigned>(1));
     if (backward && elem != sizeof(float)) {    // half gradient maps: fp32 accumulators on every path
         for (int l = 0; l < cfg->num_levels; l++)
             b += ws_bytes<float>((size_t)cfg->batch * cfg->channels * cfg->height[l] * cfg->width[l]);
@@ -1478,9 +1301,6 @@ extern "C" size_t rsdet_roi_align_rotated_workspace_bytes(const rsdet_roi_align_
 template <typename T, typename O>
 static int forward_impl(const rsdet_roi_align_cfg* cfg, const T* const* feats_host, const float* rois, int num_rois, O* out,
                         int32_t* levels_out, void* workspace, size_t workspace_bytes, cudaStream_t st) {
-#ifdef RSDET_TUNING
-    constexpr bool kF32Call = kIsF32<T> && kIsF32<O>;   // the A/B kernels of RSDET_TUNING builds exist for fp32 only
-#endif
     int rc = RSDET_OK;
     LevelSet L = make_levels(cfg);
     if (!fast_path_ok(cfg) || !nhwc_bases_aligned(cfg, feats_host, 4 * sizeof(T))) {
@@ -1500,7 +1320,7 @@ static int forward_impl(const rsdet_roi_align_cfg* cfg, const T* const* feats_ho
     Workspace ws(workspace, workspace_bytes);
     int* order_ws = ws.take<int>(num_rois);
     RoiGeom* geoms = ws.take<RoiGeom>(num_rois);
-    RoiGeom* gsorted = ws.take<RoiGeom>(num_rois + 1);
+    unsigned* counter = ws.take<unsigned>(1);
     if (cfg->channels_last) {
         for (int l = 0; l < cfg->num_levels; l++) L.feat[l] = reinterpret_cast<const float*>(feats_host[l]);
     } else {
@@ -1510,20 +1330,12 @@ static int forward_impl(const rsdet_roi_align_cfg* cfg, const T* const* feats_ho
     }
     // locality order (needs the int[K] slot at the start of the workspace; skipped for tiny calls)
     int* order = num_rois >= 256 && order_ws ? order_ws : nullptr;
-#ifdef RSDET_TUNING
-    if (getenv("RSDET_ROI_NOORDER")) order = nullptr;
-#endif
     const bool ride = !cfg->channels_last && order && num_rois <= kPrepMaxRois;
-    // lean prologue (the persistent 7x7 kernel follows): records by RoI index only, one launch, and for NCHW callers
-    // no launch at all -- order block and geometry blocks ride with the transpose
-    bool lean = fwd77_ok(cfg) && roi_path_choice() == 1 && (((size_t)out) & 15) == 0;
-#ifdef RSDET_TUNING
-    if (getenv("RSDET_ROI_NOPERSIST") || getenv("RSDET_ROI_V8") || getenv("RSDET_ROI_MINB3") || getenv("RSDET_ROI_Q") ||
-        getenv("RSDET_ROI_LD") || getenv("RSDET_ROI_WARPS") || getenv("RSDET_ROI_OLDPREP"))
-        lean = false;
-#endif
-    unsigned* const counter = reinterpret_cast<unsigned*>(gsorted + num_rois);
-    if (!lean) launch_prep(L, rois, num_rois, geoms, order, levels_out, st, ride, gsorted);
+    // the persistent 7x7 kernel (it needs a 16-byte aligned output for its bulk stores) and its lean prologue: records by
+    // RoI index only, one launch, and for NCHW callers no launch at all -- order block and geometry blocks ride with the
+    // transpose.  Everything else runs roi_align_fwd_kernel behind the order and geometry kernels.
+    const bool lean = fwd77_ok(cfg) && (((size_t)out) & 15) == 0;
+    if (!lean) launch_prep(L, rois, num_rois, geoms, order, levels_out, st, ride);
     else if (!ride) {
         roi_prep_kernel<<<(order ? 1 : 0) + ceil_div(num_rois, 1024), 1024, 0, st>>>(L, rois, num_rois, order, geoms, levels_out, counter);
         count_launch();
@@ -1537,133 +1349,29 @@ static int forward_impl(const rsdet_roi_align_cfg* cfg, const T* const* feats_ho
         rc = launch_transpose(true, feats_host, dst, cfg->height, cfg->width, cfg->num_levels, cfg->batch, cfg->channels, st,
                               ride ? &prep : nullptr);
         if (rc != RSDET_OK) return rc;
-        if (ride && !lean) launch_geometry(L, rois, num_rois, order, geoms, gsorted, levels_out, st);
+        if (ride && !lean) launch_geometry(L, rois, num_rois, order, geoms, levels_out, st);
     }
-    size_t smem = fwd_smem_bytes(cfg);
-#ifdef RSDET_TUNING
-    if (const char* e = getenv("RSDET_ROI_PAD_SMEM")) smem += (size_t)atoi(e) * 1024;   // fewer resident CTAs per SM
-#endif
-    set_dyn_smem((const void*)roi_align_fwd_kernel<1, T, O>, smem);
-    set_dyn_smem((const void*)roi_align_fwd_kernel<2, T, O>, smem);
-#ifdef RSDET_TUNING
-    if constexpr (kF32Call) {
-        int trc = RSDET_OK;
-        if (tuning_forward(cfg, L, ws, rois, order, geoms, num_rois, out, levels_out, st, &trc)) return trc;
-    }
-#endif
     GatherTimer gather_timer(st);
-    if (fwd77_ok(cfg) && roi_path_choice() == 1) {   // the Oriented R-CNN geometry: specialised kernel
-        smem = smem - fwd_smem_bytes(cfg) + kStage77Offset + sizeof(float) * 49 * 256;
-        int warps = 7;   // one warp per bin row: 7 bins each (eight warps leave one with 7 and seven with 6 bins), 72 registers
-#ifdef RSDET_TUNING
-        if (const char* e = getenv("RSDET_ROI_WARPS")) warps = atoi(e);
-#endif
-#ifdef RSDET_TUNING
-        if constexpr (kF32Call) {
-        const int flavour = getenv("RSDET_ROI_LD") ? atoi(getenv("RSDET_ROI_LD")) : 0;
-        dim3 g77(num_rois, cfg->channels / 256);
-        if (flavour == 1) { set_dyn_smem((const void*)roi_align_fwd77_kernel<8, 1>, smem); roi_align_fwd77_kernel<8, 1><<<g77, 256, smem, st>>>(L, gsorted, num_rois, out); count_launch(); return cuda_status(); }
-        if (flavour == 2) { set_dyn_smem((const void*)roi_align_fwd77_kernel<8, 2>, smem); roi_align_fwd77_kernel<8, 2><<<g77, 256, smem, st>>>(L, gsorted, num_rois, out); count_launch(); return cuda_status(); }
-        if (flavour == 3) { set_dyn_smem((const void*)roi_align_fwd77_kernel<8, 3>, smem); roi_align_fwd77_kernel<8, 3><<<g77, 256, smem, st>>>(L, gsorted, num_rois, out); count_launch(); return cuda_status(); }
-        if (const char* e = getenv("RSDET_ROI_MINB3")) {     // A/B: three CTAs per SM by launch bounds (more registers, smaller carve-out)
-            const int w = atoi(e);
-            const int carve = getenv("RSDET_ROI_CARVE") ? atoi(getenv("RSDET_ROI_CARVE")) : -1;
-#define RSDET_L3(W_) { set_dyn_smem((const void*)roi_align_fwd77_kernel<W_, 0, 3>, smem); \
-                       if (carve >= 0) cudaFuncSetAttribute(roi_align_fwd77_kernel<W_, 0, 3>, cudaFuncAttributePreferredSharedMemoryCarveout, carve); \
-                       roi_align_fwd77_kernel<W_, 0, 3><<<g77, 32 * W_, smem, st>>>(L, gsorted, num_rois, out); count_launch(); return cuda_status(); }
-            if (w == 7) RSDET_L3(7)
-            if (w == 8) RSDET_L3(8)
-            if (w == 9) RSDET_L3(9)
-            if (w == 10) RSDET_L3(10)
-#undef RSDET_L3
-        }
-        if (const char* e = getenv("RSDET_ROI_V8")) {       // A/B: 1 = LDS.128 list reads only, 2 = + 256-bit loads
-            const size_t sm8 = kStage77v8Offset + sizeof(float) * 49 * 256;
-            if (atoi(e) == 1) { set_dyn_smem((const void*)roi_align_fwd77v8_kernel<7, false>, sm8); roi_align_fwd77v8_kernel<7, false><<<g77, 224, sm8, st>>>(L, gsorted, num_rois, out); count_launch(); return cuda_status(); }
-            if (atoi(e) == 4 && cfg->channels == 256 && (((size_t)out) & 15) == 0) {
-                unsigned* ctr = nullptr;
-                cudaGetSymbolAddress((void**)&ctr, g_roi77p_counter);
-                cudaMemsetAsync(ctr, 0, sizeof(unsigned), st);
-                const int ctas = getenv("RSDET_ROI_PCTAS") ? atoi(getenv("RSDET_ROI_PCTAS")) : kNumSMs * 3;
-                const int gw = getenv("RSDET_ROI_PWARPS") ? atoi(getenv("RSDET_ROI_PWARPS")) : 8;
-                const int grid = num_rois < ctas ? num_rois : ctas;
-                const size_t smw = ((2 * 8 * 49 * 18 + 32 + 127) & ~127) + sizeof(float) * 49 * 256;
-                if (gw == 7) { set_dyn_smem((const void*)roi_align_fwd77ws_kernel<7, 3>, smw); roi_align_fwd77ws_kernel<7, 3><<<grid, 256, smw, st>>>(L, gsorted, num_rois, out); }
-                else { set_dyn_smem((const void*)roi_align_fwd77ws_kernel<8, 3>, smw); roi_align_fwd77ws_kernel<8, 3><<<grid, 288, smw, st>>>(L, gsorted, num_rois, out); }
-                count_launch();
-                return cuda_status();
-            }
-            if (atoi(e) == 2) { set_dyn_smem((const void*)roi_align_fwd77v8_kernel<7, true>, sm8); roi_align_fwd77v8_kernel<7, true><<<g77, 224, sm8, st>>>(L, gsorted, num_rois, out); count_launch(); return cuda_status(); }
-        }
-        if (getenv("RSDET_ROI_Q")) {      // A/B (old prologue: records in processing order): pipelined list build (1: dynamic bins, 2: static columns)
-            const int chunks = cfg->channels / 256;
-            const long long items = (long long)num_rois * chunks;
-            const int ctas = kNumSMs * 3;
-            const size_t smq = kStage77qOffset + sizeof(float) * 49 * 256;
-            unsigned* ctr = reinterpret_cast<unsigned*>(gsorted + num_rois);
-            const int grid = (int)(items < ctas ? items : ctas);
-            if (atoi(getenv("RSDET_ROI_Q")) == 2) {
-                set_dyn_smem((const void*)roi_align_fwd77q_kernel<8, 3, 1>, smq);
-                roi_align_fwd77q_kernel<8, 3, 1><<<grid, 256, smq, st>>>(L, gsorted, num_rois, chunks, out, ctr);
-            } else {
-                set_dyn_smem((const void*)roi_align_fwd77q_kernel<8, 3, 0>, smq);
-                roi_align_fwd77q_kernel<8, 3, 0><<<grid, 256, smq, st>>>(L, gsorted, num_rois, chunks, out, ctr);
-            }
-            count_launch();
-            return cuda_status();
-        }
-        }
-#endif
-        if (lean) {                                     // persistent kernel (needs a 16-byte aligned output block for its bulk store)
-            const int chunks = cfg->channels / 256;
-            const long long items = (long long)num_rois * chunks;
-            int ctas = kNumSMs * 3;
-#ifdef RSDET_TUNING
-            if (const char* e = getenv("RSDET_ROI_PCTAS")) ctas = atoi(e);
-#endif
-#ifdef RSDET_TUNING
-            if constexpr (kF32Call) if (const char* e = getenv("RSDET_ROI_PVAR")) {     // A/B: warps x CTAs/SM x taps per batch of the persistent kernel
-                const size_t smv = kStage77pOffset + sizeof(float) * 49 * 256;
-                unsigned* ctr = reinterpret_cast<unsigned*>(gsorted + num_rois);
-                const int v = atoi(e);
-#define RSDET_PV(W_, M_, T_) { const int grid = (int)(items < kNumSMs * M_ ? items : kNumSMs * M_); \
-                               set_dyn_smem((const void*)roi_align_fwd77p_kernel<W_, M_, T_>, smv); \
-                               roi_align_fwd77p_kernel<W_, M_, T_><<<grid, 32 * W_, smv, st>>>(L, order, geoms, num_rois, chunks, out, ctr); \
-                               count_launch(); return cuda_status(); }
-                if (v == 1062) RSDET_PV(10, 2, 6)
-                if (v == 1262) RSDET_PV(12, 2, 6)
-                if (v == 882) RSDET_PV(8, 2, 8)
-                if (v == 1082) RSDET_PV(10, 2, 8)
-                if (v == 763) RSDET_PV(7, 3, 6)
-                if (v == 863) RSDET_PV(8, 3, 6)
-                if (v == 1442) RSDET_PV(14, 2, 4)
-                if (v == 1242) RSDET_PV(12, 2, 4)
-#undef RSDET_PV
-            }
-#endif
-            const size_t smp = kStage77pOffset + sizeof(float) * 49 * 256;
-            set_dyn_smem((const void*)roi_align_fwd77p_kernel<8, 3, 4, T, O>, smp);
-            roi_align_fwd77p_kernel<8, 3, 4, T, O><<<(int)(items < ctas ? items : ctas), 256, smp, st>>>(
-                L, order, geoms, num_rois, chunks, out, counter);
-            count_launch();
-            return cuda_status();
-        }
-        if (warps == 7) {
-            set_dyn_smem((const void*)roi_align_fwd77_kernel<7, 0, 4, T, O>, smem);
-            roi_align_fwd77_kernel<7, 0, 4, T, O><<<dim3(num_rois, cfg->channels / 256), 224, smem, st>>>(L, gsorted, num_rois, out);
-        } else {
-            set_dyn_smem((const void*)roi_align_fwd77_kernel<8, 0, 4, T, O>, smem);
-            roi_align_fwd77_kernel<8, 0, 4, T, O><<<dim3(num_rois, cfg->channels / 256), 256, smem, st>>>(L, gsorted, num_rois, out);
-        }
+    if (lean) {
+        const int chunks = cfg->channels / 256;
+        const long long items = (long long)num_rois * chunks, ctas = kNumSMs * kFwd77pCtasPerSm;
+        const size_t smp = kStage77pOffset + sizeof(float) * 49 * 256;
+        set_dyn_smem((const void*)roi_align_fwd77p_kernel<T, O>, smp);
+        roi_align_fwd77p_kernel<T, O><<<(int)(items < ctas ? items : ctas), 32 * kFwd77pWarps, smp, st>>>(
+            L, order, geoms, num_rois, chunks, out, counter);
         count_launch();
         return cuda_status();
     }
+    const size_t smem = fwd_smem_bytes(cfg);
     const int Q = quads_per_chunk(cfg->channels);
     dim3 grid(num_rois, ceil_div(cfg->channels / 4, Q));
-    if (cfg->channels % 256 == 0)
+    if (cfg->channels % 256 == 0) {
+        set_dyn_smem((const void*)roi_align_fwd_kernel<2, T, O>, smem);
         roi_align_fwd_kernel<2, T, O><<<grid, kRoiThreads, smem, st>>>(L, rois, order, geoms, num_rois, out, nullptr);
-    else
+    } else {
+        set_dyn_smem((const void*)roi_align_fwd_kernel<1, T, O>, smem);
         roi_align_fwd_kernel<1, T, O><<<grid, kRoiThreads, smem, st>>>(L, rois, order, geoms, num_rois, out, nullptr);
+    }
     count_launch();
     return cuda_status();
 }
@@ -2081,13 +1789,6 @@ extern "C" int rsdet_roi_align_rotated_backward_deterministic(const rsdet_roi_al
     return RSDET_BWD_DET(float, float);
 #undef RSDET_BWD_DET
 }
-
-#ifdef RSDET_PROF
-// profiling builds only: device buffer of 8 counters filled by roi_align_fwd_px_kernel (per-phase cycle sums)
-extern "C" int rsdet_tuning_set_prof(unsigned long long* dev_counters) {
-    return (int)cudaMemcpyToSymbol(g_px_prof, &dev_counters, sizeof(dev_counters));
-}
-#endif
 
 extern "C" int rsdet_roi_align_profile_events(void* start_event, void* stop_event) {
     t_prof_start = (cudaEvent_t)start_event;

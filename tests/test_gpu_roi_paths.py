@@ -7,15 +7,16 @@ the alignment of the caller's buffers, the geometry and whether the fast path ap
   * 16-byte aligned output, NCHW, 256 <= K <= 16384: the order block and the geometry blocks ride with the pyramid
     transpose (`transpose_prep_kernel`); above K = 4160 the order block recomputes buckets in its scatter pass;
   * aligned output, NCHW, K < 256 or K > 16384, and every aligned channels-last call: `roi_prep_kernel`;
-  * output not 16-byte aligned: the old prologue (`roi_order_kernel` or the ride-along order block, then
-    `roi_geometry_kernel`) and `roi_align_fwd77_kernel<7>`; otherwise the persistent `roi_align_fwd77p_kernel`.
+  * output not 16-byte aligned: the prologue of the other geometries (`roi_order_kernel` or the ride-along order
+    block, then `roi_geometry_kernel`) and `roi_align_fwd_kernel<2>`; otherwise the persistent
+    `roi_align_fwd77p_kernel`.
 
 Other geometries run `roi_align_fwd_kernel<2>` (C % 256 == 0) or `<1>`, and configurations outside the fast path run
-`roi_align_generic_kernel`.  The order (K >= 256) changes only which CTA takes a RoI, and the 7x7 kernels are
-bit-identical, so every forward path is checked bit for bit against one reference: NCHW, aligned, K split into calls
-of at most 4000 RoIs.  A seeded subset of rows is checked against the oracle at 1e-5 of the tensor scale, every
-output buffer is prefilled with NaN (every row must be written, nothing outside it), and the levels written through
-`levels_out` must equal the oracle's.  Backward: both layouts, K below and above the order threshold, 256 and 260
+`roi_align_generic_kernel`.  The order (K >= 256) changes only which CTA takes a RoI, and the persistent kernel is
+bit-identical to `roi_align_fwd_kernel<2>`, so every forward path is checked bit for bit against one reference: NCHW,
+aligned, K split into calls of at most 4000 RoIs.  A seeded subset of rows is checked against the oracle at 1e-5 of
+the tensor scale, every output buffer is prefilled with NaN (every row must be written, nothing outside it), and the
+levels written through `levels_out` must equal the oracle's.  Backward: both layouts, K below and above the order threshold, 256 and 260
 channels (`roi_align_bwd_kernel<2>` / `<1>` with a ragged second chunk), against the oracle at 1e-4, with the
 caller's gradient buffers prefilled with NaN so that their zero fill is checked too.
 

@@ -1,10 +1,8 @@
 #!/usr/bin/env python
-"""Time the RoIAlignRotated forward paths alone (channels-last pyramid resident, 8 distinct bench tiles back to
-back = the measurement behind bench.py's `roofline`).  With a library built with RSDET_TUNING=1 the paths are
-switched through RSDET_ROI_PATH (0 pixel-major, 1 bin-major registers, 2 TMA gather4); a shipped build always
-runs its default and the sweep degenerates to one line.
+"""Time the RoIAlignRotated forward alone: channels-last pyramid resident, distinct bench tiles back to back (8 by
+default = the measurement behind bench.py's `roofline`), CUDA events around the whole loop.
 
-    python tools/roi_sweep.py [--paths 0,1,2] [--check]
+    python tools/roi_sweep.py [--reps 10] [--tiles 8]
 """
 import argparse
 import os
@@ -19,10 +17,7 @@ import workloads as W  # noqa: E402
 from rs_detection_b200 import core  # noqa: E402
 
 ap = argparse.ArgumentParser()
-ap.add_argument("--paths", default="0,1")
-ap.add_argument("--check", action="store_true", help="compare every path's output with path 1 (bin-major)")
 ap.add_argument("--reps", type=int, default=10)
-ap.add_argument("--prof", action="store_true", help="RSDET_TUNING builds: per-phase cycle sums of the one-CTA-per-RoI kernel")
 ap.add_argument("--tiles", type=int, default=8, help="distinct tiles cycled (1: the 89 MB pyramid stays L2-resident)")
 a = ap.parse_args()
 
@@ -41,52 +36,14 @@ def run():
         core.roi_align_rotated_forward(cfg, f, r, out=out)
 
 
-prof = None
-if a.prof:
-    import ctypes
-    from rs_detection_b200 import _lib
-    L = _lib.load()
-    prof = torch.zeros(8, dtype=torch.int64, device=dev)
-    fn = ctypes.CDLL(_lib.LIB_PATH if hasattr(_lib, "LIB_PATH") else os.path.join(ROOT, "rs_detection_b200", "librsdet.so")).rsdet_tuning_set_prof
-    fn.argtypes = [ctypes.c_void_p]
-    assert fn(prof.data_ptr()) == 0
-
-ref = None
-for spec in a.paths.split(","):      # "<path>" or "<path>:<prefetch 0/1>" (row-window kernels)
-    path, _, pf = spec.partition(":")
-    path = int(path)
-    os.environ["RSDET_ROI_PATH"] = str(path)
-    os.environ["RSDET_ROI_PF"] = pf or "0"
-    for _ in range(3):
-        run()
-    torch.cuda.synchronize()
-    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    e0.record()
-    for _ in range(a.reps):
-        run()
-    e1.record()
-    torch.cuda.synchronize()
-    msg = f"path {spec}: {e0.elapsed_time(e1) / (a.tiles * a.reps) * 1000:.1f} us per 4000-RoI tile (geometry + order + gather kernels)"
-    if a.check:
-        o = core.roi_align_rotated_forward(cfg, tiles[0][0], tiles[0][1]).clone()
-        if ref is None:
-            os.environ["RSDET_ROI_PATH"] = "9"      # the generic bin-major kernel
-            ref = core.roi_align_rotated_forward(cfg, tiles[0][0], tiles[0][1]).clone()
-        msg += f"; max |diff| vs generic bin-major {float((o - ref).abs().max()):.3g} (scale {float(ref.abs().max()):.3g})"
-    print(msg, flush=True)
-    if prof is not None and path in (7, 8):
-        prof.zero_()
-        run()
-        torch.cuda.synchronize()
-        c = prof.cpu().numpy().astype(float)
-        n = max(c[6], 1.0)
-        print(f"    per warp and RoI: record wait {c[0] / n:.0f}, gather {c[1] / n:.0f}, store-drain wait {c[2] / n:.0f}, wait for the slowest warp {c[3] / n:.0f} cycles; "
-              f"{c[4] / n:.1f} batches -> {c[1] / max(c[4], 1):.0f} cycles per batch ({n:.0f} warp-RoIs)")
-    if prof is not None and path == 3:
-        prof.zero_()
-        run()
-        torch.cuda.synchronize()
-        c = prof.cpu().numpy().astype(float)
-        n = max(c[6], 1.0)
-        names = ["A1 + barriers", "row build", "wait at build barrier", "gather", "wait at final barrier", "bulk store (tid 0 waits)"]
-        print("    per row-warp cycles: " + ", ".join(f"{nm} {c[i] / n:.0f}" for i, nm in enumerate(names)) + f" (total {c[:6].sum() / n:.0f}, {n:.0f} warps)")
+for _ in range(3):
+    run()
+torch.cuda.synchronize()
+e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+e0.record()
+for _ in range(a.reps):
+    run()
+e1.record()
+torch.cuda.synchronize()
+print(f"{e0.elapsed_time(e1) / (a.tiles * a.reps) * 1000:.1f} us per {B.K_ROIS}-RoI tile (prologue + gather kernels)",
+      flush=True)
