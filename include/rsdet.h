@@ -131,11 +131,22 @@ typedef struct {
     int version;                           /* 1 = ROIAlignRotated_v1 (-0.5, clockwise), 0 = v0        */
     float extend_w, extend_h;              /* RoI extension (1.2, 1.4 in orcnn configs); 1,1 = none   */
     float finest_scale;                    /* 56; used when num_levels > 1                            */
-    int channels_last;                     /* features (and grads) are NHWC instead of NCHW           */
+    int channels_last;                     /* layout bits RSDET_ROI_NHWC_* (below); 0 = NCHW-style     */
 } rsdet_roi_align_cfg;
 
-/* feats[l]: (N,C,H_l,W_l) fp32 (NCHW, or NHWC when channels_last); rois (K,6);
- * out (K,C,ph,pw) fp32 -- always the reference's NCHW-style layout.  levels_out: optional int32 (K).
+/* cfg.channels_last is a bit set.  Any other bit returns RSDET_EINVAL and makes the workspace queries return 0 (a value
+ * above 1 used to be read as "true"; it is now checked).
+ *   RSDET_ROI_NHWC_MAPS  feature maps (forward) and gradient maps (backward) are (N,H,W,C) instead of (N,C,H,W).
+ *   RSDET_ROI_NHWC_ROIS  the forward's out and the backward's grad_out are (K,ph,pw,C) instead of (K,C,ph,pw): the strides of
+ *                        a torch.channels_last (K,C,ph,pw) tensor.
+ * The RoI-tensor layout changes where values are stored, never what they are: an NHWC out is, bit for bit, the NCHW out
+ * permuted, on every path and for every dtype; a deterministic backward gives the same bits for either grad_out layout;
+ * the atomic backward agrees to the backward tolerance. */
+#define RSDET_ROI_NHWC_MAPS 1
+#define RSDET_ROI_NHWC_ROIS 2
+
+/* feats[l]: (N,C,H_l,W_l) fp32 (NCHW, or NHWC with RSDET_ROI_NHWC_MAPS); rois (K,6);
+ * out (K,C,ph,pw) fp32 -- the reference's layout -- or (K,ph,pw,C) with RSDET_ROI_NHWC_ROIS.  levels_out: optional int32 (K).
  *
  * Alignment.  fp32 / int32 pointers need only their natural 4-byte alignment; 16-byte alignment selects faster
  * kernels, never different results beyond what is stated here.  The fast path is C % 4 == 0, sampling_ratio > 0 and
@@ -147,8 +158,12 @@ typedef struct {
  *            out         16-byte aligned: the 7x7 / sampling_ratio 2 / C % 256 == 0 geometry runs the persistent kernel
  *                        and the kernels write with bulk (TMA) stores; otherwise a one-CTA-per-RoI kernel with scalar
  *                        stores.  Bit-identical results either way.
+ *                        NHWC (RSDET_ROI_NHWC_ROIS): the kernels store from registers, no staging and no bulk copy.  A base
+ *                        aligned to four elements (16 bytes fp32, 8 bytes half) takes the persistent kernel for that
+ *                        geometry and vector stores everywhere; otherwise the one-CTA-per-RoI kernel with scalar stores.
  *            levels_out  written as scalars.
  *   backward grad_out    16-byte aligned: staged with 16-byte loads; otherwise with scalar loads.  Same results.
+ *                        NHWC: read straight from global memory with the same rule, nothing staged.
  *            grad_feats  NCHW: written by the NHWC->NCHW copy, which uses 16-byte stores where the map allows them.
  *                        NHWC: the fast kernel accumulates with 16-byte vector reductions from each map's base; if
  *                        any base is not 16-byte aligned the call runs the generic kernel (scalar atomics).
@@ -201,7 +216,8 @@ int rsdet_roi_align_rotated_backward_typed(const rsdet_roi_align_cfg* cfg, int g
  *     Every multiply, divide and add is rounded separately, and taps that land on the same pixel are not merged.  Terms
  *     of weight 0 are dropped (adding +-0 to such a sum changes no bit), as are RoIs whose batch index is outside
  *     [0, batch).  Half maps get that fp32 value rounded once to nearest-even; a half grad_out converts exactly first.
- *   Consequences.  The same bits on every run, stream, CUDA-graph replay, layout (NCHW / channels-last), buffer alignment
+ *   Consequences.  The same bits on every run, stream, CUDA-graph replay, layout (NCHW / channels-last) and RoI-tensor
+ *     layout (RSDET_ROI_NHWC_ROIS), buffer alignment
  *     and batch split (a batched call equals per-image calls with each image's RoIs in the same relative order); and,
  *     for finite grad_out, bit-identity with the reference's arithmetic wherever the device's cosf / sinf agree with the
  *     host's (always at theta = 0).
@@ -211,7 +227,11 @@ int rsdet_roi_align_rotated_backward_typed(const rsdet_roi_align_cfg* cfg, int g
  *   Limit.  K * pooled_h * pooled_w * sampling_ratio^2 * 4 <= 2^28 terms and batch * sum_l(H_l * W_l) < 2^32 - 1 pixels;
  *     above either RSDET_ELIMIT (the workspace query returns 0).
  *   Resources.  No atomics, no host synchronisation, no allocation: every scratch buffer, the radix sort's temporary
- *     storage included, comes from the workspace, whose query is host-only.  Safe under CUDA-graph capture. */
+ *     storage included, comes from the workspace, whose query is host-only.  Safe under CUDA-graph capture.
+ *   RoI-tensor layout.  An NCHW-style grad_out is first copied bin-major, (K,ph,pw,C) in fp32, into the workspace.  An
+ *     NHWC grad_out (RSDET_ROI_NHWC_ROIS) is that array already: fp32 is read in place, half is converted to fp32 in the
+ *     workspace.  The query, which does not know the grad_out dtype, counts that fp32 array unless RSDET_ROI_NHWC_ROIS is
+ *     set and feat_dtype (hence grad_out) is F32. */
 size_t rsdet_roi_align_rotated_backward_deterministic_workspace_bytes(const rsdet_roi_align_cfg* cfg, int num_rois,
                                                                       int feat_dtype);
 int rsdet_roi_align_rotated_backward_deterministic(const rsdet_roi_align_cfg* cfg, int grad_out_dtype, const void* grad_out,

@@ -18,6 +18,7 @@ LIB_PATH = os.path.join(HERE, "librsdet.so")
 NMS_ROTATED, NMS_ROTATED_GE, NMS_POLY, NMS_MERGE, NMS_HBB, NMS_HBB_P1, NMS_HBB_P1_F64 = 0, 1, 2, 3, 4, 5, 6
 MAX_LEVELS = 8
 DTYPE_F32, DTYPE_F16, DTYPE_BF16 = 0, 1, 2
+ROI_NHWC_MAPS, ROI_NHWC_ROIS = 1, 2      # bits of RoiAlignCfg.channels_last
 
 _vp = C.c_void_p
 

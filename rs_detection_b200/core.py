@@ -14,7 +14,7 @@ import torch
 
 from . import _lib
 from ._lib import (DTYPE_BF16, DTYPE_F16, DTYPE_F32, MAX_LEVELS, NMS_HBB, NMS_MERGE, NMS_POLY, NMS_ROTATED, NMS_ROTATED_GE,
-                   RoiAlignCfg, check, load, ptr, stream_ptr, workspace)
+                   ROI_NHWC_MAPS, ROI_NHWC_ROIS, RoiAlignCfg, check, load, ptr, stream_ptr, workspace)
 
 _F64_KINDS = (NMS_MERGE, NMS_HBB, 6)  # 6 = NMS_HBB_P1_F64 (py_cpu_nms)
 _ROW = {NMS_ROTATED: 5, NMS_ROTATED_GE: 5, NMS_POLY: 8, NMS_MERGE: 8, NMS_HBB: 4, 5: 4, 6: 4}  # 5 = NMS_HBB_P1 (jt.nms)
@@ -287,17 +287,57 @@ def roi_feature_dtype(feats: Sequence[torch.Tensor]) -> torch.dtype:
     return half.pop()
 
 
+def _strictly_channels_last(t: torch.Tensor) -> bool:
+    """A 4-d tensor laid out (N, H, W, C) in memory that is not also plainly contiguous (C == 1 or H * W == 1 makes the
+    two layouts the same memory order; such a tensor takes the contiguous route)."""
+    return t.dim() == 4 and t.is_contiguous(memory_format=torch.channels_last) and not t.is_contiguous()
+
+
+def roi_maps_channels_last(feats: Sequence[torch.Tensor]) -> bool:
+    """Whether every level is a channels_last (N, C, H, W) tensor of a dtype the kernels read (fp32, fp16, bf16): such
+    pyramids get their gradient maps channels_last."""
+    return len(feats) > 0 and all(f.dtype in _ROI_DTYPES and _strictly_channels_last(f) for f in feats)
+
+
+def roi_maps_native(feats: Sequence[torch.Tensor]) -> bool:
+    """Whether the forward reads the levels as they are (RSDET_ROI_NHWC_MAPS): channels_last levels whose bases meet the
+    fast kernels' alignment rule of include/rsdet.h (four elements: 16 bytes fp32, 8 bytes half).  Any other base would
+    run the generic kernel, whose sums differ in the last bits from the fast kernels'; such levels take the NCHW route."""
+    return roi_maps_channels_last(feats) and all(f.data_ptr() % (4 * f.element_size()) == 0 for f in feats)
+
+
+def _roi_cfg_with(cfg: RoiAlignCfg, bits: int) -> RoiAlignCfg:
+    if not bits:
+        return cfg
+    c = RoiAlignCfg.from_buffer_copy(cfg)
+    c.channels_last |= bits
+    return c
+
+
 def roi_align_rotated_forward(cfg: RoiAlignCfg, feats: Sequence[torch.Tensor], rois: torch.Tensor, want_levels: bool = False,
-                              out: Optional[torch.Tensor] = None, out_dtype: Optional[torch.dtype] = None):
+                              out: Optional[torch.Tensor] = None, out_dtype: Optional[torch.dtype] = None,
+                              memory_format: torch.memory_format = torch.contiguous_format):
     """Half-precision levels (fp16 / bf16) are read natively; `out_dtype` is fp32 (None) or the levels' dtype.  An fp32
-    output equals, bit for bit, the call on the levels converted to fp32; a half output is that result rounded once."""
+    output equals, bit for bit, the call on the levels converted to fp32; a half output is that result rounded once.
+
+    Channels_last levels (logical (N, C, H, W)) are read in place when `roi_maps_native` holds; any other levels are
+    made contiguous first.  The output is a new (K, C, ph, pw) tensor in `memory_format` (torch.contiguous_format or
+    torch.channels_last), or `out`, contiguous or channels_last.  Layouts never change the values."""
     fdt = roi_feature_dtype(feats)
     odt = torch.float32 if out_dtype is None else out_dtype
     if odt not in (torch.float32, fdt):
         raise ValueError(f"RoIAlignRotated: out_dtype must be float32 or the features' {fdt}, got {odt}")
     if out is not None and out.dtype != odt:
         raise ValueError(f"RoIAlignRotated: out has dtype {out.dtype}, expected {odt}")
-    if fdt == torch.float32:
+    if memory_format not in (torch.contiguous_format, torch.channels_last):
+        raise ValueError(f"RoIAlignRotated: memory_format must be torch.contiguous_format or torch.channels_last, "
+                         f"got {memory_format}")
+    bits = 0
+    if not cfg.channels_last & ROI_NHWC_MAPS and roi_maps_native(feats):
+        bits |= ROI_NHWC_MAPS
+        if not all(f.is_cuda for f in feats):
+            raise RuntimeError("expected a CUDA tensor (no CPU fallback)")
+    elif fdt == torch.float32:
         feats = [_f32(f) for f in feats]
     elif all(f.is_cuda for f in feats):
         feats = [f.contiguous() for f in feats]
@@ -309,7 +349,12 @@ def roi_align_rotated_forward(cfg: RoiAlignCfg, feats: Sequence[torch.Tensor], r
     K = r.shape[0]
     dev = r.device
     if out is None:
-        out = torch.empty((K, cfg.channels, cfg.pooled_h, cfg.pooled_w), dtype=odt, device=dev)
+        out = torch.empty((K, cfg.channels, cfg.pooled_h, cfg.pooled_w), dtype=odt, device=dev, memory_format=memory_format)
+    if _strictly_channels_last(out):
+        bits |= ROI_NHWC_ROIS
+    elif not out.is_contiguous():
+        raise ValueError("RoIAlignRotated: out must be contiguous or channels_last")
+    cfg = _roi_cfg_with(cfg, bits)
     lv = torch.empty((K,), dtype=torch.int32, device=dev) if want_levels else None
     if K:
         L = load()
@@ -333,9 +378,12 @@ def roi_gather_kernel_ms(cfg: RoiAlignCfg, feats: Sequence[torch.Tensor], rois: 
 
 
 def roi_align_rotated_backward(cfg: RoiAlignCfg, grad_out: torch.Tensor, rois: torch.Tensor, feat_shapes,
-                               feat_dtype: torch.dtype = torch.float32, deterministic: bool = False):
+                               feat_dtype: torch.dtype = torch.float32, deterministic: bool = False,
+                               memory_format: torch.memory_format = torch.contiguous_format):
     """-> gradient maps in `feat_dtype` (fp32, fp16 or bf16; accumulated in fp32, rounded once).  A grad_out in fp32 or
-    in `feat_dtype` is read natively, any other dtype is cast to fp32.
+    in `feat_dtype` is read natively, any other dtype is cast to fp32.  A channels_last grad_out is read in place, a
+    contiguous one as it is, any other is made contiguous first.  `memory_format=torch.channels_last` returns logical
+    (N, C, H, W) maps laid out channels_last, written so by the library (no transpose).
 
     deterministic=False: the atomic backward (sums in an unspecified order).  deterministic=True: every gradient element
     is the reference's sequential fp32 sum in the reference's order, the same bits on every run
@@ -343,19 +391,32 @@ def roi_align_rotated_backward(cfg: RoiAlignCfg, grad_out: torch.Tensor, rois: t
     otherwise) and at most 2^28 terms K * PH * PW * sampling_ratio^2 * 4 (RuntimeError above)."""
     if feat_dtype not in _ROI_DTYPES:
         raise ValueError(f"RoIAlignRotated: gradient maps can be float32, float16 or bfloat16, not {feat_dtype}")
-    if grad_out.dtype in (torch.float32, feat_dtype):
-        if not grad_out.is_cuda:
-            raise RuntimeError("expected a CUDA tensor (no CPU fallback)")
-        g = grad_out.contiguous()
+    if memory_format not in (torch.contiguous_format, torch.channels_last):
+        raise ValueError(f"RoIAlignRotated: memory_format must be torch.contiguous_format or torch.channels_last, "
+                         f"got {memory_format}")
+    if not grad_out.is_cuda:
+        raise RuntimeError("expected a CUDA tensor (no CPU fallback)")
+    g = grad_out if grad_out.dtype in (torch.float32, feat_dtype) else grad_out.to(torch.float32)
+    bits = 0
+    if _strictly_channels_last(g):
+        bits |= ROI_NHWC_ROIS
     else:
-        g = _f32(grad_out)
+        g = g.contiguous()
+    maps_cl = memory_format == torch.channels_last and not cfg.channels_last & ROI_NHWC_MAPS
+    if maps_cl:
+        bits |= ROI_NHWC_MAPS
     r = _f32(rois)
     K = r.shape[0]
     dev = r.device
     grads = []
     for l, shp in enumerate(feat_shapes):
         n, c, h, w = [int(v) for v in shp]
-        grads.append(torch.empty((n, h, w, c) if cfg.channels_last else (n, c, h, w), dtype=feat_dtype, device=dev))
+        if maps_cl:
+            grads.append(torch.empty((n, c, h, w), dtype=feat_dtype, device=dev, memory_format=torch.channels_last))
+        else:
+            grads.append(torch.empty((n, h, w, c) if cfg.channels_last & ROI_NHWC_MAPS else (n, c, h, w), dtype=feat_dtype,
+                                     device=dev))
+    cfg = _roi_cfg_with(cfg, bits)
     L = load()
     fdt = _ROI_DTYPES[feat_dtype]
     if deterministic:

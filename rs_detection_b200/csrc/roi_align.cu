@@ -9,7 +9,7 @@
 //   * features are read channels-last (NHWC): one bilinear tap = one contiguous C*4-byte row, read as
 //     coalesced 16-byte vectors (a warp covers 512 contiguous bytes).  NCHW inputs (Jittor's layout)
 //     are transposed once per call by a tiled transpose into the workspace; callers that keep a
-//     channels-last pyramid skip it (cfg.channels_last).
+//     channels-last pyramid skip it (RSDET_ROI_NHWC_MAPS in cfg.channels_last).
 //   * one CTA per RoI.  Phase A: the RoI's sampling grid (pooled_h*pooled_w*grid^2 samples -> 4 tap
 //     offsets + 4 weights each) is computed ONCE by the first threads and staged in shared memory; the
 //     reference recomputes it, sin/cos included, in every one of its K*C*49 threads.
@@ -332,6 +332,7 @@ template <typename T> __device__ __forceinline__ decltype(auto) quad_f32(const t
 }
 // the same load as fp32
 template <typename T> __device__ __forceinline__ float4 ldg4(const T* p) { return quad_f32<T>(ldg4_raw(p)); }
+
 __device__ __forceinline__ float4 ldg_cs_v4(const float* p) {
     float4 r;
     asm volatile("ld.global.cs.v4.f32 {%0,%1,%2,%3}, [%4];" : "=f"(r.x), "=f"(r.y), "=f"(r.z), "=f"(r.w) : "l"(p));
@@ -351,6 +352,28 @@ template <typename T>
 __device__ __forceinline__ void stcs1(T* p, T v) {           // streaming scalar store
     if constexpr (kIsF32<T>) __stcs(p, v);
     else asm volatile("st.global.cs.b16 [%0], %1;" ::"l"(p), "h"(*reinterpret_cast<const unsigned short*>(&v)) : "memory");
+}
+// streaming 4-channel store of an fp32 quad: one 16-byte store (fp32) or one 8-byte store of values rounded to
+// nearest-even (p aligned to 4 * sizeof(T)); stcs4_scalar: the same values with four scalar stores
+template <typename T>
+__device__ __forceinline__ void stcs4(T* p, float4 v) {
+    if constexpr (kIsF32<T>) __stcs(reinterpret_cast<float4*>(p), v);
+    else { const uint2 u = pack4<T>(v); asm volatile("st.global.cs.v2.b32 [%0], {%1,%2};" ::"l"(p), "r"(u.x), "r"(u.y) : "memory"); }
+}
+template <typename T>
+__device__ __forceinline__ void stcs4_scalar(T* p, float4 v) {
+    stcs1(p, from_f32<T>(v.x)); stcs1(p + 1, from_f32<T>(v.y)); stcs1(p + 2, from_f32<T>(v.z)); stcs1(p + 3, from_f32<T>(v.w));
+}
+// 4-channel store with an L2 cache policy (createpolicy): 16 bytes (fp32) or 8 bytes of values rounded to nearest-even
+template <typename T>
+__device__ __forceinline__ void st4_policy(T* p, float4 v, unsigned long long pol) {
+    if constexpr (kIsF32<T>) {
+        asm volatile("st.global.L2::cache_hint.v4.f32 [%0], {%1,%2,%3,%4}, %5;" ::"l"(p), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w),
+                     "l"(pol) : "memory");
+    } else {
+        const uint2 u = pack4<T>(v);
+        asm volatile("st.global.L2::cache_hint.v2.b32 [%0], {%1,%2}, %3;" ::"l"(p), "r"(u.x), "r"(u.y), "l"(pol) : "memory");
+    }
 }
 // shared -> global bulk copy (cp.async.bulk, SASS UBLKCP) with an evict-first L2 policy: the output stream must
 // not push the feature pyramid out of L2.  Returns once the source has been read (shared memory may be reused
@@ -763,7 +786,9 @@ __device__ __forceinline__ float4 unrot4(float4 v, int o) { return rot4(v, (4 - 
 // One CTA per (RoI, chunk of up to 64 channel quads), thread = (channel quad(s), bin group).  QPT = 2:
 // the second channel quad is an immediate +512 B off the same address.  Launch bounds for THREE CTAs per SM: the driver then
 // picks the 196 KB carve-out (60 KB of L1 instead of 28) -- 143.2 -> 131.9 us per bench tile (profiles/README.md, third pass).
-template <int QPT, typename T = float, typename O = float>   // T: feature elements, O: output elements
+// NHWC_OUT: out is (K, PH, PW, C) -- a thread stores its channel quads of a bin straight to global memory, with vector stores
+// when out's base is aligned to four elements (scalar stores otherwise), and the staging block is only phase-A scratch.
+template <int QPT, typename T = float, typename O = float, bool NHWC_OUT = false>   // T: feature elements, O: output elements
 __global__ void __launch_bounds__(kRoiThreads, 3)
 roi_align_fwd_kernel(LevelSet L, const float* __restrict__ rois, const int* __restrict__ order, const RoiGeom* __restrict__ geoms,
                      int K, O* __restrict__ out, int32_t* __restrict__ levels_out) {
@@ -802,6 +827,7 @@ roi_align_fwd_kernel(LevelSet L, const float* __restrict__ rois, const int* __re
         reinterpret_cast<const typename Quad<T>::V*>(feat_base<T>(L, g.level) + (size_t)g.batch * H * W * C + chunk0) + cq;
     const bool pow2 = (spb & (spb - 1)) == 0;
     const float count = (float)max(spb, 1), inv_count = 1.f / count;
+    [[maybe_unused]] const bool out_vec = (((size_t)out) & (4 * sizeof(O) - 1)) == 0;
     if (grp < groups) {
         for (int b = grp; b < nbins; b += groups) {
             float4 acc[QPT];
@@ -839,6 +865,12 @@ roi_align_fwd_kernel(LevelSet L, const float* __restrict__ rois, const int* __re
                 if (pow2) { acc[u].x *= inv_count; acc[u].y *= inv_count; acc[u].z *= inv_count; acc[u].w *= inv_count; }
                 else { acc[u].x /= count; acc[u].y /= count; acc[u].z /= count; acc[u].w /= count; }
                 const int c0 = (cq + u * 32) * 4;
+                if constexpr (NHWC_OUT) {
+                    O* const p = out + ((size_t)roi * nbins + b) * C + chunk0 + c0;
+                    if (out_vec) stcs4(p, acc[u]);
+                    else stcs4_scalar(p, acc[u]);
+                    continue;
+                }
                 const float4 r = rot4(acc[u], oct);
                 s_stage[(c0 + ((0 + oct) & 3)) * nbins + b] = from_f32<O>(r.x);
                 s_stage[(c0 + ((1 + oct) & 3)) * nbins + b] = from_f32<O>(r.y);
@@ -847,6 +879,7 @@ roi_align_fwd_kernel(LevelSet L, const float* __restrict__ rois, const int* __re
             }
         }
     }
+    if constexpr (NHWC_OUT) return;
     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
     __syncthreads();
     // the staged block IS the output block of this (roi, chunk): one bulk copy shared -> global (TMA) when it is
@@ -890,8 +923,10 @@ constexpr int kFwd77pWarps = 8, kFwd77pCtasPerSm = 3;
 constexpr int kFwd77pTaps = 4;   // list entries per batch: 8 vector loads in flight per thread
 constexpr size_t kStage77pOffset = (8 * 49 * 18 + 16 + 48 + 127) & ~(size_t)127;   // lists | next item | next record | staging
 // T: feature elements (a half map halves the bytes of every tap load: two 8-byte loads per lane and tap); O: output
-// elements (a half output halves the staging block and its bulk store)
-template <typename T, typename O>
+// elements (a half output halves the staging block and its bulk store).  NHWC_OUT: out is (K, 7, 7, C); a lane's two
+// channel quads of a bin are contiguous 16-byte (8-byte when half) pieces of it, stored straight from registers with the
+// same evict-first L2 policy -- no staging block, no bulk copy, and only the lists and the record in shared memory.
+template <typename T, typename O, bool NHWC_OUT = false>
 __global__ void __launch_bounds__(32 * kFwd77pWarps, kFwd77pCtasPerSm)
 roi_align_fwd77p_kernel(LevelSet L, const int* __restrict__ order, const RoiGeom* __restrict__ geoms, int K, int chunks,
                         O* __restrict__ out, unsigned* __restrict__ counter) {
@@ -906,6 +941,8 @@ roi_align_fwd77p_kernel(LevelSet L, const int* __restrict__ order, const RoiGeom
     const int C = L.C, items = K * chunks;
     const int oct = (lane >> 3) & 3;
     O* const sbase = s_stage + lane * 4 * NB;
+    [[maybe_unused]] unsigned long long pol = 0;   // NHWC_OUT: the output stores' L2 policy
+    if constexpr (NHWC_OUT) asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(pol));
     int idx = blockIdx.x;
     if (tid < 3 && idx < items) {
         const int r = order ? order[idx / chunks] : idx / chunks;      // position in processing order -> RoI
@@ -954,7 +991,7 @@ roi_align_fwd77p_kernel(LevelSet L, const int* __restrict__ order, const RoiGeom
             s_list[b * PITCH + 16] = make_int2(pos, 0);
         }
         if (tid == THREADS - 1) {      // a thread without A1 / A2 work: the previous block must have left the staging area; next item
-            asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");   // returns at once when nothing is pending
+            if constexpr (!NHWC_OUT) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");   // returns at once when nothing is pending
             *s_next = (int)(atomicAdd(counter, 1u) + gridDim.x);
         }
         __syncthreads();
@@ -972,6 +1009,12 @@ roi_align_fwd77p_kernel(LevelSet L, const int* __restrict__ order, const RoiGeom
         auto stage = [&](float4 a0, float4 a1, int b) {
             a0.x *= 0.25f; a0.y *= 0.25f; a0.z *= 0.25f; a0.w *= 0.25f;   // output_val /= count (:143), count = 4: exact
             a1.x *= 0.25f; a1.y *= 0.25f; a1.z *= 0.25f; a1.w *= 0.25f;
+            if constexpr (NHWC_OUT) {
+                O* const p = out + ((size_t)roi * NB + b) * C + chunk0 + lane * 4;
+                st4_policy(p, a0, pol);
+                st4_policy(p + 128, a1, pol);
+                return;
+            }
             const float4 r0 = rot4(a0, oct), r1 = rot4(a1, oct);
             O* const sb = sbase + b;
             O* const q0 = sb + ((0 + oct) & 3) * NB;
@@ -1023,6 +1066,11 @@ roi_align_fwd77p_kernel(LevelSet L, const int* __restrict__ order, const RoiGeom
             cnt = ncnt;
         }
         if (tid < 3) asm volatile("cp.async.wait_all;" ::: "memory");
+        if constexpr (NHWC_OUT) {
+            __syncthreads();           // the record has landed, every warp is done with the lists
+            idx = *s_next;
+            continue;
+        }
         asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
         __syncthreads();
         if (tid == THREADS - 1) {      // the thread that will wait for it
@@ -1034,7 +1082,8 @@ roi_align_fwd77p_kernel(LevelSet L, const int* __restrict__ order, const RoiGeom
         }
         idx = *s_next;
     }
-    if (tid == THREADS - 1) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
+    if constexpr (!NHWC_OUT)
+        if (tid == THREADS - 1) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
 }
 
 // cudaFuncSetAttribute is per device: remember what was set for each one (a process may drive several GPUs)
@@ -1078,7 +1127,9 @@ static bool fwd77_ok(const rsdet_roi_align_cfg* c) {
 // Same CTA shape and tap lists.  The RoI's (C,7,7) gradient block is copied into shared memory as it
 // lies in memory (coalesced 16-byte loads); every merged tap becomes ONE 16-byte vector reduction per
 // channel quad (red.global.add.v4.f32) into the channels-last accumulator.
-template <int QPT, typename G = float>   // G: grad_out elements (staged as fp32); the accumulators are always fp32
+// NHWC_IN: grad_out is (K, PH, PW, C); a thread reads its channel quads of a bin straight from global memory (vector loads
+// when grad_out's base is aligned to four elements, scalar loads otherwise) and nothing is staged.
+template <int QPT, typename G = float, bool NHWC_IN = false>   // G: grad_out elements (staged as fp32); the accumulators are always fp32
 __global__ void __launch_bounds__(kRoiThreads, 4)
 roi_align_bwd_kernel(LevelSet L, const float* __restrict__ rois, const int* __restrict__ order, const RoiGeom* __restrict__ geoms,
                      int K, const G* __restrict__ grad_out) {
@@ -1105,16 +1156,18 @@ roi_align_bwd_kernel(LevelSet L, const float* __restrict__ rois, const int* __re
     const int H = L.H[g.level], W = L.W[g.level];
     build_tap_lists(g, L, H, W, s_list, s_cnt, s_stage, C >> 2);
 
-    // stage this chunk's gradient block [c_local][bin] (= memory order)
-    const G* __restrict__ src = grad_out + ((size_t)roi * C + chunk0) * nbins;
-    const int total = Qc * 4 * nbins;
-    if ((((size_t)roi * C + chunk0) * nbins & 3) == 0 && (total & 3) == 0 && (((size_t)grad_out) & (4 * sizeof(G) - 1)) == 0) {
-        float4* s4 = reinterpret_cast<float4*>(s_stage);
-        for (int e = tid; e < total / 4; e += kRoiThreads) s4[e] = ldcs4(src + (size_t)e * 4);
-    } else {
-        for (int e = tid; e < total; e += kRoiThreads) s_stage[e] = to_f32(__ldg(src + e));
+    if constexpr (!NHWC_IN) {
+        // stage this chunk's gradient block [c_local][bin] (= memory order)
+        const G* __restrict__ src = grad_out + ((size_t)roi * C + chunk0) * nbins;
+        const int total = Qc * 4 * nbins;
+        if ((((size_t)roi * C + chunk0) * nbins & 3) == 0 && (total & 3) == 0 && (((size_t)grad_out) & (4 * sizeof(G) - 1)) == 0) {
+            float4* s4 = reinterpret_cast<float4*>(s_stage);
+            for (int e = tid; e < total / 4; e += kRoiThreads) s4[e] = ldcs4(src + (size_t)e * 4);
+        } else {
+            for (int e = tid; e < total; e += kRoiThreads) s_stage[e] = to_f32(__ldg(src + e));
+        }
+        __syncthreads();
     }
-    __syncthreads();
 
     const int lanes = QPT == 2 ? 32 : Qc;
     const int groups = kRoiThreads / lanes;
@@ -1123,12 +1176,18 @@ roi_align_bwd_kernel(LevelSet L, const float* __restrict__ rois, const int* __re
     float4* __restrict__ gfeat = reinterpret_cast<float4*>(L.grad[g.level] + (size_t)g.batch * H * W * C + chunk0) + cq;
     const bool pow2 = (spb & (spb - 1)) == 0;
     const float count = (float)spb, inv_count = 1.f / count;  // no max(.,1) in backward (:246)
+    [[maybe_unused]] const bool g_vec = (((size_t)grad_out) & (4 * sizeof(G) - 1)) == 0;
     if (grp < groups) {
         for (int b = grp; b < nbins; b += groups) {
             float4 top[QPT];
 #pragma unroll
             for (int u = 0; u < QPT; u++) {
                 const int c0 = (cq + u * 32) * 4;
+                if constexpr (NHWC_IN) {
+                    const G* const p = grad_out + ((size_t)roi * nbins + b) * C + chunk0 + c0;
+                    top[u] = g_vec ? ldcs4(p) : make_float4(to_f32(__ldg(p)), to_f32(__ldg(p + 1)), to_f32(__ldg(p + 2)), to_f32(__ldg(p + 3)));
+                    continue;
+                }
                 float4 r;
                 r.x = s_stage[(c0 + ((0 + oct) & 3)) * nbins + b];
                 r.y = s_stage[(c0 + ((1 + oct) & 3)) * nbins + b];
@@ -1170,15 +1229,24 @@ __device__ __forceinline__ size_t feat_index(int cl, int n, int c, int pix, int 
 }
 
 // T: feature elements (forward); O: output elements (forward) or grad_out elements (backward); gradients accumulate in
-// fp32 maps (M.grad) in the caller's layout
-template <bool BACKWARD, typename T = float, typename O = float>
+// fp32 maps (M.grad) in the caller's layout.  NHWC_ROIS: out / grad_out is (K, PH, PW, C), and consecutive threads take
+// consecutive channels of it.
+template <bool BACKWARD, typename T = float, typename O = float, bool NHWC_ROIS = false>
 __global__ void roi_align_generic_kernel(LevelSet L, GenericMaps M, const float* __restrict__ rois, int K,
                                          O* __restrict__ out_or_gradout, int32_t* __restrict__ levels_out) {
     const int nbins = L.PH * L.PW;
     const long long total = (long long)K * L.C * nbins;
     for (long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x; idx < total; idx += (long long)gridDim.x * blockDim.x) {
-        int pw = (int)(idx % L.PW), ph = (int)((idx / L.PW) % L.PH);
-        int c = (int)((idx / nbins) % L.C), n = (int)(idx / nbins / L.C);
+        int pw, ph, c, n;
+        if constexpr (NHWC_ROIS) {
+            c = (int)(idx % L.C);
+            const int bin = (int)((idx / L.C) % nbins);
+            n = (int)(idx / L.C / nbins);
+            ph = bin / L.PW; pw = bin % L.PW;
+        } else {
+            pw = (int)(idx % L.PW); ph = (int)((idx / L.PW) % L.PH);
+            c = (int)((idx / nbins) % L.C); n = (int)(idx / nbins / L.C);
+        }
         RoiGeom g = roi_geometry(rois + (size_t)n * 6, L);
         if (!BACKWARD && levels_out && c == 0 && ph == 0 && pw == 0) levels_out[n] = g.level;
         const int H = L.H[g.level], W = L.W[g.level];
@@ -1227,9 +1295,13 @@ static bool fast_path_ok(const rsdet_roi_align_cfg* c) {
 // accesses from each level's base pointer (16 bytes for fp32, 8 for half maps); a base that is not aligned to that goes
 // to the scalar generic kernel, which addresses NHWC maps directly.  NCHW maps are only read by the transposes, which
 // check alignment themselves.
+// the layout bits of cfg.channels_last (include/rsdet.h)
+static bool nhwc_maps(const rsdet_roi_align_cfg* c) { return (c->channels_last & RSDET_ROI_NHWC_MAPS) != 0; }
+static bool nhwc_rois(const rsdet_roi_align_cfg* c) { return (c->channels_last & RSDET_ROI_NHWC_ROIS) != 0; }
+
 template <typename P>
 static bool nhwc_bases_aligned(const rsdet_roi_align_cfg* c, P const* maps, size_t align) {
-    if (!c->channels_last) return true;
+    if (!nhwc_maps(c)) return true;
     for (int l = 0; l < c->num_levels; l++)
         if (((size_t)maps[l]) & (align - 1)) return false;
     return true;
@@ -1239,6 +1311,7 @@ static int check_cfg(const rsdet_roi_align_cfg* c) {
     if (!c) return RSDET_EINVAL;
     if (c->num_levels < 1 || c->num_levels > RSDET_MAX_LEVELS || c->batch < 1 || c->channels < 1) return RSDET_EINVAL;
     if (c->pooled_h < 1 || c->pooled_w < 1 || (c->version != 0 && c->version != 1)) return RSDET_EINVAL;
+    if (c->channels_last & ~(RSDET_ROI_NHWC_MAPS | RSDET_ROI_NHWC_ROIS)) return RSDET_EINVAL;
     for (int l = 0; l < c->num_levels; l++)
         if (c->height[l] < 1 || c->width[l] < 1) return RSDET_EINVAL;
     return RSDET_OK;
@@ -1281,7 +1354,7 @@ static size_t roi_workspace_bytes(const rsdet_roi_align_cfg* cfg, int num_rois, 
             b += ws_bytes<float>((size_t)cfg->batch * cfg->channels * cfg->height[l] * cfg->width[l]);
         return b + 256;
     }
-    if (cfg->channels_last || !fast_path_ok(cfg)) return b + 256;
+    if (nhwc_maps(cfg) || !fast_path_ok(cfg)) return b + 256;
     for (int l = 0; l < cfg->num_levels; l++)      // NHWC copy of the pyramid (forward) / fp32 NHWC accumulators (backward)
         b += align256(elem * cfg->batch * cfg->channels * cfg->height[l] * cfg->width[l]);
     return b + 256;
@@ -1297,22 +1370,22 @@ extern "C" size_t rsdet_roi_align_rotated_workspace_bytes(const rsdet_roi_align_
     return rsdet_roi_align_rotated_workspace_bytes_typed(cfg, num_rois, backward, RSDET_DTYPE_F32);
 }
 
-// T: feature elements, O: output elements (float or T).  Arguments are checked by the caller.
-template <typename T, typename O>
+// T: feature elements, O: output elements (float or T), NHWC_OUT: out is (K, PH, PW, C).  Arguments are checked by the caller.
+template <typename T, typename O, bool NHWC_OUT>
 static int forward_impl(const rsdet_roi_align_cfg* cfg, const T* const* feats_host, const float* rois, int num_rois, O* out,
                         int32_t* levels_out, void* workspace, size_t workspace_bytes, cudaStream_t st) {
     int rc = RSDET_OK;
     LevelSet L = make_levels(cfg);
     if (!fast_path_ok(cfg) || !nhwc_bases_aligned(cfg, feats_host, 4 * sizeof(T))) {
         GenericMaps M;
-        M.channels_last = cfg->channels_last;
+        M.channels_last = nhwc_maps(cfg);
         for (int l = 0; l < RSDET_MAX_LEVELS; l++) {
             M.feat[l] = l < cfg->num_levels ? reinterpret_cast<const float*>(feats_host[l]) : nullptr;
             M.grad[l] = nullptr;
         }
         long long total = (long long)num_rois * cfg->channels * cfg->pooled_h * cfg->pooled_w;
         int grid = (int)(ceil_div_ll(total, 256) < (long long)kNumSMs * 16 ? ceil_div_ll(total, 256) : (long long)kNumSMs * 16);
-        roi_align_generic_kernel<false, T, O><<<grid, 256, 0, st>>>(L, M, rois, num_rois, out, levels_out);
+        roi_align_generic_kernel<false, T, O, NHWC_OUT><<<grid, 256, 0, st>>>(L, M, rois, num_rois, out, levels_out);
         count_launch();
         return cuda_status();
     }
@@ -1321,7 +1394,7 @@ static int forward_impl(const rsdet_roi_align_cfg* cfg, const T* const* feats_ho
     int* order_ws = ws.take<int>(num_rois);
     RoiGeom* geoms = ws.take<RoiGeom>(num_rois);
     unsigned* counter = ws.take<unsigned>(1);
-    if (cfg->channels_last) {
+    if (nhwc_maps(cfg)) {
         for (int l = 0; l < cfg->num_levels; l++) L.feat[l] = reinterpret_cast<const float*>(feats_host[l]);
     } else {
         for (int l = 0; l < cfg->num_levels; l++)
@@ -1330,17 +1403,18 @@ static int forward_impl(const rsdet_roi_align_cfg* cfg, const T* const* feats_ho
     }
     // locality order (needs the int[K] slot at the start of the workspace; skipped for tiny calls)
     int* order = num_rois >= 256 && order_ws ? order_ws : nullptr;
-    const bool ride = !cfg->channels_last && order && num_rois <= kPrepMaxRois;
-    // the persistent 7x7 kernel (it needs a 16-byte aligned output for its bulk stores) and its lean prologue: records by
-    // RoI index only, one launch, and for NCHW callers no launch at all -- order block and geometry blocks ride with the
-    // transpose.  Everything else runs roi_align_fwd_kernel behind the order and geometry kernels.
-    const bool lean = fwd77_ok(cfg) && (((size_t)out) & 15) == 0;
+    const bool ride = !nhwc_maps(cfg) && order && num_rois <= kPrepMaxRois;
+    // the persistent 7x7 kernel (it needs a 16-byte aligned output for its bulk stores; an NHWC output, stored from
+    // registers, needs four-element alignment) and its lean prologue: records by RoI index only, one launch, and for NCHW
+    // callers no launch at all -- order block and geometry blocks ride with the transpose.  Everything else runs
+    // roi_align_fwd_kernel behind the order and geometry kernels.
+    const bool lean = fwd77_ok(cfg) && (((size_t)out) & (NHWC_OUT ? 4 * sizeof(O) - 1 : 15)) == 0;
     if (!lean) launch_prep(L, rois, num_rois, geoms, order, levels_out, st, ride);
     else if (!ride) {
         roi_prep_kernel<<<(order ? 1 : 0) + ceil_div(num_rois, 1024), 1024, 0, st>>>(L, rois, num_rois, order, geoms, levels_out, counter);
         count_launch();
     }
-    if (!cfg->channels_last) {
+    if (!nhwc_maps(cfg)) {
         // NCHW -> NHWC copy of the pyramid; the locality-order block rides along as block 0 of the same launch
         PrepArgs prep = {&L, rois, num_rois, order};
         if (lean) { prep.geoms = geoms; prep.levels_out = levels_out; prep.counter = counter; }
@@ -1355,9 +1429,9 @@ static int forward_impl(const rsdet_roi_align_cfg* cfg, const T* const* feats_ho
     if (lean) {
         const int chunks = cfg->channels / 256;
         const long long items = (long long)num_rois * chunks, ctas = kNumSMs * kFwd77pCtasPerSm;
-        const size_t smp = kStage77pOffset + sizeof(float) * 49 * 256;
-        set_dyn_smem((const void*)roi_align_fwd77p_kernel<T, O>, smp);
-        roi_align_fwd77p_kernel<T, O><<<(int)(items < ctas ? items : ctas), 32 * kFwd77pWarps, smp, st>>>(
+        const size_t smp = kStage77pOffset + (NHWC_OUT ? 0 : sizeof(float) * 49 * 256);
+        set_dyn_smem((const void*)roi_align_fwd77p_kernel<T, O, NHWC_OUT>, smp);
+        roi_align_fwd77p_kernel<T, O, NHWC_OUT><<<(int)(items < ctas ? items : ctas), 32 * kFwd77pWarps, smp, st>>>(
             L, order, geoms, num_rois, chunks, out, counter);
         count_launch();
         return cuda_status();
@@ -1366,11 +1440,11 @@ static int forward_impl(const rsdet_roi_align_cfg* cfg, const T* const* feats_ho
     const int Q = quads_per_chunk(cfg->channels);
     dim3 grid(num_rois, ceil_div(cfg->channels / 4, Q));
     if (cfg->channels % 256 == 0) {
-        set_dyn_smem((const void*)roi_align_fwd_kernel<2, T, O>, smem);
-        roi_align_fwd_kernel<2, T, O><<<grid, kRoiThreads, smem, st>>>(L, rois, order, geoms, num_rois, out, nullptr);
+        set_dyn_smem((const void*)roi_align_fwd_kernel<2, T, O, NHWC_OUT>, smem);
+        roi_align_fwd_kernel<2, T, O, NHWC_OUT><<<grid, kRoiThreads, smem, st>>>(L, rois, order, geoms, num_rois, out, nullptr);
     } else {
-        set_dyn_smem((const void*)roi_align_fwd_kernel<1, T, O>, smem);
-        roi_align_fwd_kernel<1, T, O><<<grid, kRoiThreads, smem, st>>>(L, rois, order, geoms, num_rois, out, nullptr);
+        set_dyn_smem((const void*)roi_align_fwd_kernel<1, T, O, NHWC_OUT>, smem);
+        roi_align_fwd_kernel<1, T, O, NHWC_OUT><<<grid, kRoiThreads, smem, st>>>(L, rois, order, geoms, num_rois, out, nullptr);
     }
     count_launch();
     return cuda_status();
@@ -1389,8 +1463,11 @@ extern "C" int rsdet_roi_align_rotated_forward_typed(const rsdet_roi_align_cfg* 
         if (!feats_host[l]) return RSDET_EINVAL;
     cudaStream_t st = (cudaStream_t)stream;
     const bool half_out = out_dtype != RSDET_DTYPE_F32;
-#define RSDET_FWD(T_, O_) forward_impl<T_, O_>(cfg, reinterpret_cast<const T_* const*>(feats_host), rois, num_rois, static_cast<O_*>(out), \
-                                               levels_out, workspace, workspace_bytes, st)
+#define RSDET_FWD(T_, O_)                                                                                                      \
+    (nhwc_rois(cfg) ? forward_impl<T_, O_, true>(cfg, reinterpret_cast<const T_* const*>(feats_host), rois, num_rois,             \
+                                                 static_cast<O_*>(out), levels_out, workspace, workspace_bytes, st)              \
+                    : forward_impl<T_, O_, false>(cfg, reinterpret_cast<const T_* const*>(feats_host), rois, num_rois,            \
+                                                  static_cast<O_*>(out), levels_out, workspace, workspace_bytes, st))
     if (feat_dtype == RSDET_DTYPE_F16) return half_out ? RSDET_FWD(__half, __half) : RSDET_FWD(__half, float);
     if (feat_dtype == RSDET_DTYPE_BF16) return half_out ? RSDET_FWD(__nv_bfloat16, __nv_bfloat16) : RSDET_FWD(__nv_bfloat16, float);
     return RSDET_FWD(float, float);
@@ -1426,13 +1503,13 @@ static int launch_convert(const rsdet_roi_align_cfg* cfg, float* const* acc, D* 
 // generic kernel -- and ONE pass writes the caller's maps from them, rounding to nearest-even: the NHWC->NCHW transpose,
 // or a conversion that keeps the layout.  The fast kernels then never touch the caller's maps, so their alignment does
 // not matter.
-template <typename G, typename T>
+template <typename G, typename T, bool NHWC_IN>   // NHWC_IN: grad_out is (K, PH, PW, C)
 static int backward_impl(const rsdet_roi_align_cfg* cfg, const G* grad_out, const float* rois, int num_rois, T* const* grad_feats_host,
                          void* workspace, size_t workspace_bytes, cudaStream_t st) {
     int rc = RSDET_OK;
     LevelSet L = make_levels(cfg);
     const bool fast = fast_path_ok(cfg) && (!kIsF32<T> || nhwc_bases_aligned(cfg, grad_feats_host, 16));
-    const bool direct = kIsF32<T> && (cfg->channels_last || !fast);  // accumulate straight into the caller's buffers
+    const bool direct = kIsF32<T> && (nhwc_maps(cfg) || !fast);  // accumulate straight into the caller's buffers
     float* acc[RSDET_MAX_LEVELS];
     if (workspace_bytes < roi_workspace_bytes(cfg, num_rois, 1, sizeof(T))) return RSDET_EWORKSPACE;
     Workspace ws(workspace, workspace_bytes);
@@ -1454,27 +1531,27 @@ static int backward_impl(const rsdet_roi_align_cfg* cfg, const G* grad_out, cons
         if (!grad_out || !rois) return RSDET_EINVAL;
         if (!fast) {
             GenericMaps M;
-            M.channels_last = cfg->channels_last;
+            M.channels_last = nhwc_maps(cfg);
             for (int l = 0; l < RSDET_MAX_LEVELS; l++) { M.feat[l] = nullptr; M.grad[l] = l < cfg->num_levels ? acc[l] : nullptr; }
             long long total = (long long)num_rois * cfg->channels * cfg->pooled_h * cfg->pooled_w;
             int grid = (int)(ceil_div_ll(total, 256) < (long long)kNumSMs * 16 ? ceil_div_ll(total, 256) : (long long)kNumSMs * 16);
-            roi_align_generic_kernel<true, float, G><<<grid, 256, 0, st>>>(L, M, rois, num_rois, const_cast<G*>(grad_out), nullptr);
+            roi_align_generic_kernel<true, float, G, NHWC_IN><<<grid, 256, 0, st>>>(L, M, rois, num_rois, const_cast<G*>(grad_out), nullptr);
         } else {
             size_t smem = fwd_smem_bytes(cfg);
-            set_dyn_smem((const void*)roi_align_bwd_kernel<1, G>, smem);
-            set_dyn_smem((const void*)roi_align_bwd_kernel<2, G>, smem);
+            set_dyn_smem((const void*)roi_align_bwd_kernel<1, G, NHWC_IN>, smem);
+            set_dyn_smem((const void*)roi_align_bwd_kernel<2, G, NHWC_IN>, smem);
             int* order = num_rois >= 256 ? order_ws : nullptr;
             launch_prep(L, rois, num_rois, geoms, order, nullptr, st);
             int Q = quads_per_chunk(cfg->channels);
             dim3 grid(num_rois, ceil_div(cfg->channels / 4, Q));
-            if (cfg->channels % 256 == 0) roi_align_bwd_kernel<2, G><<<grid, kRoiThreads, smem, st>>>(L, rois, order, geoms, num_rois, grad_out);
-            else roi_align_bwd_kernel<1, G><<<grid, kRoiThreads, smem, st>>>(L, rois, order, geoms, num_rois, grad_out);
+            if (cfg->channels % 256 == 0) roi_align_bwd_kernel<2, G, NHWC_IN><<<grid, kRoiThreads, smem, st>>>(L, rois, order, geoms, num_rois, grad_out);
+            else roi_align_bwd_kernel<1, G, NHWC_IN><<<grid, kRoiThreads, smem, st>>>(L, rois, order, geoms, num_rois, grad_out);
         }
         count_launch();
     }
     if (!direct) {
         if constexpr (!kIsF32<T>) {
-            if (!fast || cfg->channels_last) return launch_convert(cfg, acc, grad_feats_host, st);
+            if (!fast || nhwc_maps(cfg)) return launch_convert(cfg, acc, grad_feats_host, st);
         }
         rc = launch_transpose(false, acc, grad_feats_host, cfg->height, cfg->width, cfg->num_levels, cfg->batch, cfg->channels, st);
         if (rc != RSDET_OK) return rc;
@@ -1493,8 +1570,11 @@ extern "C" int rsdet_roi_align_rotated_backward_typed(const rsdet_roi_align_cfg*
         if (!grad_feats_host[l]) return RSDET_EINVAL;
     cudaStream_t st = (cudaStream_t)stream;
     const bool half_g = grad_out_dtype != RSDET_DTYPE_F32;
-#define RSDET_BWD(G_, T_) backward_impl<G_, T_>(cfg, static_cast<const G_*>(grad_out), rois, num_rois, \
-                                                reinterpret_cast<T_* const*>(grad_feats_host), workspace, workspace_bytes, st)
+#define RSDET_BWD(G_, T_)                                                                                                      \
+    (nhwc_rois(cfg) ? backward_impl<G_, T_, true>(cfg, static_cast<const G_*>(grad_out), rois, num_rois,                         \
+                                                  reinterpret_cast<T_* const*>(grad_feats_host), workspace, workspace_bytes, st) \
+                    : backward_impl<G_, T_, false>(cfg, static_cast<const G_*>(grad_out), rois, num_rois,                        \
+                                                   reinterpret_cast<T_* const*>(grad_feats_host), workspace, workspace_bytes, st))
     if (feat_dtype == RSDET_DTYPE_F16) return half_g ? RSDET_BWD(__half, __half) : RSDET_BWD(float, __half);
     if (feat_dtype == RSDET_DTYPE_BF16) return half_g ? RSDET_BWD(__nv_bfloat16, __nv_bfloat16) : RSDET_BWD(float, __nv_bfloat16);
     return RSDET_BWD(float, float);
@@ -1518,7 +1598,8 @@ extern "C" int rsdet_roi_align_rotated_backward(const rsdet_roi_align_cfg* cfg, 
 //      nothing to a sum that starts at +0), the entry index and the weight;
 //   2. a stable LSD radix sort of (key, entry index) over the key's bits groups the entries by pixel and keeps the
 //      reference's order inside each pixel;
-//   3. grad_out (K, C, bins) is copied bin-major to (K, bins, C), so that a term reads C contiguous values;
+//   3. grad_out (K, C, bins) is copied bin-major to (K, bins, C), so that a term reads C contiguous values (a (K, bins, C)
+//      grad_out is read in place when fp32 and widened to fp32 when half);
 //   4. roi_bwd_det_gather_kernel: one warp per touched pixel, lanes over channels, adds the pixel's terms in sorted
 //      order with separately rounded multiply, divide and add, and stores the C sums once (plain stores, no atomics).
 // Untouched pixels keep the zero fill that precedes step 4; NCHW and fp32-accumulated half maps reuse the output passes
@@ -1644,6 +1725,13 @@ __global__ void __launch_bounds__(256) roi_bwd_det_gather_kernel(DetJob J, const
     }
 }
 
+// a (K, PH, PW, C) half grad_out -> the fp32 bin-major array the gather reads (exact conversion, same layout)
+template <typename G>
+__global__ void __launch_bounds__(256) widen_kernel(const G* __restrict__ src, float* __restrict__ dst, size_t n) {
+    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x)
+        dst[i] = to_f32(__ldg(src + i));
+}
+
 // Sizes of one call; false when the call is outside the contract (adaptive grid, entry or pixel count too large).
 struct DetPlan {
     long long entries;      // K * bins * sr^2 * 4
@@ -1671,11 +1759,14 @@ static bool det_plan(const rsdet_roi_align_cfg* c, int num_rois, DetPlan* p) {
     return true;
 }
 
-static size_t det_workspace_bytes(const rsdet_roi_align_cfg* c, int num_rois, const DetPlan& p) {
+static size_t det_workspace_bytes(const rsdet_roi_align_cfg* c, int num_rois, const DetPlan& p, bool f32) {
     const size_t E = (size_t)(p.entries > 0 ? p.entries : 1);
     size_t b = 4 * ws_bytes<uint32_t>(E) + ws_bytes<float>(E);        // keys x2, entry indices x2, weights
-    b += ws_bytes<float>((size_t)(num_rois > 0 ? num_rois : 1) * c->pooled_h * c->pooled_w * c->channels);   // bin-major grad_out
-    if (!c->channels_last)                                             // fp32 NHWC accumulators
+    // the fp32 bin-major copy of grad_out.  An NHWC fp32 grad_out is that array already; the query does not know the
+    // grad_out dtype, so it reserves the copy unless the maps -- and hence grad_out -- are fp32.
+    if (!nhwc_rois(c) || !f32)
+        b += ws_bytes<float>((size_t)(num_rois > 0 ? num_rois : 1) * c->pooled_h * c->pooled_w * c->channels);
+    if (!nhwc_maps(c))                                                 // fp32 NHWC accumulators
         for (int l = 0; l < c->num_levels; l++) b += ws_bytes<float>((size_t)c->batch * c->channels * c->height[l] * c->width[l]);
     return b + align256(p.cub_bytes) + 256;
 }
@@ -1689,7 +1780,7 @@ static int backward_det_impl(const rsdet_roi_align_cfg* cfg, const DetPlan& plan
         count_launch(cfg->num_levels);
         return cuda_status();
     }
-    if (workspace_bytes < det_workspace_bytes(cfg, num_rois, plan)) return RSDET_EWORKSPACE;
+    if (workspace_bytes < det_workspace_bytes(cfg, num_rois, plan, kIsF32<T>)) return RSDET_EWORKSPACE;
     const int E = (int)plan.entries, nbins = cfg->pooled_h * cfg->pooled_w;
     Workspace ws(workspace, workspace_bytes);
     uint32_t* keyA = ws.take<uint32_t>(E);
@@ -1697,9 +1788,13 @@ static int backward_det_impl(const rsdet_roi_align_cfg* cfg, const DetPlan& plan
     int* idxA = ws.take<int>(E);
     int* idxB = ws.take<int>(E);
     float* wts = ws.take<float>(E);
-    float* top = ws.take<float>((size_t)num_rois * nbins * cfg->channels);
+    // an fp32 (K, PH, PW, C) grad_out already is the bin-major array the gather reads
+    const float* top = nullptr;
+    float* top_ws = nullptr;
+    if constexpr (kIsF32<G>) { if (nhwc_rois(cfg)) top = grad_out; }
+    if (!top) top = top_ws = ws.take<float>((size_t)num_rois * nbins * cfg->channels);
     float* acc[RSDET_MAX_LEVELS];
-    if (!cfg->channels_last)
+    if (!nhwc_maps(cfg))
         for (int l = 0; l < cfg->num_levels; l++) acc[l] = ws.take<float>((size_t)cfg->batch * cfg->channels * cfg->height[l] * cfg->width[l]);
     void* cub_tmp = ws.take<char>(plan.cub_bytes);
     if (!ws.ok()) return RSDET_EWORKSPACE;
@@ -1715,11 +1810,11 @@ static int backward_det_impl(const rsdet_roi_align_cfg* cfg, const DetPlan& plan
     for (int l = 0; l <= RSDET_MAX_LEVELS; l++) {
         J.pix_base[l] = base;
         if (l < cfg->num_levels) base += (unsigned)((size_t)cfg->batch * cfg->height[l] * cfg->width[l]);
-        if (l < RSDET_MAX_LEVELS) J.out[l] = l < cfg->num_levels ? (cfg->channels_last ? (void*)grad_feats_host[l] : (void*)acc[l]) : nullptr;
+        if (l < RSDET_MAX_LEVELS) J.out[l] = l < cfg->num_levels ? (nhwc_maps(cfg) ? (void*)grad_feats_host[l] : (void*)acc[l]) : nullptr;
     }
     // zero fill of whatever the gather writes into; an NCHW caller's maps are written whole by the transpose
     for (int l = 0; l < cfg->num_levels; l++) {
-        if (cfg->channels_last) cudaMemsetAsync(grad_feats_host[l], 0, map_bytes(l), st);
+        if (nhwc_maps(cfg)) cudaMemsetAsync(grad_feats_host[l], 0, map_bytes(l), st);
         else cudaMemsetAsync(acc[l], 0, sizeof(float) * (size_t)cfg->batch * cfg->channels * cfg->height[l] * cfg->width[l], st);
     }
     count_launch(cfg->num_levels);
@@ -1727,14 +1822,23 @@ static int backward_det_impl(const rsdet_roi_align_cfg* cfg, const DetPlan& plan
     roi_bwd_det_entries_kernel<<<(unsigned)(ceil_div_ll(samples, 256) < kNumSMs * 16 ? ceil_div_ll(samples, 256) : kNumSMs * 16),
                                  256, 0, st>>>(J, rois, num_rois, keyA, idxA, wts);
     count_launch();
-    // bin-major copy of grad_out: the NCHW -> NHWC transpose with K images of PH x PW pixels
-    TransposeJob tj;
-    tj.num_levels = 1; tj.N = num_rois; tj.C = cfg->channels;
-    tj.src[0] = grad_out; tj.dst[0] = top; tj.HW[0] = nbins;
-    tj.tile_begin[0] = 0;
-    tj.tile_begin[1] = num_rois * ceil_div(nbins, 64) * ceil_div(cfg->channels, 64);
-    transpose_kernel<G, float, true><<<tj.tile_begin[1], 256, 0, st>>>(tj);
-    count_launch();
+    if (nhwc_rois(cfg) && top_ws) {
+        if constexpr (!kIsF32<G>) {   // half (K, PH, PW, C) grad_out: already bin-major, widened exactly to fp32
+            const size_t n = (size_t)num_rois * nbins * cfg->channels;
+            const long long blocks = ceil_div_ll((long long)n, 256);
+            widen_kernel<G><<<(unsigned)(blocks < kNumSMs * 16 ? blocks : kNumSMs * 16), 256, 0, st>>>(grad_out, top_ws, n);
+            count_launch();
+        }
+    } else if (!nhwc_rois(cfg)) {
+        // bin-major copy of grad_out: the NCHW -> NHWC transpose with K images of PH x PW pixels
+        TransposeJob tj;
+        tj.num_levels = 1; tj.N = num_rois; tj.C = cfg->channels;
+        tj.src[0] = grad_out; tj.dst[0] = top_ws; tj.HW[0] = nbins;
+        tj.tile_begin[0] = 0;
+        tj.tile_begin[1] = num_rois * ceil_div(nbins, 64) * ceil_div(cfg->channels, 64);
+        transpose_kernel<G, float, true><<<tj.tile_begin[1], 256, 0, st>>>(tj);
+        count_launch();
+    }
     bool in_b = false;
     rc = sort_pairs_u32(cub_tmp, &need, keyA, keyB, idxA, idxB, E, plan.key_bits, &in_b, st);
     if (rc != RSDET_OK) return rc;
@@ -1745,12 +1849,12 @@ static int backward_det_impl(const rsdet_roi_align_cfg* cfg, const DetPlan& plan
     const unsigned blocks = (unsigned)(ceil_div_ll(chunks, 8) < kNumSMs * 8 ? ceil_div_ll(chunks, 8) : kNumSMs * 8);
     const int spb = cfg->sampling_ratio * cfg->sampling_ratio;
     const bool pow2 = (spb & (spb - 1)) == 0;
-    if (cfg->channels_last && pow2) roi_bwd_det_gather_kernel<T, true><<<blocks, 256, 0, st>>>(J, keys, idx, wts, top, E);
-    else if (cfg->channels_last) roi_bwd_det_gather_kernel<T, false><<<blocks, 256, 0, st>>>(J, keys, idx, wts, top, E);
+    if (nhwc_maps(cfg) && pow2) roi_bwd_det_gather_kernel<T, true><<<blocks, 256, 0, st>>>(J, keys, idx, wts, top, E);
+    else if (nhwc_maps(cfg)) roi_bwd_det_gather_kernel<T, false><<<blocks, 256, 0, st>>>(J, keys, idx, wts, top, E);
     else if (pow2) roi_bwd_det_gather_kernel<float, true><<<blocks, 256, 0, st>>>(J, keys, idx, wts, top, E);
     else roi_bwd_det_gather_kernel<float, false><<<blocks, 256, 0, st>>>(J, keys, idx, wts, top, E);
     count_launch();
-    if (!cfg->channels_last) {
+    if (!nhwc_maps(cfg)) {
         rc = launch_transpose(false, acc, grad_feats_host, cfg->height, cfg->width, cfg->num_levels, cfg->batch,
                                         cfg->channels, st);
         if (rc != RSDET_OK) return rc;
@@ -1764,7 +1868,7 @@ extern "C" size_t rsdet_roi_align_rotated_backward_deterministic_workspace_bytes
                                                                                  int feat_dtype) {
     DetPlan plan;
     if (!dtype_ok(feat_dtype) || check_cfg(cfg) != RSDET_OK || !det_plan(cfg, num_rois, &plan)) return 0;
-    return det_workspace_bytes(cfg, num_rois, plan);
+    return det_workspace_bytes(cfg, num_rois, plan, feat_dtype == RSDET_DTYPE_F32);
 }
 
 extern "C" int rsdet_roi_align_rotated_backward_deterministic(const rsdet_roi_align_cfg* cfg, int grad_out_dtype,

@@ -10,7 +10,7 @@ from torch import nn
 
 from .... import core
 from ...ops import roi_align_rotated_v1
-from ...ops.roi_align_rotated_v1 import _deterministic_backward, _grad_dtype
+from ...ops.roi_align_rotated_v1 import _deterministic_backward, _grad_dtype, _maps_format
 
 
 def _pair(x):
@@ -19,25 +19,26 @@ def _pair(x):
 
 class _FusedExtractFn(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, rois, cfg, *feats):
+    def forward(ctx, rois, cfg, memory_format, *feats):
         ctx.cfg = cfg
         ctx.shapes = [tuple(f.shape) for f in feats]
         ctx.dtype = _grad_dtype(feats[0].dtype)      # core rejects levels that mix fp16 / bf16 with another dtype
+        ctx.maps_format = _maps_format(feats)
         ctx.save_for_backward(rois)
-        return core.roi_align_rotated_forward(cfg, feats, rois)
+        return core.roi_align_rotated_forward(cfg, feats, rois, memory_format=memory_format)
 
     @staticmethod
     def backward(ctx, grad_output):
         (rois,) = ctx.saved_tensors
         det = _deterministic_backward(ctx.cfg, "RoI extractor (RoIAlignRotated)")
-        grads = core.roi_align_rotated_backward(ctx.cfg, grad_output.contiguous(), rois, ctx.shapes, feat_dtype=ctx.dtype,
-                                                deterministic=det)
-        return (None, None, *grads)
+        grads = core.roi_align_rotated_backward(ctx.cfg, grad_output, rois, ctx.shapes, feat_dtype=ctx.dtype,
+                                                deterministic=det, memory_format=ctx.maps_format)
+        return (None, None, None, *grads)
 
 
 class OrientedSingleRoIExtractor(nn.Module):
     """Extract RoI features from a single level feature map (each RoI is mapped to one FPN level by its
-    extended scale).  Args as in the reference (:22-34)."""
+    extended scale).  Args as in the reference (:22-34).  The output layout is the roi layer's `memory_format`."""
 
     def __init__(self, roi_layer, out_channels, featmap_strides, extend_factor=(1., 1.), finest_scale=56):
         super(OrientedSingleRoIExtractor, self).__init__()
@@ -92,6 +93,6 @@ class OrientedSingleRoIExtractor(nn.Module):
         cfg = core.make_roi_cfg([tuple(f.shape) for f in feats], [l.spatial_scale for l in self.roi_layers[:len(feats)]],
                                 layer.output_size, int(layer.sampling_ratio), version=1, extend=(eh, ew),
                                 finest_scale=float(self.finest_scale))
-        return _FusedExtractFn.apply(rois, cfg, *feats)
+        return _FusedExtractFn.apply(rois, cfg, layer.memory_format, *feats)
 
     execute = forward

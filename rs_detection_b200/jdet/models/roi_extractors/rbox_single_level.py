@@ -49,6 +49,6 @@ class RboxSingleRoIExtractor(nn.Module):
         cfg = core.make_roi_cfg([tuple(f.shape) for f in feats], [l.spatial_scale for l in self.roi_layers[:len(feats)]],
                                 layer.output_size, int(layer.sampling_ratio), version=0, extend=(1.0, 1.0),
                                 finest_scale=float(self.finest_scale))
-        return _FusedExtractFn.apply(rois, cfg, *feats)
+        return _FusedExtractFn.apply(rois, cfg, layer.memory_format, *feats)
 
     execute = forward
