@@ -85,16 +85,20 @@ int rsdet_assign_wrt_overlaps(const float* overlaps, int num_gts, int n, float p
  *   dets    : (n, row_floats(kind)) of fp32 or fp64 as the kind says
  *   scores  : (n) fp32, or fp64 for MERGE/HBB/HBB_P1_F64
  *   labels  : (n) int32 group ids (any values) or NULL
- *   thr     : scalar threshold, used when thr_per_label == NULL
- *   thr_per_label : optional device array indexed by label value (0 <= label < num_thr)
- *                   (result_merge.py:26-27 per-class thresholds)
+ *   thr     : scalar threshold, used when thr_per_label == NULL and for every label outside [0, num_thr)
+ *   thr_per_label : optional device array indexed by label value (result_merge.py:26-27 per-class thresholds);
+ *                   labels outside [0, num_thr) fall back to `thr`.  Ignored when labels == NULL.
+ * Every threshold is exact, including those at which a pair of IoU 0 suppresses (thr < 0; thr <= 0 for ROTATED_GE and
+ * HBB): such a label group keeps only its top box (and boxes whose IoU with it is NaN), as in the reference.  Those
+ * groups evaluate every pair instead of filtering out the disjoint ones, and the call does not take the sparse path.
  * Outputs (any may be NULL):
  *   keep_mask     uint8 (n), 1 = kept, ORIGINAL index space  (the `keep` bool Var of nms_rotated_cuda)
  *   keep_sorted_idx int64 (n): kept ORIGINAL indices in ascending index order  (jt.where(keep)[0])
  *   keep_score_idx  int64 (n): kept ORIGINAL indices in descending score order (order_t[keep], poly_nms;
  *                              py_cpu_nms_poly_fast's python list)
  *   num_keep      int32 (1) device counter
- * Score ties are broken by lower original index first (the reference leaves this unspecified).
+ * Score ties are broken by lower original index first for the fp32 kinds, higher index first for MERGE, HBB and
+ * HBB_P1_F64 (`argsort(kind='stable')[::-1]`); -0.0 and +0.0 tie.
  * Limit: n <= 2^18 boxes per call (RSDET_ELIMIT above; the workspace query then returns 0). */
 size_t rsdet_nms_workspace_bytes(int kind, int n);
 int rsdet_nms(int kind, const void* dets, const void* scores, const int32_t* labels, int n, double thr,
@@ -108,7 +112,9 @@ int rsdet_nms(int kind, const void* dets, const void* scores, const int32_t* lab
  *   multi_bboxes : (n,5) or (n,5*(num_classes+1)) as bbox_dim says;  multi_scores : (n,num_classes+1)
  *   score_factors: (n) or NULL
  *   out_dets (cap,6) [cx,cy,w,h,theta,score], out_labels int32 (cap), out_count int32 (1);
- *   cap = n*num_classes rows must be available; n*num_classes <= 2^20 (RSDET_ELIMIT above). */
+ *   cap = n*num_classes rows must be available; n*num_classes <= 2^20 (RSDET_ELIMIT above).
+ *   iou_thr < 0 returns RSDET_EINVAL: at such thresholds disjoint pairs suppress, and the decision matrix only
+ *   evaluates overlapping ones. */
 size_t rsdet_multiclass_nms_rotated_workspace_bytes(int n, int num_classes);
 int rsdet_multiclass_nms_rotated(const float* multi_bboxes, int bbox_dim, const float* multi_scores, int n,
                                  int num_classes, float score_thr, float iou_thr, int max_num,

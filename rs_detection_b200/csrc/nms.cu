@@ -48,6 +48,10 @@ constexpr int kFastSegs = 2048;  // segment starts collected with atomics + one 
 // ----------------------------------------------------------------------------- predicates
 struct HBox { double x1, y1, x2, y2; };
 
+// suppress() is the reference's predicate for any pair.  cheap() and refine*() drop only pairs of IoU 0 (or pairs the
+// bounds prove below thr), which is exact as long as the kind's rule keeps an IoU of 0 at that threshold;
+// zero_suppressed(thr) says when it does not (thr < 0 for most kinds, thr <= 0 for ROTATED_GE and HBB): then every pair
+// goes to suppress() (mask_tiles_kernel<KIND, true>) and the sparse path is not used.
 template <int KIND> struct Traits;
 
 template <> struct Traits<RSDET_NMS_ROTATED> {
@@ -63,11 +67,13 @@ template <> struct Traits<RSDET_NMS_ROTATED> {
     __device__ static bool suppress(const Box& a, const Box& b, Thr thr, float2* q) {
         return rotated_iou_pair<kNmsThreads>(a, b, q) > thr;
     }
+    __host__ __device__ static bool zero_suppressed(Thr thr) { return 0.f > thr; }
 };
 template <> struct Traits<RSDET_NMS_ROTATED_GE> : Traits<RSDET_NMS_ROTATED> {
     __device__ static bool suppress(const Box& a, const Box& b, Thr thr, float2* q) {
         return rotated_iou_pair<kNmsThreads>(a, b, q) >= thr;
     }
+    __host__ __device__ static bool zero_suppressed(Thr thr) { return 0.f >= thr; }
 };
 template <> struct Traits<RSDET_NMS_POLY> {
     using Box = PolyBox; using Raw = float; using Thr = float;
@@ -81,6 +87,7 @@ template <> struct Traits<RSDET_NMS_POLY> {
     __device__ static bool suppress(const Box& a, const Box& b, Thr thr, float2* q) {
         return poly_iou_f32<kNmsThreads>(a, b, q) > thr;
     }
+    __host__ __device__ static bool zero_suppressed(Thr thr) { return 0.f > thr; }
 };
 template <> struct Traits<RSDET_NMS_MERGE> {
     using Box = MBox; using Raw = double; using Thr = double;
@@ -100,8 +107,11 @@ template <> struct Traits<RSDET_NMS_MERGE> {
     __device__ static bool cheap(const Box& a, const Box& b) { return merge_hbb_overlap(a, b); }
     __device__ static bool refine1(const Box&, const Box&, Thr) { return true; }
     __device__ static bool refine2(const Box&, const Box&, Thr) { return true; }
-    // survivors are `iou <= thr` (result_merge.py:118)
+    // survivors are `iou <= thr` (result_merge.py:118).  The reference gives pairs whose hbbs do not overlap ovr = 0
+    // (result_merge.py:97-100); the clipper gives them some IoU >= 0 instead.  Such pairs reach this test only when
+    // zero_suppressed(thr) (thr < 0 or NaN), and there every IoU >= 0 suppresses as 0 does
     __device__ static bool suppress(const Box& a, const Box& b, Thr thr, float2*) { return !(iou_poly_d(a, b) <= thr); }
+    __host__ __device__ static bool zero_suppressed(Thr thr) { return !(0.0 <= thr); }
 };
 template <> struct Traits<RSDET_NMS_HBB> {
     using Box = HBox; using Raw = double; using Thr = double;
@@ -123,6 +133,7 @@ template <> struct Traits<RSDET_NMS_HBB> {
         double iou = ov / ((a.x2 - a.x1) * (a.y2 - a.y1) + (b.x2 - b.x1) * (b.y2 - b.y1) - ov);
         return !(iou < thr);
     }
+    __host__ __device__ static bool zero_suppressed(Thr thr) { return !(0.0 < thr); }
 };
 
 // py_cpu_nms (data/devkits/result_merge.py:143-174, used by mergebyrec): float64, "+1" widths, survivors ovr <= thresh
@@ -131,8 +142,11 @@ template <> struct Traits<RSDET_NMS_HBB_P1_F64> {
     static constexpr int kRow = 4; static constexpr bool kScratch = false;
     static constexpr bool kRefine = false;
     __device__ static Box prep(const Raw* r) { Box b; b.x1 = r[0]; b.y1 = r[1]; b.x2 = r[2]; b.y2 = r[3]; return b; }
+    // pairs without a "+1" overlap have ovr = 0 / (A + B): kept for thresh >= 0 -- EXCEPT when the "+1" areas sum to
+    // zero (0/0 = NaN, and `NaN <= thresh` is false: suppressed), so those pairs pass the filter
     __device__ static bool cheap(const Box& a, const Box& b) {
-        return fmin(a.x2, b.x2) - fmax(a.x1, b.x1) + 1.0 > 0.0 && fmin(a.y2, b.y2) - fmax(a.y1, b.y1) + 1.0 > 0.0;
+        return (fmin(a.x2, b.x2) - fmax(a.x1, b.x1) + 1.0 > 0.0 && fmin(a.y2, b.y2) - fmax(a.y1, b.y1) + 1.0 > 0.0) ||
+               (a.x2 - a.x1 + 1.0) * (a.y2 - a.y1 + 1.0) + (b.x2 - b.x1 + 1.0) * (b.y2 - b.y1 + 1.0) == 0.0;
     }
     __device__ static bool refine1(const Box&, const Box&, Thr) { return true; }
     __device__ static bool refine2(const Box&, const Box&, Thr) { return true; }
@@ -142,6 +156,7 @@ template <> struct Traits<RSDET_NMS_HBB_P1_F64> {
         double ovr = inter / ((a.x2 - a.x1 + 1.0) * (a.y2 - a.y1 + 1.0) + (b.x2 - b.x1 + 1.0) * (b.y2 - b.y1 + 1.0) - inter);
         return !(ovr <= thr);
     }
+    __host__ __device__ static bool zero_suppressed(Thr thr) { return !(0.0 <= thr); }
 };
 
 // jt.nms (Jittor 1.3.4.7 misc.py `nms`, called from oriented_rpn_head.py:208): fp32 boxes, the "+1" pixel
@@ -164,6 +179,7 @@ template <> struct Traits<RSDET_NMS_HBB_P1> {
         float sa = (a.x2 - a.x1 + 1.f) * (a.y2 - a.y1 + 1.f), sb = (b.x2 - b.x1 + 1.f) * (b.y2 - b.y1 + 1.f);
         return (double)(inter / (sa + sb - inter)) > thr;
     }
+    __host__ __device__ static bool zero_suppressed(Thr thr) { return 0.0 > thr; }
 };
 
 // ----------------------------------------------------------------------------- segment table
@@ -413,7 +429,9 @@ __device__ __forceinline__ int compact_queue(const unsigned short* __restrict__ 
     return *s_counter;
 }
 
-template <int KIND>
+// ZERO_CHECK: a segment whose threshold suppresses an IoU of 0 skips the filters (every pair goes to suppress()).
+// Instantiated only for calls that may have such a segment, so the filtered kernel stays as it is.
+template <int KIND, bool ZERO_CHECK>
 __global__ void __launch_bounds__(kNmsThreads)
 mask_tiles_kernel(const typename Traits<KIND>::Box* __restrict__ boxes, SegTable tb, unsigned long long* __restrict__ mask,
                   const int* __restrict__ gate) {
@@ -463,6 +481,7 @@ mask_tiles_kernel(const typename Traits<KIND>::Box* __restrict__ boxes, SegTable
         const int cb = rb + (int)(u - ((long long)rb * T - (long long)rb * (rb - 1) / 2));
         const int nr = min(64, ns - rb * 64), nc = min(64, ns - cb * 64);
         const typename Tr::Thr thr = (typename Tr::Thr)tb.seg_thr[s];
+        const bool all_pairs = ZERO_CHECK && Tr::zero_suppressed(thr);
 
         if (tid < 64) {
             if (tid < nr) s_row[tid] = boxes[st + rb * 64 + tid];
@@ -484,7 +503,7 @@ mask_tiles_kernel(const typename Traits<KIND>::Box* __restrict__ boxes, SegTable
 #pragma unroll 4
                 for (int k = 0; k < 32; k++) {
                     const int r = 2 * k + rhalf;
-                    const bool cand = r < nr && (!diag || c > r) && Tr::cheap(s_row[r], colbox);
+                    const bool cand = r < nr && (!diag || c > r) && (all_pairs || Tr::cheap(s_row[r], colbox));
                     hits |= (cand ? 1u : 0u) << k;
                 }
             }
@@ -508,7 +527,7 @@ mask_tiles_kernel(const typename Traits<KIND>::Box* __restrict__ boxes, SegTable
         }
         __syncthreads();
         const int cnt = s_count;
-        if (Tr::kRefine) {
+        if (Tr::kRefine && !all_pairs) {
             for (int q0 = 0; q0 < cnt; q0 += kQ2) {
                 const int n2 = compact_queue(s_queue + q0, min(kQ2, cnt - q0), s_queue2, &s_count2, s_wsum,
                                              [&](int p) { return Tr::refine1(s_row[p >> 6], s_col[p & 63], thr); });
@@ -1507,6 +1526,9 @@ __global__ void sp_keys_kernel(const typename SpAdapt<KIND>::Box* __restrict__ b
         if (tb.seg_start[mid] <= p) lo = mid; else hi = mid;
     }
     w.seg_of[p] = lo;
+    // the sweep only finds overlapping pairs: a segment whose threshold suppresses an IoU of 0 hands the call to the dense
+    // kernels (per-label thresholds; a scalar one that does never takes this path)
+    if (Traits<KIND>::zero_suppressed((typename Traits<KIND>::Thr)tb.seg_thr[lo])) w.ctl[0] = 1;
     // (group | y band | x1 rounded DOWN: never right of the true x1)
     w.keyA[p] = ((unsigned long long)lo << (32 + kBandBits)) | ((unsigned long long)sp_band(A::y1(boxes[p]), sp_band_h(w)) << 32) |
                 ord_f32(__double2float_rd(A::x1(boxes[p])));
@@ -1559,7 +1581,7 @@ __global__ void sp_sweep_kernel(const typename SpAdapt<KIND>::Box* __restrict__ 
     using Box = typename A::Box;
     const int q = blockIdx.x * blockDim.x + threadIdx.x;
     const int n_eff = min(tb.hdr[1], n_max);
-    if (q >= n_eff) return;
+    if (q >= n_eff || w.ctl[0]) return;   // gate already open (sp_keys_kernel): the dense kernels take the call
     if ((unsigned long long)(unsigned int)w.ctl[7] * 64ull > (unsigned long long)kSparseMaxVisits * (unsigned long long)n_eff + 4096ull) {
         if (q == 0) w.ctl[0] = 1;   // a crowd: the dense kernels take the call
         return;
@@ -1721,8 +1743,25 @@ size_t nms_ws_bytes(int kind, int n, size_t mask_words) {
 }
 
 template <int KIND>
+static bool zero_suppressed_kind(double thr) { return Traits<KIND>::zero_suppressed((typename Traits<KIND>::Thr)thr); }
+
+// whether the kind's rule suppresses a pair of IoU 0 at this threshold (host side of Traits<KIND>::zero_suppressed)
+static bool zero_suppressed(int kind, double thr) {
+    switch (kind) {
+        case RSDET_NMS_ROTATED: return zero_suppressed_kind<RSDET_NMS_ROTATED>(thr);
+        case RSDET_NMS_ROTATED_GE: return zero_suppressed_kind<RSDET_NMS_ROTATED_GE>(thr);
+        case RSDET_NMS_POLY: return zero_suppressed_kind<RSDET_NMS_POLY>(thr);
+        case RSDET_NMS_MERGE: return zero_suppressed_kind<RSDET_NMS_MERGE>(thr);
+        case RSDET_NMS_HBB_P1: return zero_suppressed_kind<RSDET_NMS_HBB_P1>(thr);
+        case RSDET_NMS_HBB_P1_F64: return zero_suppressed_kind<RSDET_NMS_HBB_P1_F64>(thr);
+        default: return zero_suppressed_kind<RSDET_NMS_HBB>(thr);
+    }
+}
+
+template <int KIND>
 static void launch_kind(const NmsArgs& a, const int* idx, void* boxes, int32_t* label_sorted, SegTable tb,
-                        unsigned long long* mask, cudaStream_t st, bool mask_phase, int* starts_unsorted, const int* gate = nullptr) {
+                        unsigned long long* mask, cudaStream_t st, bool mask_phase, int* starts_unsorted, const int* gate = nullptr,
+                        bool zero_check = false) {
     using Tr = Traits<KIND>;
     if (!mask_phase) {
         prep_sorted_kernel<KIND><<<ceil_div(a.n_max, 256), 256, 0, st>>>((const typename Tr::Raw*)a.dets, a.labels, idx, a.n_max,
@@ -1732,21 +1771,23 @@ static void launch_kind(const NmsArgs& a, const int* idx, void* boxes, int32_t* 
         long long T = (a.n_max + 63) / 64;
         long long tiles = T * (T + 1) / 2;
         int grid = (int)(tiles < (long long)kNumSMs * 5 ? tiles : (long long)kNumSMs * 5);  // 5 CTAs/SM fit (39 KB smem, 91 regs)
-        mask_tiles_kernel<KIND><<<grid, kNmsThreads, 0, st>>>((const typename Tr::Box*)boxes, tb, mask, gate);
+        if (zero_check) mask_tiles_kernel<KIND, true><<<grid, kNmsThreads, 0, st>>>((const typename Tr::Box*)boxes, tb, mask, gate);
+        else mask_tiles_kernel<KIND, false><<<grid, kNmsThreads, 0, st>>>((const typename Tr::Box*)boxes, tb, mask, gate);
     }
     count_launch();
 }
 
 static void dispatch_kind(const NmsArgs& a, const int* idx, void* boxes, int32_t* label_sorted, SegTable tb,
-                          unsigned long long* mask, cudaStream_t st, bool mask_phase, int* starts_unsorted, const int* gate = nullptr) {
+                          unsigned long long* mask, cudaStream_t st, bool mask_phase, int* starts_unsorted, const int* gate = nullptr,
+                          bool zero_check = false) {
     switch (a.kind) {
-        case RSDET_NMS_ROTATED: launch_kind<RSDET_NMS_ROTATED>(a, idx, boxes, label_sorted, tb, mask, st, mask_phase, starts_unsorted, gate); break;
-        case RSDET_NMS_ROTATED_GE: launch_kind<RSDET_NMS_ROTATED_GE>(a, idx, boxes, label_sorted, tb, mask, st, mask_phase, starts_unsorted, gate); break;
-        case RSDET_NMS_POLY: launch_kind<RSDET_NMS_POLY>(a, idx, boxes, label_sorted, tb, mask, st, mask_phase, starts_unsorted, gate); break;
-        case RSDET_NMS_MERGE: launch_kind<RSDET_NMS_MERGE>(a, idx, boxes, label_sorted, tb, mask, st, mask_phase, starts_unsorted, gate); break;
-        case RSDET_NMS_HBB_P1: launch_kind<RSDET_NMS_HBB_P1>(a, idx, boxes, label_sorted, tb, mask, st, mask_phase, starts_unsorted, gate); break;
-        case RSDET_NMS_HBB_P1_F64: launch_kind<RSDET_NMS_HBB_P1_F64>(a, idx, boxes, label_sorted, tb, mask, st, mask_phase, starts_unsorted, gate); break;
-        default: launch_kind<RSDET_NMS_HBB>(a, idx, boxes, label_sorted, tb, mask, st, mask_phase, starts_unsorted, gate); break;
+        case RSDET_NMS_ROTATED: launch_kind<RSDET_NMS_ROTATED>(a, idx, boxes, label_sorted, tb, mask, st, mask_phase, starts_unsorted, gate, zero_check); break;
+        case RSDET_NMS_ROTATED_GE: launch_kind<RSDET_NMS_ROTATED_GE>(a, idx, boxes, label_sorted, tb, mask, st, mask_phase, starts_unsorted, gate, zero_check); break;
+        case RSDET_NMS_POLY: launch_kind<RSDET_NMS_POLY>(a, idx, boxes, label_sorted, tb, mask, st, mask_phase, starts_unsorted, gate, zero_check); break;
+        case RSDET_NMS_MERGE: launch_kind<RSDET_NMS_MERGE>(a, idx, boxes, label_sorted, tb, mask, st, mask_phase, starts_unsorted, gate, zero_check); break;
+        case RSDET_NMS_HBB_P1: launch_kind<RSDET_NMS_HBB_P1>(a, idx, boxes, label_sorted, tb, mask, st, mask_phase, starts_unsorted, gate, zero_check); break;
+        case RSDET_NMS_HBB_P1_F64: launch_kind<RSDET_NMS_HBB_P1_F64>(a, idx, boxes, label_sorted, tb, mask, st, mask_phase, starts_unsorted, gate, zero_check); break;
+        default: launch_kind<RSDET_NMS_HBB>(a, idx, boxes, label_sorted, tb, mask, st, mask_phase, starts_unsorted, gate, zero_check); break;
     }
 }
 
@@ -1942,7 +1983,10 @@ int nms_run(const NmsArgs& a, void* workspace, size_t workspace_bytes, cudaStrea
     const int* gate = nullptr;
     const size_t mask_cap = a.mask_words ? a.mask_words : N * ((N + 63) / 64);
     const bool sparse_kind = a.kind == RSDET_NMS_MERGE || ((a.kind == RSDET_NMS_ROTATED || a.kind == RSDET_NMS_ROTATED_GE) && !a.labels);
-    if (sparse_kind && n >= (a.kind == RSDET_NMS_MERGE ? kSparseMinBoxes : kSparseMinRotated)) {
+    // per-label thresholds are read on the device: every segment checks its own (mask_tiles_kernel, sp_keys_kernel)
+    const bool per_label_thr = a.thr_per_label && a.labels;
+    const bool zero_all = !per_label_thr && zero_suppressed(a.kind, a.thr);
+    if (sparse_kind && !zero_all && n >= (a.kind == RSDET_NMS_MERGE ? kSparseMinBoxes : kSparseMinRotated)) {
         Workspace mw(mask, mask_cap * sizeof(unsigned long long));
         SparseWs w;
         w.keyA = mw.take<unsigned long long>(N);
@@ -2003,7 +2047,7 @@ int nms_run(const NmsArgs& a, void* workspace, size_t workspace_bytes, cudaStrea
         }
     }
     // 4. suppression mask over the upper-triangular tiles of every segment
-    dispatch_kind(a, idx_ls, boxes, label_sorted, tb, mask, st, true, starts_unsorted, gate);
+    dispatch_kind(a, idx_ls, boxes, label_sorted, tb, mask, st, true, starts_unsorted, gate, per_label_thr || zero_all);
     // 5. greedy scan
     {
         size_t smem = sizeof(unsigned long long) * ((N + 63) / 64);
@@ -2483,6 +2527,9 @@ extern "C" int rsdet_multiclass_nms_rotated(const float* multi_bboxes, int bbox_
                                             int32_t* out_count, void* workspace, size_t workspace_bytes, void* stream) {
     if (n < 0 || num_classes <= 0 || !out_count) return RSDET_EINVAL;
     if (bbox_dim != 5 && bbox_dim != 5 * (num_classes + 1)) return RSDET_EINVAL;
+    // below 0 every pair of a class suppresses, disjoint ones included; the decision matrix filters keep only
+    // overlapping pairs, so such thresholds are refused rather than answered wrongly
+    if (iou_thr < 0.f) return RSDET_EINVAL;
     cudaStream_t st = (cudaStream_t)stream;
     if (n == 0) {
         cudaMemsetAsync(out_count, 0, sizeof(int32_t), st);

@@ -41,13 +41,15 @@ def py_cpu_nms_poly_fast(dets, thresh):
 
 def py_cpu_nms_poly(dets, thresh):
     """:30-63 -- the same predicate as the `_fast` variant without the hbb prefilter (pairs whose hbbs do not
-    overlap have IoU 0, which no non-negative threshold suppresses): one engine, same result."""
+    overlap have IoU 0, which both variants suppress exactly when thresh < 0): one engine, same result."""
     return py_cpu_nms_poly_fast(dets, thresh)
 
 
 def py_cpu_nms(dets, thresh):
     """:143-174 -- horizontal boxes (n,5) float64 [x1,y1,x2,y2,score], '+1' areas, survivors `ovr <= thresh`;
-    returns the kept indices in descending-score order (python list)."""
+    returns the kept indices in descending-score order (python list).  A pair without a '+1' overlap whose '+1' areas
+    sum to 0 has ovr = 0/0 = NaN and is suppressed, as in the reference; any other such pair has ovr = 0, suppressed
+    only when thresh < 0."""
     require_cuda()
     d = np.ascontiguousarray(dets, dtype=np.float64).reshape(-1, 5)
     if d.shape[0] == 0:
