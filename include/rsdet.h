@@ -66,6 +66,40 @@ int rsdet_assign_wrt_overlaps(const float* overlaps, int num_gts, int n, float p
                               int32_t labels_fill, int32_t* assigned_gt_inds, float* max_overlaps,
                               int32_t* assigned_labels, void* workspace, size_t workspace_bytes, void* stream);
 
+/* ---------------------------------------------------------------- horizontal IoU / RPN anchor assignment
+ * BboxOverlaps2D (mode='iou', not aligned): the mmdet 2.x bbox_overlaps that JDet's models/boxes/iou_calculator.py
+ * copies, the default calculator of the oriented RPN's MaxIoUAssigner.  Boxes are [x1, y1, x2, y2], fp32, no "+1":
+ *     area = (x2 - x1) * (y2 - y1);  w = max(min(x2a, x2b) - max(x1a, x1b), 0);  h likewise on y
+ *     iou = (w * h) / max((area_a + area_b) - w * h, 1e-6)
+ * each operation rounded on its own.  This formula is restated, not pinned by a reference fixture (DESIGN.md §3).
+ * The sign of a zero IoU is not part of the contract (the library writes +0.0).  Coordinates must be finite.
+ * boxes1 (n1,4), boxes2 (n2,4) -> ious (n1,n2).  n1 * n2 <= 2^40 (RSDET_ELIMIT above). */
+int rsdet_bbox_overlaps(const float* boxes1, int n1, const float* boxes2, int n2, float* ious, void* stream);
+
+/* MaxIoU assignment of n anchors to num_gts horizontal GTs without the (num_gts, n) overlaps matrix: the result is bit for
+ * bit rsdet_assign_wrt_overlaps(rsdet_bbox_overlaps(gt_hbb, anchors), ...) with the same arguments -- assigned_gt_inds,
+ * max_overlaps and assigned_labels, with its tie rules (first maximal GT per anchor, first maximal anchor per GT, the
+ * last low-quality match wins).  The pairs are recomputed instead of stored, so memory does not grow with num_gts * n.
+ *   gt_hbb (num_gts,4), anchors (n,4) [x1, y1, x2, y2] fp32.
+ *   valid: optional uint8 (n) mask (the RPN's anchor_inside_flags; nonzero = valid), NULL = every anchor is valid.
+ *     On valid anchors the result equals the assignment of the compacted anchors[valid], including the per-GT maxima
+ *     of the low-quality pass, which see valid anchors only.  Invalid anchors get gt_ind -1, max_overlap +0.0 and
+ *     labels_fill.  A mask with no valid anchor gives that on every anchor.
+ *   Other arguments and outputs: as rsdet_assign_wrt_overlaps.
+ * No host synchronisation and no allocation: the workspace (needed only when match_low_quality != 0; the query
+ * returns the size for that case) holds per-GT (IoU, anchor) keys that the call itself initialises on `stream`, so the
+ * call can be captured in a CUDA graph and run on concurrent streams with separate workspaces.
+ * Limits: num_gts <= RSDET_ASSIGN_HBB_MAX_GTS and n <= RSDET_ASSIGN_HBB_MAX_ANCHORS (anchor indices are packed into
+ * 32-bit keys); RSDET_ELIMIT above, and the workspace query then returns 0 (also for num_gts <= 0 or n <= 0).
+ * Argument errors are returned before anything is launched. */
+#define RSDET_ASSIGN_HBB_MAX_GTS (1 << 24)
+#define RSDET_ASSIGN_HBB_MAX_ANCHORS (1 << 30)
+size_t rsdet_assign_hbb_workspace_bytes(int num_gts, int n);
+int rsdet_assign_hbb(const float* gt_hbb, int num_gts, const float* anchors, int n, const uint8_t* valid, float pos_iou_thr,
+                     float neg_lo, float neg_hi, float min_pos_iou, int match_low_quality, int gt_max_assign_all,
+                     const int32_t* gt_labels, int32_t labels_fill, int32_t* assigned_gt_inds, float* max_overlaps,
+                     int32_t* assigned_labels, void* workspace, size_t workspace_bytes, void* stream);
+
 /* ---------------------------------------------------------------- NMS (rotated / poly / merge)
  * One engine, one pair predicate per `kind`: */
 #define RSDET_NMS_ROTATED 0 /* dets (n,5) fp32 obb; suppress IoU >  thr: ops/nms_rotated.py:353-411,450-493 */

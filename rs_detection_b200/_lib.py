@@ -54,6 +54,10 @@ SIGNATURES = {
     "rsdet_assign_workspace_bytes": (C.c_size_t, [C.c_int]),
     "rsdet_assign_wrt_overlaps": (C.c_int, [_vp, C.c_int, C.c_int, C.c_float, C.c_float, C.c_float, C.c_float, C.c_int,
                                             C.c_int, _vp, C.c_int32, _vp, _vp, _vp, _vp, C.c_size_t, _vp]),
+    "rsdet_bbox_overlaps": (C.c_int, [_vp, C.c_int, _vp, C.c_int, _vp, _vp]),
+    "rsdet_assign_hbb_workspace_bytes": (C.c_size_t, [C.c_int, C.c_int]),
+    "rsdet_assign_hbb": (C.c_int, [_vp, C.c_int, _vp, C.c_int, _vp, C.c_float, C.c_float, C.c_float, C.c_float, C.c_int,
+                                   C.c_int, _vp, C.c_int32, _vp, _vp, _vp, _vp, C.c_size_t, _vp]),
     "rsdet_nms_workspace_bytes": (C.c_size_t, [C.c_int, C.c_int]),
     "rsdet_nms": (C.c_int, [C.c_int, _vp, _vp, _vp, C.c_int, C.c_double, _vp, C.c_int, _vp, _vp, _vp, _vp, _vp,
                             C.c_size_t, _vp]),

@@ -84,6 +84,55 @@ def box_iou_rotated(boxes1: torch.Tensor, boxes2: torch.Tensor, version: int = 0
     return out
 
 
+def _neg_range(neg_iou_thr):
+    """Negatives are neg_lo <= max_overlap < neg_hi; a scalar threshold t means (0, t)."""
+    if isinstance(neg_iou_thr, (tuple, list)):
+        return float(neg_iou_thr[0]), float(neg_iou_thr[1])
+    return 0.0, float(neg_iou_thr)
+
+
+def bbox_overlaps(bboxes1: torch.Tensor, bboxes2: torch.Tensor) -> torch.Tensor:
+    """BboxOverlaps2D (mode='iou', not aligned): (n1,4) x (n2,4) [x1,y1,x2,y2] -> (n1,n2) fp32 (include/rsdet.h)."""
+    b1, b2 = _f32(bboxes1), _f32(bboxes2)
+    n1, n2 = b1.shape[0], b2.shape[0]
+    out = torch.empty((n1, n2), dtype=torch.float32, device=b1.device)
+    if n1 == 0 or n2 == 0:
+        return out
+    check(load().rsdet_bbox_overlaps(ptr(b1), n1, ptr(b2), n2, ptr(out), stream_ptr()), "bbox_overlaps")
+    return out
+
+
+def assign_hbb(gt_hbb: torch.Tensor, anchors: torch.Tensor, pos_iou_thr: float, neg_iou_thr, min_pos_iou: float = 0.0,
+               match_low_quality: bool = False, gt_max_assign_all: bool = True, gt_labels: Optional[torch.Tensor] = None,
+               labels_fill: int = -1, valid: Optional[torch.Tensor] = None):
+    """assign_wrt_overlaps(bbox_overlaps(gt_hbb, anchors), ...) bit for bit, without the (G, n) overlaps matrix.
+    `valid` (n,) bool / uint8: on valid anchors the result is that of anchors[valid]; the others get -1, +0.0 and
+    `labels_fill`.  Returns (gt_inds int32, max_overlaps fp32, labels int32 or None)."""
+    g, a = _f32(gt_hbb), _f32(anchors)
+    G, n = g.shape[0], a.shape[0]
+    if G == 0 or n == 0:
+        raise ValueError("No gt or proposals")
+    if g.shape[-1] != 4 or a.shape[-1] != 4:
+        raise ValueError("gt_hbb and anchors must be (N, 4) [x1, y1, x2, y2]")
+    m = None
+    if valid is not None:
+        if not valid.is_cuda or valid.numel() != n:
+            raise ValueError(f"valid must be a CUDA mask of {n} anchors")
+        m = valid.reshape(-1).to(torch.uint8).contiguous()
+    neg_lo, neg_hi = _neg_range(neg_iou_thr)
+    gt_inds = torch.empty((n,), dtype=torch.int32, device=a.device)
+    max_ov = torch.empty((n,), dtype=torch.float32, device=a.device)
+    labels = torch.empty((n,), dtype=torch.int32, device=a.device) if gt_labels is not None else None
+    gl = gt_labels.to(torch.int32).contiguous() if gt_labels is not None else None
+    L = load()
+    wsb = L.rsdet_assign_hbb_workspace_bytes(G, n)
+    ws = workspace(wsb) if match_low_quality else None
+    check(L.rsdet_assign_hbb(ptr(g), G, ptr(a), n, ptr(m), pos_iou_thr, neg_lo, neg_hi, min_pos_iou, int(match_low_quality),
+                             int(gt_max_assign_all), ptr(gl), labels_fill, ptr(gt_inds), ptr(max_ov), ptr(labels), ptr(ws),
+                             0 if ws is None else ws.numel(), stream_ptr()), "assign_hbb")
+    return gt_inds, max_ov, labels
+
+
 def assign_wrt_overlaps(overlaps: torch.Tensor, pos_iou_thr: float, neg_iou_thr, min_pos_iou: float = 0.0,
                         match_low_quality: bool = False, gt_max_assign_all: bool = True,
                         gt_labels: Optional[torch.Tensor] = None, labels_fill: int = -1):
@@ -91,10 +140,7 @@ def assign_wrt_overlaps(overlaps: torch.Tensor, pos_iou_thr: float, neg_iou_thr,
     G, n = ov.shape
     if G == 0 or n == 0:
         raise ValueError("No gt or proposals")
-    if isinstance(neg_iou_thr, (tuple, list)):
-        neg_lo, neg_hi = float(neg_iou_thr[0]), float(neg_iou_thr[1])
-    else:
-        neg_lo, neg_hi = 0.0, float(neg_iou_thr)
+    neg_lo, neg_hi = _neg_range(neg_iou_thr)
     gt_inds = torch.empty((n,), dtype=torch.int32, device=ov.device)
     max_ov = torch.empty((n,), dtype=torch.float32, device=ov.device)
     labels = torch.empty((n,), dtype=torch.int32, device=ov.device) if gt_labels is not None else None

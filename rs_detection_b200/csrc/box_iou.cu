@@ -2,7 +2,8 @@
 //
 // Replaces box_iou_rotated_cuda_kernel (python/jdet/ops/box_iou_rotated.py:413-461, v1 copy
 // box_iou_rotated_v1.py:418-466) and the Python body of MaxIoUAssigner.assign_wrt_overlaps
-// (python/jdet/models/boxes/assigner.py:111-170).
+// (python/jdet/models/boxes/assigner.py:111-170).  Also the horizontal BboxOverlaps2D matrix and the RPN's anchor
+// assignment fused with it (rsdet_assign_hbb), which never stores the (num_gts, n) matrix.
 //
 // Kernel plan (FP32-ALU bound; no tensor cores -- nothing here is a contraction):
 //   prep  : one thread per box -> RBox (double sin/cos once per box, not once per pair)
@@ -182,6 +183,251 @@ __global__ void assign_col_kernel(const float* __restrict__ ov, int G, int n, fl
     if (labels) labels[j] = (a > 0 && gt_labels) ? gt_labels[a - 1] : labels_fill;
 }
 
+// ------------------------------------------------------------------ horizontal IoU + fused anchor assignment
+// BboxOverlaps2D, mode='iou', not aligned: the mmdet 2.x bbox_overlaps that JDet's models/boxes/iou_calculator.py copies.
+// fp32, no "+1", every operation rounded on its own (this unit is built with -fmad=false).  NOT pinned by a fixture
+// (DESIGN.md section 3): both kernels below call this one function so that a fixture can correct it in one place.
+// A disjoint or touching pair gives +0.0 (never -0.0), so every finite IoU is >= +0.0; the fused assignment relies on it.
+__device__ __forceinline__ float hbb_iou(float ax1, float ay1, float ax2, float ay2, float bx1, float by1, float bx2, float by2) {
+    const float area_a = (ax2 - ax1) * (ay2 - ay1);
+    const float area_b = (bx2 - bx1) * (by2 - by1);
+    const float dw = fminf(ax2, bx2) - fmaxf(ax1, bx1);
+    const float dh = fminf(ay2, by2) - fmaxf(ay1, by1);
+    const float w = dw > 0.f ? dw : 0.f;
+    const float h = dh > 0.f ? dh : 0.f;
+    const float overlap = w * h;
+    const float uni = fmaxf((area_a + area_b) - overlap, 1e-6f);
+    return overlap / uni;
+}
+
+__device__ __forceinline__ float hbb_iou(float4 a, float4 b) { return hbb_iou(a.x, a.y, a.z, a.w, b.x, b.y, b.z, b.w); }
+
+constexpr int kOvRows = 8;  // rows of the (n1, n2) matrix per CTA pass: one column box in registers serves 8 rows
+
+__global__ void __launch_bounds__(256)
+bbox_overlaps_kernel(const float* __restrict__ b1, int n1, const float* __restrict__ b2, int n2, float* __restrict__ out) {
+    const int j = blockIdx.x * 256 + threadIdx.x;
+    if (j >= n2) return;
+    const float bx1 = b2[4 * (size_t)j], by1 = b2[4 * (size_t)j + 1], bx2 = b2[4 * (size_t)j + 2], by2 = b2[4 * (size_t)j + 3];
+    for (int r0 = blockIdx.y * kOvRows; r0 < n1; r0 += gridDim.y * kOvRows) {
+        const int r1 = min(r0 + kOvRows, n1);
+        for (int r = r0; r < r1; r++) {
+            const float* a = b1 + 4 * (size_t)r;
+            out[(size_t)r * n2 + j] = hbb_iou(a[0], a[1], a[2], a[3], bx1, by1, bx2, by2);
+        }
+    }
+}
+
+// The fused MaxIoU assignment (rsdet_assign_hbb).  A CTA owns 256 consecutive anchors.  The anchors of one pyramid level
+// are stored in (h, w, a) order, so a CTA's anchors form a thin strip of the image, and most GTs miss it.  A GT "misses"
+// the strip when one of its edges lies beyond the strip's hull on the far side:
+//     gx1 >= max(ax2) || gx2 <= min(ax1) || gy1 >= max(ay2) || gy2 <= min(ay1)
+// Then for every anchor of the strip min(ax2, gx2) <= max(ax1, gx1) (or likewise on y), the difference is <= 0 in fp32
+// too, and the IoU is exactly +0.0.  Skipping such a GT changes no decision of the CTA's anchors:
+//   * column max / argmax: all IoUs are >= +0.0 and the first maximal GT wins, so starting from (+0.0, GT 0) instead of
+//     (-inf, -) gives the same pair, also for a column whose GTs are all skipped (max +0.0, argmax 0);
+//   * low-quality pass: a GT with gt_max > 0 matches only anchors with IoU == gt_max > 0 (its argmax anchor among them),
+//     none of which is in a strip it misses.  A GT with gt_max == 0 >= min_pos_iou matches IoU-0 anchors, so such a GT
+//     is never skipped.
+// NaN coordinates widen the hull to +-inf and fail every comparison, so a GT is never skipped because of one.
+constexpr int kHbbThreads = 256;
+constexpr int kHbbChunk = 1024;  // GTs staged in shared memory per chunk
+
+struct StripHull {
+    float x1, y1, x2, y2;  // min x1, min y1, max x2, max y2 over the CTA's valid anchors
+    int any;               // the CTA has a valid anchor
+};
+
+__device__ __forceinline__ float nan_to(float v, float to) { return v == v ? v : to; }
+
+// Block-wide hull of the valid anchors; every thread gets the result.
+__device__ StripHull strip_hull(bool live, float x1, float y1, float x2, float y2) {
+    __shared__ float s_h[4][kHbbThreads / 32];
+    __shared__ int s_any[kHbbThreads / 32];
+    float a = live ? nan_to(x1, -INFINITY) : INFINITY, b = live ? nan_to(y1, -INFINITY) : INFINITY;
+    float c = live ? nan_to(x2, INFINITY) : -INFINITY, d = live ? nan_to(y2, INFINITY) : -INFINITY;
+    for (int o = 16; o; o >>= 1) {
+        a = fminf(a, __shfl_xor_sync(0xffffffffu, a, o));
+        b = fminf(b, __shfl_xor_sync(0xffffffffu, b, o));
+        c = fmaxf(c, __shfl_xor_sync(0xffffffffu, c, o));
+        d = fmaxf(d, __shfl_xor_sync(0xffffffffu, d, o));
+    }
+    const int anyw = __any_sync(0xffffffffu, live);
+    const int w = threadIdx.x >> 5;
+    if ((threadIdx.x & 31) == 0) { s_h[0][w] = a; s_h[1][w] = b; s_h[2][w] = c; s_h[3][w] = d; s_any[w] = anyw; }
+    __syncthreads();
+    StripHull h{INFINITY, INFINITY, -INFINITY, -INFINITY, 0};
+    for (int k = 0; k < kHbbThreads / 32; k++) {
+        h.x1 = fminf(h.x1, s_h[0][k]); h.y1 = fminf(h.y1, s_h[1][k]);
+        h.x2 = fmaxf(h.x2, s_h[2][k]); h.y2 = fmaxf(h.y2, s_h[3][k]);
+        h.any |= s_any[k];
+    }
+    return h;
+}
+
+__device__ __forceinline__ bool misses(const StripHull& h, float4 g) {
+    return g.x >= h.x2 || g.z <= h.x1 || g.y >= h.y2 || g.w <= h.y1;
+}
+
+__device__ __forceinline__ float4 load_box(const float* __restrict__ p, size_t i) {
+    return make_float4(p[4 * i], p[4 * i + 1], p[4 * i + 2], p[4 * i + 3]);
+}
+
+// gt_key[g] = max over valid anchors of (IoU bits << 32 | ~anchor): the largest IoU, then the first anchor.  Only IoUs
+// > 0 are posted, so a key of 0 means gt_max = +0.0 with the first valid anchor as argmax.
+__device__ __forceinline__ void decode_gt_key(unsigned long long key, unsigned first_valid, float& gm, int& ga) {
+    const unsigned hi = (unsigned)(key >> 32);
+    gm = __uint_as_float(hi);
+    ga = hi ? (int)~(unsigned)key : (int)first_valid;
+}
+
+__global__ void assign_hbb_init_kernel(unsigned long long* __restrict__ gt_key, int G, unsigned* __restrict__ first_valid) {
+    for (int g = blockIdx.x * blockDim.x + threadIdx.x; g < G; g += gridDim.x * blockDim.x) gt_key[g] = 0ull;
+    if (blockIdx.x == 0 && threadIdx.x == 0) *first_valid = 0xffffffffu;
+}
+
+// Row pass (match_low_quality only): per-GT max / first argmax over the valid anchors.  The CTA stages its valid anchors
+// in order; each thread takes whole GTs of the compacted non-missing list and scans the strip, so ties keep the first
+// anchor without any reduction; one 64-bit atomicMax per (GT, CTA) with a positive maximum.
+__global__ void __launch_bounds__(kHbbThreads)
+assign_hbb_gt_max_kernel(const float* __restrict__ gts, int G, const float* __restrict__ anchors, int n,
+                         const uint8_t* __restrict__ valid, unsigned long long* __restrict__ gt_key,
+                         unsigned* __restrict__ first_valid) {
+    __shared__ float4 s_anc[kHbbThreads];
+    __shared__ int s_aidx[kHbbThreads];
+    __shared__ int s_wcnt[kHbbThreads / 32];
+    __shared__ float4 s_gt[kHbbChunk];
+    __shared__ int s_gidx[kHbbChunk];
+    __shared__ int s_ng;
+    const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
+    const int j = blockIdx.x * kHbbThreads + tid;
+    const bool live = j < n && (!valid || valid[j]);
+    const float4 a = j < n ? load_box(anchors, j) : make_float4(0.f, 0.f, 0.f, 0.f);
+    const StripHull hull = strip_hull(live, a.x, a.y, a.z, a.w);
+    if (!hull.any) return;
+
+    // order-preserving compaction of the valid anchors
+    const unsigned m = __ballot_sync(0xffffffffu, live);
+    if (lane == 0) s_wcnt[wid] = __popc(m);
+    __syncthreads();
+    int base = 0, na = 0;
+    for (int k = 0; k < kHbbThreads / 32; k++) {
+        base += k < wid ? s_wcnt[k] : 0;
+        na += s_wcnt[k];
+    }
+    const int pos = base + __popc(m & ((1u << lane) - 1));
+    if (live) { s_anc[pos] = a; s_aidx[pos] = j; }
+    if (live && pos == 0) atomicMin(first_valid, (unsigned)j);
+
+    for (int c0 = 0; c0 < G; c0 += kHbbChunk) {
+        const int cn = min(kHbbChunk, G - c0);
+        if (tid == 0) s_ng = 0;
+        __syncthreads();  // s_anc written
+        for (int k = tid; k < cn; k += kHbbThreads) {
+            const float4 g = load_box(gts, (size_t)(c0 + k));
+            if (!misses(hull, g)) {
+                const int p = atomicAdd(&s_ng, 1);  // the per-GT maxima do not depend on the list's order
+                s_gt[p] = g;
+                s_gidx[p] = c0 + k;
+            }
+        }
+        __syncthreads();
+        const int ng = s_ng;
+        for (int k = tid; k < ng; k += kHbbThreads) {
+            const float4 g = s_gt[k];
+            float best = 0.f;
+            int bi = -1;
+            for (int q = 0; q < na; q++) {
+                const float v = hbb_iou(g, s_anc[q]);
+                if (v > best) { best = v; bi = q; }
+            }
+            if (bi >= 0)
+                atomicMax(gt_key + s_gidx[k], ((unsigned long long)__float_as_uint(best) << 32) | (unsigned)~(unsigned)s_aidx[bi]);
+        }
+        __syncthreads();  // the list and s_ng fully read before the next chunk resets them
+    }
+}
+
+// Column pass: one thread per anchor over the GTs that do not miss the CTA's strip, staged in chunks and in GT order
+// (the first maximal GT wins the argmax, the last low-quality match wins).  The decisions are assign_col_kernel's.
+__global__ void __launch_bounds__(kHbbThreads)
+assign_hbb_col_kernel(const float* __restrict__ gts, int G, const float* __restrict__ anchors, int n,
+                      const uint8_t* __restrict__ valid, float pos_thr, float neg_lo, float neg_hi, float min_pos_iou,
+                      int match_low_quality, int assign_all, const unsigned long long* __restrict__ gt_key,
+                      const unsigned* __restrict__ first_valid, const int32_t* __restrict__ gt_labels,
+                      int32_t labels_fill, int32_t* __restrict__ gt_inds, float* __restrict__ max_ov,
+                      int32_t* __restrict__ labels) {
+    __shared__ float4 s_gt[kHbbChunk];
+    __shared__ int s_gidx[kHbbChunk];
+    __shared__ float s_gm[kHbbChunk];
+    __shared__ int s_ga[kHbbChunk];
+    __shared__ int s_wcnt[kHbbThreads / 32];
+    const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
+    const int j = blockIdx.x * kHbbThreads + tid;
+    const bool live = j < n && (!valid || valid[j]);
+    const float4 a = j < n ? load_box(anchors, j) : make_float4(0.f, 0.f, 0.f, 0.f);
+    const StripHull hull = strip_hull(live, a.x, a.y, a.z, a.w);
+
+    float best = 0.f;
+    int bi = 0, lowq = 0;
+    if (hull.any) {
+        const unsigned fv = match_low_quality ? *first_valid : 0u;
+        for (int c0 = 0; c0 < G; c0 += kHbbChunk) {
+            const int cn = min(kHbbChunk, G - c0);
+            int base = 0;
+            for (int r0 = 0; r0 < cn; r0 += kHbbThreads) {
+                const int k = r0 + tid;
+                float4 g = make_float4(0.f, 0.f, 0.f, 0.f);
+                float gm = 0.f;
+                int ga = 0;
+                bool keep = false;
+                if (k < cn) {
+                    g = load_box(gts, (size_t)(c0 + k));
+                    keep = !misses(hull, g);
+                    if (match_low_quality) {
+                        decode_gt_key(gt_key[c0 + k], fv, gm, ga);
+                        keep |= gm == 0.f && gm >= min_pos_iou;
+                    }
+                }
+                const unsigned m = __ballot_sync(0xffffffffu, keep);
+                __syncthreads();  // s_wcnt free (and, on the first round, the previous chunk's list fully read)
+                if (lane == 0) s_wcnt[wid] = __popc(m);
+                __syncthreads();
+                int pos = base, tot = 0;
+                for (int w = 0; w < kHbbThreads / 32; w++) {
+                    pos += w < wid ? s_wcnt[w] : 0;
+                    tot += s_wcnt[w];
+                }
+                pos += __popc(m & ((1u << lane) - 1));
+                if (keep) { s_gt[pos] = g; s_gidx[pos] = c0 + k; s_gm[pos] = gm; s_ga[pos] = ga; }
+                base += tot;
+            }
+            __syncthreads();
+            if (live) {
+                for (int q = 0; q < base; q++) {
+                    const float v = hbb_iou(s_gt[q], a);
+                    const int g = s_gidx[q];
+                    if (v > best) { best = v; bi = g; }
+                    if (match_low_quality) {
+                        const float gm = s_gm[q];
+                        if (gm >= min_pos_iou && (assign_all ? (v == gm) : (s_ga[q] == j))) lowq = g + 1;
+                    }
+                }
+            }
+        }
+    }
+    if (j >= n) return;
+    int r = -1;
+    if (live) {
+        if (best >= neg_lo && best < neg_hi) r = 0;
+        if (best >= pos_thr) r = bi + 1;
+        if (lowq) r = lowq;
+    }
+    gt_inds[j] = r;
+    if (max_ov) max_ov[j] = best;
+    if (labels) labels[j] = (r > 0 && gt_labels) ? gt_labels[r - 1] : labels_fill;
+}
+
 }  // namespace rsdet
 
 using namespace rsdet;
@@ -235,6 +481,56 @@ extern "C" int rsdet_assign_wrt_overlaps(const float* overlaps, int num_gts, int
     assign_col_kernel<<<ceil_div(n, 128), 128, 0, st>>>(overlaps, num_gts, n, pos_iou_thr, neg_lo, neg_hi, min_pos_iou,
                                                          match_low_quality, gt_max_assign_all, gt_max, gt_arg, gt_labels,
                                                          labels_fill, assigned_gt_inds, max_overlaps, assigned_labels);
+    count_launch();
+    return cuda_status();
+}
+
+extern "C" int rsdet_bbox_overlaps(const float* boxes1, int n1, const float* boxes2, int n2, float* ious, void* stream) {
+    if (n1 < 0 || n2 < 0) return RSDET_EINVAL;
+    if (n1 == 0 || n2 == 0) return RSDET_OK;
+    if (!boxes1 || !boxes2 || !ious) return RSDET_EINVAL;
+    if ((long long)n1 * n2 > (1ll << 40)) return RSDET_ELIMIT;
+    const int row_groups = ceil_div(n1, kOvRows);
+    dim3 grid(ceil_div(n2, 256), row_groups < 65535 ? row_groups : 65535);
+    bbox_overlaps_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(boxes1, n1, boxes2, n2, ious);
+    count_launch();
+    return cuda_status();
+}
+
+static bool assign_hbb_sizes_ok(int num_gts, int n) {
+    return num_gts <= RSDET_ASSIGN_HBB_MAX_GTS && n <= RSDET_ASSIGN_HBB_MAX_ANCHORS;
+}
+
+extern "C" size_t rsdet_assign_hbb_workspace_bytes(int num_gts, int n) {
+    if (num_gts <= 0 || n <= 0 || !assign_hbb_sizes_ok(num_gts, n)) return 0;
+    return ws_bytes<unsigned long long>(num_gts) + ws_bytes<unsigned>(1);
+}
+
+extern "C" int rsdet_assign_hbb(const float* gt_hbb, int num_gts, const float* anchors, int n, const uint8_t* valid,
+                                float pos_iou_thr, float neg_lo, float neg_hi, float min_pos_iou, int match_low_quality,
+                                int gt_max_assign_all, const int32_t* gt_labels, int32_t labels_fill,
+                                int32_t* assigned_gt_inds, float* max_overlaps, int32_t* assigned_labels, void* workspace,
+                                size_t workspace_bytes, void* stream) {
+    if (num_gts <= 0 || n <= 0) return RSDET_EINVAL;  // as rsdet_assign_wrt_overlaps
+    if (!gt_hbb || !anchors || !assigned_gt_inds) return RSDET_EINVAL;
+    if (!assign_hbb_sizes_ok(num_gts, n)) return RSDET_ELIMIT;
+    cudaStream_t st = (cudaStream_t)stream;
+    unsigned long long* gt_key = nullptr;
+    unsigned* first_valid = nullptr;
+    if (match_low_quality) {
+        Workspace ws(workspace, workspace_bytes);
+        gt_key = ws.take<unsigned long long>(num_gts);
+        first_valid = ws.take<unsigned>(1);
+        if (!ws.ok()) return RSDET_EWORKSPACE;
+        const int init_grid = ceil_div(num_gts, 256) < kNumSMs ? ceil_div(num_gts, 256) : kNumSMs;
+        assign_hbb_init_kernel<<<init_grid, 256, 0, st>>>(gt_key, num_gts, first_valid);
+        assign_hbb_gt_max_kernel<<<ceil_div(n, kHbbThreads), kHbbThreads, 0, st>>>(gt_hbb, num_gts, anchors, n, valid, gt_key,
+                                                                                 first_valid);
+        count_launch(2);
+    }
+    assign_hbb_col_kernel<<<ceil_div(n, kHbbThreads), kHbbThreads, 0, st>>>(
+        gt_hbb, num_gts, anchors, n, valid, pos_iou_thr, neg_lo, neg_hi, min_pos_iou, match_low_quality, gt_max_assign_all,
+        gt_key, first_valid, gt_labels, labels_fill, assigned_gt_inds, max_overlaps, assigned_labels);
     count_launch();
     return cuda_status();
 }

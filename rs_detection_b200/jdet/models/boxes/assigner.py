@@ -2,13 +2,17 @@
 
 `assign_wrt_overlaps` is one kernel (column max/argmax + thresholds + optional low-quality matching)
 instead of ~10 small Jittor ops and a Python loop over GTs with `jt.sync_all()` every 100 (:152-160).
+With the horizontal calculator `BboxOverlaps2D` (the oriented RPN's), `assign` takes `core.assign_hbb`, which gives
+the same bits without storing the (num_gts, n) overlaps matrix, at every number of GTs.
 """
 import torch
 
 from .... import core
-from .iou_calculator import BboxOverlaps2D_rotated, BboxOverlaps2D_rotated_v1
+from ...ops._io import back, dev
+from .iou_calculator import BboxOverlaps2D, BboxOverlaps2D_rotated, BboxOverlaps2D_rotated_v1
 
-_CALCULATORS = {'BboxOverlaps2D_rotated': BboxOverlaps2D_rotated, 'BboxOverlaps2D_rotated_v1': BboxOverlaps2D_rotated_v1}
+_CALCULATORS = {'BboxOverlaps2D_rotated': BboxOverlaps2D_rotated, 'BboxOverlaps2D_rotated_v1': BboxOverlaps2D_rotated_v1,
+                'BboxOverlaps2D': BboxOverlaps2D}
 
 
 class AssignResult:
@@ -45,11 +49,26 @@ class MaxIoUAssigner:
     def assign(self, bboxes, gt_bboxes, gt_bboxes_ignore=None, gt_labels=None):
         if bboxes.shape[0] == 0 or gt_bboxes.shape[0] == 0:
             raise ValueError('No gt or bboxes')
+        if isinstance(self.iou_calculator, BboxOverlaps2D):
+            return self._assign_hbb(bboxes, gt_bboxes, gt_bboxes_ignore, gt_labels)
         overlaps = self.iou_calculator(gt_bboxes, bboxes)
         if (self.ignore_iof_thr > 0) and (gt_bboxes_ignore is not None) and (gt_bboxes_ignore.numel() > 0):
             raise NotImplementedError("'iof' ignore regions are not on the rotated hot path (the rotated "
                                       "calculators assert mode == 'iou', iou_calculator.py:108,148)")
         return self.assign_wrt_overlaps(overlaps, gt_labels)
+
+    def _assign_hbb(self, bboxes, gt_bboxes, gt_bboxes_ignore, gt_labels):
+        """assign_wrt_overlaps(BboxOverlaps2D()(gt_bboxes, bboxes)) in one fused call (rsdet_assign_hbb)."""
+        if (self.ignore_iof_thr > 0) and (gt_bboxes_ignore is not None) and (gt_bboxes_ignore.numel() > 0):
+            raise NotImplementedError("'iof' ignore regions are not supported by the fused horizontal assignment")
+        assert gt_bboxes.size(-1) in [4, 5] and bboxes.size(-1) in [4, 5]
+        anchors, fl = dev(bboxes[..., :4])
+        gts, _ = dev(gt_bboxes[..., :4])
+        gl = None if gt_labels is None else dev(gt_labels, torch.int32)[0]
+        gt_inds, max_overlaps, labels = core.assign_hbb(
+            gts.reshape(-1, 4), anchors.reshape(-1, 4), float(self.pos_iou_thr), self.neg_iou_thr, float(self.min_pos_iou),
+            bool(self.match_low_quality), bool(self.gt_max_assign_all), gl, int(self.assigned_labels_filled))
+        return AssignResult(gts.shape[0], back(gt_inds, fl), back(max_overlaps, fl), labels=back(labels, fl))
 
     def assign_wrt_overlaps(self, overlaps, gt_labels=None):
         if overlaps.numel() == 0:

@@ -137,6 +137,47 @@ def assign_wrt_overlaps(overlaps, pos_iou_thr, neg_iou_thr, min_pos_iou=0.0, mat
     return outs[0], outs[1], (outs[2] if gt_labels is not None else None)
 
 
+# ------------------------------------------------------------------------------------------------ horizontal IoU
+def bbox_overlaps(bboxes1, bboxes2):
+    """BboxOverlaps2D (mode='iou', not aligned; models/boxes/iou_calculator.py): (n1,4) x (n2,4) -> (n1,n2)."""
+    jt = _jt()
+    n1, n2 = bboxes1.shape[0], bboxes2.shape[0]
+    if n1 == 0 or n2 == 0:
+        return jt.zeros((n1, n2), dtype="float32")
+    ious = _code((n1 * n2,), "float32", [bboxes1, bboxes2], r'''
+        RSDET_FN(rsdet_bbox_overlaps);
+        rsdet_check(fn_rsdet_bbox_overlaps(in0_p, in0_shape0, in1_p, in1_shape0, out0_p, 0), "bbox_overlaps");''')
+    return ious.reshape(n1, n2)
+
+
+def assign_hbb(gt_hbb, anchors, pos_iou_thr, neg_iou_thr, min_pos_iou=0.0, match_low_quality=True, gt_max_assign_all=True,
+               gt_labels=None, assigned_labels_filled=0, valid=None):
+    """assign_wrt_overlaps(bbox_overlaps(gt_hbb, anchors), ...) fused (rsdet_assign_hbb); `valid` is an optional uint8
+    (n,) mask (anchor_inside_flags).  -> (assigned_gt_inds int32, max_overlaps, assigned_labels int32 or None)."""
+    G, n = gt_hbb.shape[0], anchors.shape[0]
+    if G == 0 or n == 0:
+        raise ValueError('No gt or proposals')
+    neg_lo, neg_hi = (neg_iou_thr if isinstance(neg_iou_thr, tuple) else (0.0, neg_iou_thr))
+    ins = [gt_hbb, anchors]
+    labels_in = valid_in = "nullptr"
+    if gt_labels is not None:
+        labels_in = "(const int32_t*)in%d_p" % len(ins)
+        ins.append(gt_labels.int32())
+    if valid is not None:
+        valid_in = "(const uint8_t*)in%d_p" % len(ins)
+        ins.append(valid)
+    outs = _code([(n,), (n,), (n,)], ["int32", "float32", "int32"], ins, r'''
+        RSDET_FN(rsdet_assign_hbb_workspace_bytes);
+        RSDET_FN(rsdet_assign_hbb);
+        int G = in0_shape0, n = in1_shape0;
+        Scratch s(fn_rsdet_assign_hbb_workspace_bytes(G, n));
+        rsdet_check(fn_rsdet_assign_hbb(in0_p, G, in1_p, n, %s, %rf, %rf, %rf, %rf, %d, %d, %s, %d, (int32_t*)out0_p, out1_p,
+                                        (int32_t*)out2_p, s.p, s.bytes, 0), "assign_hbb");'''
+                 % (valid_in, float(pos_iou_thr), float(neg_lo), float(neg_hi), float(min_pos_iou), int(match_low_quality),
+                    int(gt_max_assign_all), labels_in, int(assigned_labels_filled)))
+    return outs[0], outs[1], (outs[2] if gt_labels is not None else None)
+
+
 # ------------------------------------------------------------------------------------------------ NMS family
 def _nms_keep(kind, dets, scores, labels, thr):
     """bool keep mask in ORIGINAL index space (nms_rotated_cuda's `keep`, nms_rotated.py:506-513)."""
