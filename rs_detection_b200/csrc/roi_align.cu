@@ -200,15 +200,14 @@ __global__ void __launch_bounds__(256) convert_maps_kernel(ConvertJob job) {
 
 struct LevelSet;
 struct RoiGeom;
-struct PrepArgs {                 // order block riding along with the NCHW->NHWC transpose (see roi_order_block)
+struct PrepArgs {                 // order block and geometry blocks riding along with the NCHW->NHWC transpose
     const LevelSet* L;
     const float* rois;
     int K;
     int* order;
-    // lean flow (persistent forward kernel): geometry blocks ride along as well
-    RoiGeom* geoms = nullptr;
-    int32_t* levels_out = nullptr;
-    unsigned* counter = nullptr;
+    RoiGeom* geoms;
+    int32_t* levels_out;
+    unsigned* counter;
 };
 template <typename S, typename D>
 static int launch_transpose(bool to_nhwc, const S* const* src, D* const* dst, const int* H, const int* W, int L, int N,
@@ -397,19 +396,6 @@ __device__ __forceinline__ void red_add_v4(float* p, float4 v) {
 __host__ __device__ inline size_t list_bytes(size_t nbins, size_t cap) { return (8 * nbins * (cap + 1) + 15) & ~(size_t)15; }
 __host__ __device__ inline int quads_per_chunk(int C) { return (C / 4) < 64 ? (C / 4) : 64; }
 
-// ---------------------------------------------------------------------------------- per-RoI geometry
-// sin/cos/log2/sqrt and six divisions per RoI: done by K parallel threads here instead of by thread 0 of
-// every RoI's CTA (a ~1.5 us serial chain in front of each CTA's barrier).
-__global__ void roi_geometry_kernel(LevelSet L, const float* __restrict__ rois, int K, const int* __restrict__ order,
-                                    RoiGeom* __restrict__ geoms, int32_t* __restrict__ levels_out) {
-    const int p = blockIdx.x * blockDim.x + threadIdx.x;   // position in processing order
-    if (p >= K) return;
-    const int i = order ? order[p] : p;
-    const RoiGeom g = roi_geometry(rois + (size_t)i * 6, L);
-    geoms[i] = g;
-    if (levels_out) levels_out[i] = g.level;
-}
-
 // ---------------------------------------------------------------------------------- processing order
 // RoIs are independent, so the ORDER in which CTAs take them is free.  A one-CTA counting sort buckets
 // them by (level, 128-pixel image cell): CTAs that run at the same time then read the same few MB of
@@ -419,11 +405,6 @@ constexpr int kCellShift = 7;   // 128-pixel cells in image coordinates
 constexpr int kCellsPerAxis = 16;
 constexpr int kBuckets = RSDET_MAX_LEVELS * kCellsPerAxis * kCellsPerAxis;
 
-// The locality order of a call (what roi_order_kernel does) as ONE block of any size, so that for NCHW callers it can
-// ride along as an extra block of the NCHW->NHWC transpose: the order kernel is a 7.8 us single-CTA latency chain in
-// front of every gather, the transpose of a 1024^2 pyramid keeps the other SMs busy for 30 us anyway.  (Doing the
-// geometry in the same block as well was measured and dropped: sin/cos/log2 of 4000 RoIs on one SM take longer than
-// the two launches they replace.)  geoms[] must have been written by roi_geometry_kernel.  s_hist: kBuckets ints.
 // bucket of a RoI in the locality order.  One image: (level, 128-px cell, boustrophedon rows).  A batch of images: the image
 // is the major key -- CTAs that run at the same time then read ONE image's maps (8 images x 89 MB do not fit L2 together) --
 // with 256-px cells so that (image slot, level, cell) still fits kBuckets.
@@ -443,6 +424,11 @@ __device__ __forceinline__ int roi_bucket(const float* __restrict__ r, int lvl, 
 }
 
 constexpr int kPrepMaxRois = 16384;
+// The locality order of a call as ONE block of any size: block 0 of roi_prep_kernel, or for NCHW callers an extra block
+// of the NCHW->NHWC transpose, whose other SMs are busy for 30 us on a 1024^2 pyramid anyway (the order is a 7.8 us
+// single-CTA latency chain).  Doing the geometry in the same block as well was measured and dropped: sin/cos/log2 of 4000
+// RoIs on one SM take longer than the launch they replace.  s_hist: kBuckets ints, s_warp: 32 ints.
+static_assert(kBuckets <= 65536, "bucket ids are cached as unsigned short");
 template <int THREADS>
 __device__ __forceinline__ void roi_order_block(const LevelSet& L, const float* __restrict__ rois, int K,
                                                 int* __restrict__ order, int* s_hist, int* s_warp, unsigned short* s_bkt, int bkt_cap) {
@@ -484,69 +470,13 @@ __device__ __forceinline__ void roi_order_block(const LevelSet& L, const float* 
     }
 }
 
-__device__ __forceinline__ void roi_order_1024(const LevelSet& L, const float* __restrict__ rois, int K, int* __restrict__ order) {
-    __shared__ int s_hist[kBuckets];
-    __shared__ int s_warp[32];
-    const int tid = threadIdx.x;
-    for (int i = tid; i < kBuckets; i += 1024) s_hist[i] = 0;
-    __syncthreads();
-    auto bucket_of = [&](int i, int& lvl) {
-        const float* r = rois + (size_t)i * 6;
-        lvl = roi_level(r, L);
-        return roi_bucket(r, lvl, L);
-    };
-    int cached[4] = {0, 0, 0, 0};   // buckets of this thread's first four RoIs: the scatter pass reloads nothing for K <= 4096
-#pragma unroll
-    for (int c = 0; c < 4; c++) {
-        const int i = tid + 1024 * c;
-        if (i < K) {
-            int lvl;
-            cached[c] = bucket_of(i, lvl);
-            atomicAdd(&s_hist[cached[c]], 1);
-        }
-    }
-    for (int i = tid + 4096; i < K; i += 1024) {
-        int lvl;
-        atomicAdd(&s_hist[bucket_of(i, lvl)], 1);
-    }
-    __syncthreads();
-    // exclusive scan of kBuckets (=2048) counters: 2 per thread
-    int a0 = s_hist[2 * tid], a1 = s_hist[2 * tid + 1];
-    int sum = a0 + a1, x = sum;
-    const int lane = tid & 31, w = tid >> 5;
-    for (int o = 1; o < 32; o <<= 1) { int y = __shfl_up_sync(0xffffffffu, x, o); if (lane >= o) x += y; }
-    if (lane == 31) s_warp[w] = x;
-    __syncthreads();
-    if (w == 0) {
-        int v = s_warp[lane];
-        for (int o = 1; o < 32; o <<= 1) { int y = __shfl_up_sync(0xffffffffu, v, o); if (lane >= o) v += y; }
-        s_warp[lane] = v;
-    }
-    __syncthreads();
-    int excl = (w ? s_warp[w - 1] : 0) + x - sum;
-    s_hist[2 * tid] = excl;
-    s_hist[2 * tid + 1] = excl + a0;
-    __syncthreads();
-#pragma unroll
-    for (int c = 0; c < 4; c++) {
-        const int i = tid + 1024 * c;
-        if (i < K) order[atomicAdd(&s_hist[cached[c]], 1)] = i;
-    }
-    for (int i = tid + 4096; i < K; i += 1024) {
-        int lvl;
-        int bkt = bucket_of(i, lvl);
-        order[atomicAdd(&s_hist[bkt], 1)] = i;
-    }
-}
-
-__global__ void __launch_bounds__(1024) roi_order_kernel(LevelSet L, const float* __restrict__ rois, int K,
-                                                         int* __restrict__ order) {
-    roi_order_1024(L, rois, K, order);
-}
-
-// Lean prologue of the persistent forward kernel, ONE launch: block 0 = the locality order (when there is one), the other
-// blocks = the per-RoI geometry records BY ROI INDEX (the persistent kernel looks a record up through order[] while it
-// gathers the previous item, so nothing has to be written in processing order) + the reset of its work counter.
+// The prologue of a fast call, ONE launch: block 0 = the locality order (when there is one), the other blocks = the
+// per-RoI geometry records BY ROI INDEX + the reset of the persistent forward kernel's work counter (when there is one:
+// the backward has none).  The gather kernels look a record up through order[] (the persistent one while it gathers the
+// previous item), so nothing has to be written in processing order and order and geometry do not depend on each other.
+// sin/cos/log2/sqrt and six divisions per RoI are done by K parallel threads here instead of by thread 0 of every RoI's
+// CTA (a ~1.5 us serial chain in front of each CTA's barrier).
+constexpr int kPrepBucketCache = 16384;   // buckets cached by the order block: 32 KB + the 8 KB histogram of static smem
 __device__ __forceinline__ void roi_geometry_by_index(const LevelSet& L, const float* __restrict__ rois, int K, int i,
                                                       RoiGeom* __restrict__ geoms, int32_t* __restrict__ levels_out) {
     if (i >= K) return;
@@ -559,14 +489,19 @@ __global__ void __launch_bounds__(1024) roi_prep_kernel(LevelSet L, const float*
                                                         unsigned* __restrict__ counter) {
     int gb = blockIdx.x;
     if (order) {
-        if (gb == 0) { roi_order_1024(L, rois, K, order); return; }
+        if (gb == 0) {
+            __shared__ int s_hist[kBuckets + 32];
+            __shared__ unsigned short s_bkt[kPrepBucketCache];
+            roi_order_block<1024>(L, rois, K, order, s_hist, s_hist + kBuckets, s_bkt, kPrepBucketCache);
+            return;
+        }
         gb--;
     }
-    if (gb == 0 && threadIdx.x == 0) *counter = 0u;
+    if (gb == 0 && threadIdx.x == 0 && counter) *counter = 0u;
     roi_geometry_by_index(L, rois, K, gb * 1024 + threadIdx.x, geoms, levels_out);
 }
 
-// NCHW callers: the pyramid transpose with the order block riding along as block 0
+// NCHW callers: the pyramid transpose with the order block riding along as block 0 and the geometry blocks after it
 template <typename T>
 __global__ void __launch_bounds__(256) transpose_prep_kernel(TransposeJob job, LevelSet L, const float* __restrict__ rois, int K,
                                                              int* __restrict__ order, RoiGeom* __restrict__ geoms,
@@ -576,13 +511,12 @@ __global__ void __launch_bounds__(256) transpose_prep_kernel(TransposeJob job, L
     static_assert(sizeof(float) * 64 * 65 >= sizeof(int) * (kBuckets + 32), "the prep block borrows the transpose tile");
     if (blockIdx.x == 0) {
         int* s_hist = reinterpret_cast<int*>(&tile[0][0]);
-        static_assert(kBuckets <= 65536, "bucket ids are cached as unsigned short");
         unsigned short* s_bkt = reinterpret_cast<unsigned short*>(s_hist + kBuckets + 32);
         const int bkt_cap = (int)((sizeof(float) * 64 * 65 - sizeof(int) * (kBuckets + 32)) / sizeof(unsigned short));
         roi_order_block<256>(L, rois, K, order, s_hist, s_hist + kBuckets, s_bkt, bkt_cap);
         return;
     }
-    if ((int)blockIdx.x <= geom_blocks) {      // lean flow: geometry records by RoI index, 256 per block
+    if ((int)blockIdx.x <= geom_blocks) {      // geometry records by RoI index, 256 per block
         if (blockIdx.x == 1 && threadIdx.x == 0) *counter = 0u;
         roi_geometry_by_index(L, rois, K, ((int)blockIdx.x - 1) * 256 + threadIdx.x, geoms, levels_out);
         return;
@@ -605,7 +539,7 @@ static int launch_transpose(bool to_nhwc, const S* const* src, D* const* dst, co
     job.tile_begin[L] = total;
     if constexpr (std::is_same<S, D>::value) {
         if (prep && to_nhwc) {
-            const int geom_blocks = prep->geoms ? ceil_div(prep->K, 256) : 0;
+            const int geom_blocks = ceil_div(prep->K, 256);
             transpose_prep_kernel<S><<<total + 1 + geom_blocks, 256, 0, st>>>(job, *prep->L, prep->rois, prep->K, prep->order,
                                                                                prep->geoms, prep->levels_out, prep->counter,
                                                                                geom_blocks);
@@ -621,24 +555,6 @@ static int launch_transpose(bool to_nhwc, const S* const* src, D* const* dst, co
     }
     count_launch();
     return cuda_status();
-}
-
-// locality order (calls of >= 256 RoIs) and geometry of a call.  The order comes first: the geometry kernel takes the
-// RoIs in processing order and writes each record at its RoI index.  order_rides_with_transpose: the caller's transpose
-// launch produces the order (block 0) and the caller launches the geometry kernel after it.
-static void launch_geometry(const LevelSet& L, const float* rois, int K, const int* order, RoiGeom* geoms, int32_t* levels_out,
-                            cudaStream_t st) {
-    roi_geometry_kernel<<<ceil_div(K, 128), 128, 0, st>>>(L, rois, K, order, geoms, levels_out);
-    count_launch();
-}
-static void launch_prep(const LevelSet& L, const float* rois, int K, RoiGeom* geoms, int* order, int32_t* levels_out, cudaStream_t st,
-                        bool order_rides_with_transpose = false) {
-    if (order_rides_with_transpose) return;
-    if (order) {
-        roi_order_kernel<<<1, 1024, 0, st>>>(L, rois, K, order);
-        count_launch();
-    }
-    launch_geometry(L, rois, K, order, geoms, levels_out, st);
 }
 
 // ---------------------------------------------------------------------------------- tap lists
@@ -790,8 +706,7 @@ __device__ __forceinline__ float4 unrot4(float4 v, int o) { return rot4(v, (4 - 
 // when out's base is aligned to four elements (scalar stores otherwise), and the staging block is only phase-A scratch.
 template <int QPT, typename T = float, typename O = float, bool NHWC_OUT = false>   // T: feature elements, O: output elements
 __global__ void __launch_bounds__(kRoiThreads, 3)
-roi_align_fwd_kernel(LevelSet L, const float* __restrict__ rois, const int* __restrict__ order, const RoiGeom* __restrict__ geoms,
-                     int K, O* __restrict__ out, int32_t* __restrict__ levels_out) {
+roi_align_fwd_kernel(LevelSet L, const int* __restrict__ order, const RoiGeom* __restrict__ geoms, int K, O* __restrict__ out) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int roi = order ? order[blockIdx.x] : blockIdx.x;
     const int tid = threadIdx.x;
@@ -806,16 +721,8 @@ roi_align_fwd_kernel(LevelSet L, const float* __restrict__ rois, const int* __re
     int2* s_list = reinterpret_cast<int2*>(smem_raw);
     int* s_cnt = reinterpret_cast<int*>(smem_raw + list_bytes(nbins, cap));
     O* s_stage = reinterpret_cast<O*>(smem_raw + list_bytes(nbins, cap) + ((nbins * 4 + 15) & ~15));
-    __shared__ RoiGeom s_g;
 
-    if (!geoms) {
-        if (tid == 0) {
-            s_g = roi_geometry(rois + (size_t)roi * 6, L);
-            if (levels_out && blockIdx.y == 0) levels_out[roi] = s_g.level;
-        }
-        __syncthreads();
-    }
-    const RoiGeom g = geoms ? geoms[roi] : s_g;
+    const RoiGeom g = geoms[roi];
     const int H = L.H[g.level], W = L.W[g.level];
     build_tap_lists(g, L, H, W, s_list, s_cnt, reinterpret_cast<float*>(s_stage), C >> 2);   // the scratch is dead after its final barrier
 
@@ -1131,8 +1038,8 @@ static bool fwd77_ok(const rsdet_roi_align_cfg* c) {
 // when grad_out's base is aligned to four elements, scalar loads otherwise) and nothing is staged.
 template <int QPT, typename G = float, bool NHWC_IN = false>   // G: grad_out elements (staged as fp32); the accumulators are always fp32
 __global__ void __launch_bounds__(kRoiThreads, 4)
-roi_align_bwd_kernel(LevelSet L, const float* __restrict__ rois, const int* __restrict__ order, const RoiGeom* __restrict__ geoms,
-                     int K, const G* __restrict__ grad_out) {
+roi_align_bwd_kernel(LevelSet L, const int* __restrict__ order, const RoiGeom* __restrict__ geoms, int K,
+                     const G* __restrict__ grad_out) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int roi = order ? order[blockIdx.x] : blockIdx.x;
     const int tid = threadIdx.x;
@@ -1146,13 +1053,8 @@ roi_align_bwd_kernel(LevelSet L, const float* __restrict__ rois, const int* __re
     int2* s_list = reinterpret_cast<int2*>(smem_raw);
     int* s_cnt = reinterpret_cast<int*>(smem_raw + list_bytes(nbins, cap));
     float* s_stage = reinterpret_cast<float*>(smem_raw + list_bytes(nbins, cap) + ((nbins * 4 + 15) & ~15));
-    __shared__ RoiGeom s_g;
 
-    if (!geoms) {
-        if (tid == 0) s_g = roi_geometry(rois + (size_t)roi * 6, L);
-        __syncthreads();
-    }
-    const RoiGeom g = geoms ? geoms[roi] : s_g;
+    const RoiGeom g = geoms[roi];
     const int H = L.H[g.level], W = L.W[g.level];
     build_tap_lists(g, L, H, W, s_list, s_cnt, s_stage, C >> 2);
 
@@ -1338,6 +1240,26 @@ static size_t fwd_smem_bytes(const rsdet_roi_align_cfg* c) {
     return list_bytes(nbins, ntaps / nbins) + ((nbins * 4 + 15) & ~(size_t)15) + (stage > tmp ? stage : tmp);
 }
 
+// roi_align_generic_kernel over the caller's maps (forward: feature maps, backward: fp32 gradient maps), one thread per
+// output element, at most 16 CTAs per SM
+template <bool BACKWARD, typename T, typename O, bool NHWC_ROIS, typename P>
+static void launch_generic(const rsdet_roi_align_cfg* cfg, const LevelSet& L, P const* maps, const float* rois, int K,
+                           O* out_or_gradout, int32_t* levels_out, cudaStream_t st) {
+    GenericMaps M;
+    M.channels_last = nhwc_maps(cfg);
+    for (int l = 0; l < RSDET_MAX_LEVELS; l++) {
+        M.feat[l] = nullptr;
+        M.grad[l] = nullptr;
+        if (l >= cfg->num_levels) continue;
+        if constexpr (BACKWARD) M.grad[l] = maps[l];
+        else M.feat[l] = reinterpret_cast<const float*>(maps[l]);
+    }
+    const long long blocks = ceil_div_ll((long long)K * cfg->channels * cfg->pooled_h * cfg->pooled_w, 256);
+    roi_align_generic_kernel<BACKWARD, T, O, NHWC_ROIS><<<(int)(blocks < kNumSMs * 16 ? blocks : kNumSMs * 16), 256, 0, st>>>(
+        L, M, rois, K, out_or_gradout, levels_out);
+    count_launch();
+}
+
 }  // namespace rsdet
 
 using namespace rsdet;
@@ -1377,16 +1299,7 @@ static int forward_impl(const rsdet_roi_align_cfg* cfg, const T* const* feats_ho
     int rc = RSDET_OK;
     LevelSet L = make_levels(cfg);
     if (!fast_path_ok(cfg) || !nhwc_bases_aligned(cfg, feats_host, 4 * sizeof(T))) {
-        GenericMaps M;
-        M.channels_last = nhwc_maps(cfg);
-        for (int l = 0; l < RSDET_MAX_LEVELS; l++) {
-            M.feat[l] = l < cfg->num_levels ? reinterpret_cast<const float*>(feats_host[l]) : nullptr;
-            M.grad[l] = nullptr;
-        }
-        long long total = (long long)num_rois * cfg->channels * cfg->pooled_h * cfg->pooled_w;
-        int grid = (int)(ceil_div_ll(total, 256) < (long long)kNumSMs * 16 ? ceil_div_ll(total, 256) : (long long)kNumSMs * 16);
-        roi_align_generic_kernel<false, T, O, NHWC_OUT><<<grid, 256, 0, st>>>(L, M, rois, num_rois, out, levels_out);
-        count_launch();
+        launch_generic<false, T, O, NHWC_OUT>(cfg, L, feats_host, rois, num_rois, out, levels_out, st);
         return cuda_status();
     }
     if (workspace_bytes < roi_workspace_bytes(cfg, num_rois, 0, sizeof(T))) return RSDET_EWORKSPACE;
@@ -1401,32 +1314,28 @@ static int forward_impl(const rsdet_roi_align_cfg* cfg, const T* const* feats_ho
             L.feat[l] = reinterpret_cast<const float*>(ws.take<T>((size_t)cfg->batch * cfg->channels * cfg->height[l] * cfg->width[l]));
         if (!ws.ok()) return RSDET_EWORKSPACE;
     }
-    // locality order (needs the int[K] slot at the start of the workspace; skipped for tiny calls)
+    // locality order (needs the int[K] slot at the start of the workspace; skipped for tiny calls) and geometry records:
+    // for NCHW callers with an order of at most kPrepMaxRois RoIs, order block and geometry blocks ride with the
+    // pyramid transpose; every other call launches roi_prep_kernel (then NCHW callers the plain transpose)
     int* order = num_rois >= 256 && order_ws ? order_ws : nullptr;
     const bool ride = !nhwc_maps(cfg) && order && num_rois <= kPrepMaxRois;
-    // the persistent 7x7 kernel (it needs a 16-byte aligned output for its bulk stores; an NHWC output, stored from
-    // registers, needs four-element alignment) and its lean prologue: records by RoI index only, one launch, and for NCHW
-    // callers no launch at all -- order block and geometry blocks ride with the transpose.  Everything else runs
-    // roi_align_fwd_kernel behind the order and geometry kernels.
-    const bool lean = fwd77_ok(cfg) && (((size_t)out) & (NHWC_OUT ? 4 * sizeof(O) - 1 : 15)) == 0;
-    if (!lean) launch_prep(L, rois, num_rois, geoms, order, levels_out, st, ride);
-    else if (!ride) {
+    if (!ride) {
         roi_prep_kernel<<<(order ? 1 : 0) + ceil_div(num_rois, 1024), 1024, 0, st>>>(L, rois, num_rois, order, geoms, levels_out, counter);
         count_launch();
     }
     if (!nhwc_maps(cfg)) {
-        // NCHW -> NHWC copy of the pyramid; the locality-order block rides along as block 0 of the same launch
-        PrepArgs prep = {&L, rois, num_rois, order};
-        if (lean) { prep.geoms = geoms; prep.levels_out = levels_out; prep.counter = counter; }
+        PrepArgs prep = {&L, rois, num_rois, order, geoms, levels_out, counter};
         T* dst[RSDET_MAX_LEVELS];
         for (int l = 0; l < cfg->num_levels; l++) dst[l] = reinterpret_cast<T*>(const_cast<float*>(L.feat[l]));
         rc = launch_transpose(true, feats_host, dst, cfg->height, cfg->width, cfg->num_levels, cfg->batch, cfg->channels, st,
                               ride ? &prep : nullptr);
         if (rc != RSDET_OK) return rc;
-        if (ride && !lean) launch_geometry(L, rois, num_rois, order, geoms, levels_out, st);
     }
+    // the persistent 7x7 kernel needs a 16-byte aligned output for its bulk stores (an NHWC output, stored from registers,
+    // four-element alignment); everything else runs roi_align_fwd_kernel
+    const bool persistent = fwd77_ok(cfg) && (((size_t)out) & (NHWC_OUT ? 4 * sizeof(O) - 1 : 15)) == 0;
     GatherTimer gather_timer(st);
-    if (lean) {
+    if (persistent) {
         const int chunks = cfg->channels / 256;
         const long long items = (long long)num_rois * chunks, ctas = kNumSMs * kFwd77pCtasPerSm;
         const size_t smp = kStage77pOffset + (NHWC_OUT ? 0 : sizeof(float) * 49 * 256);
@@ -1441,10 +1350,10 @@ static int forward_impl(const rsdet_roi_align_cfg* cfg, const T* const* feats_ho
     dim3 grid(num_rois, ceil_div(cfg->channels / 4, Q));
     if (cfg->channels % 256 == 0) {
         set_dyn_smem((const void*)roi_align_fwd_kernel<2, T, O, NHWC_OUT>, smem);
-        roi_align_fwd_kernel<2, T, O, NHWC_OUT><<<grid, kRoiThreads, smem, st>>>(L, rois, order, geoms, num_rois, out, nullptr);
+        roi_align_fwd_kernel<2, T, O, NHWC_OUT><<<grid, kRoiThreads, smem, st>>>(L, order, geoms, num_rois, out);
     } else {
         set_dyn_smem((const void*)roi_align_fwd_kernel<1, T, O, NHWC_OUT>, smem);
-        roi_align_fwd_kernel<1, T, O, NHWC_OUT><<<grid, kRoiThreads, smem, st>>>(L, rois, order, geoms, num_rois, out, nullptr);
+        roi_align_fwd_kernel<1, T, O, NHWC_OUT><<<grid, kRoiThreads, smem, st>>>(L, order, geoms, num_rois, out);
     }
     count_launch();
     return cuda_status();
@@ -1530,24 +1439,19 @@ static int backward_impl(const rsdet_roi_align_cfg* cfg, const G* grad_out, cons
     if (num_rois > 0) {
         if (!grad_out || !rois) return RSDET_EINVAL;
         if (!fast) {
-            GenericMaps M;
-            M.channels_last = nhwc_maps(cfg);
-            for (int l = 0; l < RSDET_MAX_LEVELS; l++) { M.feat[l] = nullptr; M.grad[l] = l < cfg->num_levels ? acc[l] : nullptr; }
-            long long total = (long long)num_rois * cfg->channels * cfg->pooled_h * cfg->pooled_w;
-            int grid = (int)(ceil_div_ll(total, 256) < (long long)kNumSMs * 16 ? ceil_div_ll(total, 256) : (long long)kNumSMs * 16);
-            roi_align_generic_kernel<true, float, G, NHWC_IN><<<grid, 256, 0, st>>>(L, M, rois, num_rois, const_cast<G*>(grad_out), nullptr);
+            launch_generic<true, float, G, NHWC_IN>(cfg, L, acc, rois, num_rois, const_cast<G*>(grad_out), nullptr, st);
         } else {
             size_t smem = fwd_smem_bytes(cfg);
             set_dyn_smem((const void*)roi_align_bwd_kernel<1, G, NHWC_IN>, smem);
             set_dyn_smem((const void*)roi_align_bwd_kernel<2, G, NHWC_IN>, smem);
             int* order = num_rois >= 256 ? order_ws : nullptr;
-            launch_prep(L, rois, num_rois, geoms, order, nullptr, st);
+            roi_prep_kernel<<<(order ? 1 : 0) + ceil_div(num_rois, 1024), 1024, 0, st>>>(L, rois, num_rois, order, geoms, nullptr, nullptr);
             int Q = quads_per_chunk(cfg->channels);
             dim3 grid(num_rois, ceil_div(cfg->channels / 4, Q));
-            if (cfg->channels % 256 == 0) roi_align_bwd_kernel<2, G, NHWC_IN><<<grid, kRoiThreads, smem, st>>>(L, rois, order, geoms, num_rois, grad_out);
-            else roi_align_bwd_kernel<1, G, NHWC_IN><<<grid, kRoiThreads, smem, st>>>(L, rois, order, geoms, num_rois, grad_out);
+            if (cfg->channels % 256 == 0) roi_align_bwd_kernel<2, G, NHWC_IN><<<grid, kRoiThreads, smem, st>>>(L, order, geoms, num_rois, grad_out);
+            else roi_align_bwd_kernel<1, G, NHWC_IN><<<grid, kRoiThreads, smem, st>>>(L, order, geoms, num_rois, grad_out);
+            count_launch(2);
         }
-        count_launch();
     }
     if (!direct) {
         if constexpr (!kIsF32<T>) {

@@ -98,8 +98,8 @@ def big_scene(cuda):
 @pytest.mark.parametrize("shifted", [False, True], ids=["aligned", "shifted"])
 @pytest.mark.parametrize("maps_nhwc", [False, True], ids=["nchw", "nhwc"])
 def test_forward_77_paths(big_scene, maps_nhwc, shifted, K, dts):
-    """7x7 / sr 2 / C 256: aligned -> persistent kernel (ride-along prologue for NCHW maps and 256 <= K <= 16384,
-    roi_prep_kernel otherwise), shifted -> roi_align_fwd_kernel<2> with scalar stores."""
+    """7x7 / sr 2 / C 256, behind the ride-along prologue for NCHW maps and 256 <= K <= 16384 and roi_prep_kernel
+    otherwise: aligned -> persistent kernel, shifted -> roi_align_fwd_kernel<2> with scalar stores."""
     from test_gpu_roi_paths import Scene
     scene = Scene(big_scene.np, big_scene.rois_np[:K], big_scene.scales)
     scene.nchw, scene.nhwc = big_scene.nchw, big_scene.nhwc

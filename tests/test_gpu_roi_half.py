@@ -160,7 +160,7 @@ def batch8_scene(cuda):
 @pytest.mark.parametrize("dtype", HALF, ids=HALF_IDS)
 @pytest.mark.parametrize("channels_last", [False, True], ids=["nchw", "nhwc"])
 def test_forward_batch8_32000(batch8_scene, dtype, channels_last):
-    """The benchmark's batched call: 8 tiles, 32 000 RoIs (the lean roi_prep_kernel prologue)."""
+    """The benchmark's batched call: 8 tiles, 32 000 RoIs (the roi_prep_kernel prologue)."""
     h = _clone(batch8_scene)
     h.nchw = [x.to(dtype) for x in batch8_scene.nchw]
     h.nhwc = [x.to(dtype) for x in batch8_scene.nhwc]

@@ -2,7 +2,7 @@
 
 bench.py measures one 8-tile step (`run_ours` -> `device_step`): eight obb2poly + multiclass_nms_rotated chains on
 high-priority side streams (each multiclass call forks its class sort onto a library-internal side lane) and ONE
-extractor call over all 8 tiles -- 32 000 RoIs, batch 8, which takes the lean `roi_prep_kernel` prologue
+extractor call over all 8 tiles -- 32 000 RoIs, batch 8, which takes the `roi_prep_kernel` prologue
 (K > kPrepMaxRois) instead of the transpose ride-along every per-tile call takes -- captured once into a CUDA graph
 and replayed.  These tests rebuild that step, check every output of an eager step against the oracle and against
 per-tile extractor calls, check that graph replays (also after the inputs are overwritten in place) reproduce the
@@ -210,7 +210,7 @@ def _check_vs_reference(snap, want, ref8, perm=tuple(range(T))):
         scale = float(np.abs(w["feat_rows"]).max())
         nbad, err, _ = close_report(got, w["feat_rows"], 1e-5, 1e-5 * scale)
         assert nbad == 0, f"slot {i} (tile {t}): {nbad} RoI feature values off the oracle (max abs err {err:.3g}, scale {scale:.3g})"
-        # The batched call (lean prologue, batch-aware locality order) and the per-tile call (prologue riding with the
+        # The batched call (roi_prep_kernel prologue, batch-aware locality order) and the per-tile call (prologue riding with the
         # transpose) run the same geometry and gather arithmetic per RoI: only WHICH CTA takes a RoI differs.
         _assert_rows_equal(out8[i * K:(i + 1) * K], ref8[t * K:(t + 1) * K], f"slot {i} (tile {t}) vs its per-tile extractor call")
 
