@@ -297,6 +297,16 @@ int rsdet_iou_poly_pairs(const double* polys1, const double* polys2, int n, doub
  * polys (n,8) fp64 in-tile coords; offs (n,3) fp64 [x, y, rate] per row. */
 int rsdet_poly2origpoly(const double* polys, const double* offs, int n, double* out, void* stream);
 
+/* ops/bbox_transforms.py:549-575 and merge.py:73-100 poly2obb on 4-point polygons: cv2.minAreaRect of the corners
+ * rounded to float32 (round to nearest, as astype(np.float32)), then the le90 step in float64.  polys (n,8) fp64 ->
+ * obb (n,5) fp64 [cx, cy, w, h, theta], bit-identical to the host function with OpenCV 4.13 (agreement with the
+ * reference's pinned 4.5.5 is unverified).  The angle passes through one double atan2 (CUDA: within 2 ulp; host:
+ * glibc), rounded to float afterwards: the two can only disagree where the exact value lies within a few double ulps
+ * of a float rounding boundary.  One thread per quad; no workspace, no allocation, no host synchronisation.  NaN or
+ * Inf coordinates give undefined results.  n < 0, or a null pointer with n > 0, returns RSDET_EINVAL before any
+ * launch. */
+int rsdet_poly2obb(const double* polys, int n, double* obb, void* stream);
+
 /* ---------------------------------------------------------------- SURVEY 8(f) rank 1: head tail fusion
  * models/roi_heads/oriented_head.py:498-536 (get_bboxes) + :279-305 (get_results), with
  * OrientedDeltaXYWHTCoder.decode (models/boxes/coder.py:477-514), regular_theta / regular_obb

@@ -48,6 +48,7 @@ SIGNATURES = {
     "rsdet_obb2hbb": (C.c_int, [_vp, C.c_int, _vp, _vp]),
     "rsdet_poly2hbb": (C.c_int, [_vp, C.c_int, C.c_int, _vp, _vp]),
     "rsdet_poly2origpoly": (C.c_int, [_vp, _vp, C.c_int, _vp, _vp]),
+    "rsdet_poly2obb": (C.c_int, [_vp, C.c_int, _vp, _vp]),
     "rsdet_iou_poly_pairs": (C.c_int, [_vp, _vp, C.c_int, _vp, _vp]),
     "rsdet_box_iou_rotated_workspace_bytes": (C.c_size_t, [C.c_int, C.c_int]),
     "rsdet_box_iou_rotated": (C.c_int, [_vp, C.c_int, _vp, C.c_int, C.c_int, C.c_int, _vp, _vp, C.c_size_t, _vp]),

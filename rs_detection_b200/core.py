@@ -60,6 +60,19 @@ def poly2origpoly(polys: torch.Tensor, offs: torch.Tensor) -> torch.Tensor:
     return out
 
 
+def poly2obb(polys: torch.Tensor) -> torch.Tensor:
+    """(n, 8) CUDA quads -> (n, 5) fp64 [cx, cy, w, h, theta]: cv2.minAreaRect of the corners as float32 points, then
+    the le90 step, bit for bit as jdet.ops.bbox_transforms.poly2obb (include/rsdet.h)."""
+    if not polys.is_cuda:
+        raise RuntimeError("expected a CUDA tensor (no CPU fallback)")
+    p = polys.to(torch.float64).contiguous()
+    if p.dim() != 2 or p.shape[1] != 8:
+        raise ValueError(f"poly2obb: expected (n, 8) quads, got {tuple(p.shape)}")
+    out = torch.empty((p.shape[0], 5), dtype=torch.float64, device=p.device)
+    check(load().rsdet_poly2obb(ptr(p), p.shape[0], ptr(out), stream_ptr()), "poly2obb")
+    return out
+
+
 def iou_poly_pairs(p: torch.Tensor, q: torch.Tensor) -> torch.Tensor:
     a = p.to(torch.float64).contiguous().reshape(-1, 8)
     b = q.to(torch.float64).contiguous().reshape(-1, 8)

@@ -61,15 +61,16 @@ def py_cpu_nms(dets, thresh):
 
 
 def py_cpu_nms_obb(dets, thresh):
-    """:128-141 -- polygons -> oriented boxes (`poly2obb`: cv2.minAreaRect on the host, as in the reference) ->
-    `nms_rotated_cpu` (suppress IoU >= thresh) -> kept indices in ASCENDING index order (`jt.where(keep)[0]`)."""
-    from ...ops.bbox_transforms import poly2obb
+    """:128-141 -- polygons -> oriented boxes (`poly2obb`: the device restatement of the reference's cv2.minAreaRect,
+    bit for bit) -> `nms_rotated_cpu` (suppress IoU >= thresh) -> kept indices in ASCENDING index order
+    (`jt.where(keep)[0]`)."""
     require_cuda()
     d = np.ascontiguousarray(dets, dtype=np.float64).reshape(-1, 9)
     if d.shape[0] == 0:
         return np.array([])
-    obb = torch.from_numpy(poly2obb(d[:, :8]).astype(np.float32)).cuda()
-    sc = torch.from_numpy(d[:, 8].astype(np.float32)).cuda()
+    t = torch.from_numpy(d).cuda()
+    obb = core.poly2obb(t[:, :8]).to(torch.float32)
+    sc = t[:, 8].to(torch.float32)
     res = core.nms(NMS_ROTATED_GE, obb, sc, float(thresh), want_mask=False, want_sorted=True, ws_tag="merge")
     return res.sorted_idx.cpu().numpy()
 

@@ -2,9 +2,10 @@
 
 The horizontal NMS (`nms`, keeps `iou < thresh`) runs on the device: `merge_csv_with_class` /
 `merge_csv_without_class` send EVERY (image, class) group of the ensemble through one launch of the
-engine (`RSDET_NMS_HBB`, float64).  `poly2obb` keeps the reference's OpenCV call
-(`cv2.minAreaRect` on float32 points, merge.py:86): that is the reference's own third-party
-dependency and a per-row format conversion, not part of the suppression arithmetic.
+engine (`RSDET_NMS_HBB`, float64).  The ensemble converts its rows with `rsdet_poly2obb`, the device
+restatement of the reference's `cv2.minAreaRect` + le90 step (merge.py:73-100), bit for bit; `obb2hbb`
+stays numpy float64, whose `cos`/`sin` bits decide the NMS.  `poly2obb` below is the host OpenCV
+function, kept as the reference for the device call.
 """
 import numpy as np
 import torch
@@ -71,7 +72,8 @@ def _grouped_nms(dets, group, thr_per_group):
     """dets (n,11), group (n,) int32 ascending-group output order; returns kept row indices ordered by
     (group asc, score desc)."""
     require_cuda()
-    hbb = obb2hbb(poly2obb(dets[:, 1:9]))
+    polys = torch.from_numpy(np.ascontiguousarray(dets[:, 1:9], dtype=np.float64)).cuda()
+    hbb = obb2hbb(core.poly2obb(polys).cpu().numpy())
     b = torch.from_numpy(np.ascontiguousarray(hbb, dtype=np.float64)).cuda()
     s = torch.from_numpy(np.ascontiguousarray(dets[:, 9], dtype=np.float64)).cuda()
     res = core.nms(NMS_HBB, b, s, float(thr_per_group[0]), labels=torch.from_numpy(group.astype(np.int32)).cuda(),

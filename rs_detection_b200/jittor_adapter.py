@@ -93,6 +93,14 @@ def poly2hbb(polys):
     return _transform("rsdet_poly2hbb", polys, 4, ", %d" % (polys.shape[-1] // 2))
 
 
+def poly2obb(polys):
+    """ops/bbox_transforms.py:549-575 on 4-point polygons (cv2.minAreaRect + le90): (..., 8) -> (..., 5) float64."""
+    assert polys.shape[-1] == 8, "poly2obb: 4-point polygons only"
+    if polys.dtype != "float64":
+        polys = polys.float64()
+    return _transform("rsdet_poly2obb", polys, 5)
+
+
 # ------------------------------------------------------------------------------------------------ rotated IoU
 def box_iou_rotated(boxes1, boxes2, version=0):
     """jdet.ops.box_iou_rotated / box_iou_rotated_v1 (box_iou_rotated.py:502-509, box_iou_rotated_v1.py:507-524)."""

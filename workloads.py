@@ -147,6 +147,24 @@ FAIR1M_CLASSES = ['Airplane', 'Ship', 'Vehicle', 'Basketball_Court', 'Tennis_Cou
                   'Baseball_Field', 'Intersection', 'Roundabout', 'Bridge']
 
 
+def csv_submissions(num_images=20, objects_per_image=500, scene=15000.0, seed=0):
+    """Two FAIR1M CSV submissions of the same scenes as `merge.read_csv_to_numpy` returns them: (n,11) float64 rows
+    [image id, 8 coords rounded to 4 decimals, score, class 1..10].  The second run sees the same objects with
+    jittered corners and its own scores, so the ensemble NMS has overlapping pairs to suppress."""
+    rng = np.random.default_rng(seed + 7919)
+    subs = [[], []]
+    for img in range(num_images):
+        o = rotated_boxes(objects_per_image, seed * 1000 + img, canvas=scene, smin=8.0, smax=256.0, dtype=np.float64)
+        cls = rng.integers(1, 11, objects_per_image)
+        for run in range(2):
+            q = o.copy()
+            q[:, :2] += rng.normal(0, 2.0, (objects_per_image, 2))
+            p = np.round(obb_to_poly64(q) + rng.normal(0, 0.5, (objects_per_image, 8)), 4)
+            sc = np.round(rng.uniform(0.05, 1.0, objects_per_image), 4)
+            subs[run].append(np.concatenate([np.full((objects_per_image, 1), img), p, sc[:, None], cls[:, None]], 1))
+    return [np.concatenate(s) for s in subs]
+
+
 def tile_results(num_objects=300, num_classes=10, scene=3000, num_scenes=2, seed=0, tile=TILE, gap=200, rates=(0.5, 1.0),
                  jitter_px=1.0):
     """The runner's per-tile result list `[((polys (k,8), scores (k,), labels (k,)), {"img_file": ...}), ...]` as
